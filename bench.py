@@ -29,6 +29,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "full-dynamics Talos MPC solves/sec at batch 4096"
+DUMP_INSTANCES = 512  # --dump-outputs: ~38 MB of results; every instance of batch 4096 would be ~300 MB
 UNIT = "solves/s"
 WORKLOADS = {
     "walk": ("BASELINE configs[4]: full-dynamics Talos MPC tick (solver.setup + 1 ProxDDP iteration), T=100, global batch 4096; instance i sits at tick "
@@ -59,7 +60,12 @@ def parse():
     ap.add_argument("--no-qp", action="store_true", help="skip the batched whole-body QP leg (SURVEY 8f row f-3)")
     ap.add_argument("--qp-only", action="store_true", help="run only the batched whole-body QP leg and print its object")
     ap.add_argument("--latency-ticks", type=int, default=200, help="warm single-instance MPC ticks for the p50 latency (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (xs, us, K0, info) for a "
+                    f"fixed, seeded sample of at most {DUMP_INSTANCES} instances of the global batch, and their indices, as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -240,6 +246,8 @@ def main():
     if G % world:
         raise SystemExit("bench.py: the global batch must be divisible by the number of GPUs")
     gather = world > 1 and not args.no_gather
+    if args.dump_outputs and world > 1 and not gather:
+        raise SystemExit("bench.py: --dump-outputs needs the gather of the results when there are several GPUs")
     prob = make_problem(args, count=B, lo=lo)
     solver = BatchSolver(prob["robot"], prob["cfg"], B, device=local)
     # untimed preparation = the reference's first solve (fulldynamic_talos.py:386-397): ProxDDP from the cold start at the
@@ -321,6 +329,8 @@ def main():
     wall = time.time() - t0
     dev_ms = ev0.elapsed_time(ev1)
     nric = klaunch["riccati"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gathered if gather else pack, G, world, T, nx, m, n)
     # ---- timed region 2: end to end through the host-buffer C-ABI
     tick_e2e()
     barrier()
@@ -421,6 +431,25 @@ def main():
     solver.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, packed, G, world, T, nx, m, n):
+    """Writes xs [S][T+1][nx], us [S][T][m], K0 [S][m][n] and info [S][8] of the instances `instances` [S] (a fixed, seeded sample
+    of S = min(G, DUMP_INSTANCES) instances of the global batch, in ascending order) from the packed result buffer of the last
+    step: one [xs | us | K0 | info] block per rank, ranks holding contiguous shards in rank order."""
+    import torch
+
+    Bl = G // world
+    idx = np.sort(np.random.default_rng(0).choice(G, size=min(G, DUMP_INSTANCES), replace=False))
+    sel = torch.from_numpy(idx).to(packed.device)
+    blocks = packed.view(world, -1)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instances.npy"), idx.astype(np.float64))
+    off = 0
+    for name, shape in (("xs", (T + 1, nx)), ("us", (T, m)), ("K0", (m, n)), ("info", (8,))):
+        size = Bl * int(np.prod(shape))
+        np.save(os.path.join(out_dir, name + ".npy"), blocks[:, off:off + size].reshape(G, *shape)[sel].cpu().numpy())
+        off += size
 
 
 def dgemm_peak(torch):

@@ -1,11 +1,12 @@
 #!/usr/bin/env python
-"""Generates tests/golden/*.npz.  Run in the BUILD container (needs /root/reference for the script-derived fixtures):
+"""Generates tests/golden/*.npz:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [REFERENCE_DIR]
 
-1. ref_flat_{full,kino,cent}.npz — the flat descriptor obtained by executing the TOP HALF of the unmodified reference script
-   (/root/reference/{fulldynamic,kinodynamic,centroidal}_talos.py up to the cold solve) through this package's aligator/pinocchio
-   shim (tests/ref_harness.py), plus the cold-solve result of the CPU ORACLE on that descriptor.
+1. ref_flat_{full,kino,cent}.npz (only with REFERENCE_DIR, a checkout of the edantec/MPC_benchmark scripts) — the flat descriptor
+   obtained by executing the TOP HALF of the unmodified reference script (REFERENCE_DIR/{fulldynamic,kinodynamic,centroidal}_talos.py
+   up to the cold solve) through this package's aligator/pinocchio shim (tests/ref_harness.py), plus the cold-solve result of the
+   CPU ORACLE on that descriptor (without the feedback gains, which no test reads: they would take the files over 1 MB).
 2. walk_full.npz — 4 instances of the synthetic random-schedule workload (bench.py) with 6 oracle iterations and one
    warm MPC tick (active cone / box constraints, non-zero multipliers).
 
@@ -39,15 +40,16 @@ def info_arrays(info):
                 traj_cost=np.array([i.traj_cost for i in info]), ls_evals=np.array([i.ls_evals for i in info]))
 
 
-def main():
-    if H.available():
+def main(ref_dir=None):
+    if ref_dir:
         for script, tag in [("fulldynamic_talos.py", "full"), ("kinodynamic_talos.py", "kino"), ("centroidal_talos.py", "cent")]:
-            ns, cap = H.run_top_half(script)
+            ns, cap = H.run_top_half(script, ref_dir)
+            assert [c[0] for c in cap] == ["setup", "run"], script
             flat, xs, us = cap[-1][1], cap[-1][2], cap[-1][3]
             prob = dict(robot=flat.robot, cfg=flat.cfg, knots=flat.knots, terms=flat.terms, x0=flat.x0, xs=xs[None], us=us[None])
             r = O.solve(prob, knot_threads=8)
             out = pack(prob)
-            out.update({"sol_" + k: r[k] for k in ["xs", "us", "K", "vs", "lams", "stage0"]})
+            out.update({"sol_" + k: r[k] for k in ["xs", "us", "vs", "lams", "stage0"]})
             out.update({"sol_" + k: v for k, v in info_arrays(r["info"]).items()})
             np.savez_compressed(os.path.join(HERE, f"ref_flat_{tag}.npz"), **out)
             print(script, "iters", out["sol_num_iters"], "conv", out["sol_conv"], "prim", out["sol_prim_infeas"])
@@ -64,4 +66,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1] if len(sys.argv) > 1 else None)

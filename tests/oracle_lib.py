@@ -3,6 +3,7 @@ nothing under mpc_benchmark_b200/ imports this module."""
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -10,7 +11,6 @@ from mpc_benchmark_b200 import _abi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _LIB = os.path.join(ROOT, "oracle", "_build", "liboracle.so")
-_LIB_NATIVE = os.path.join(ROOT, "oracle", "_build", "liboracle_native.so")
 
 dp = C.POINTER(C.c_double)
 
@@ -35,16 +35,20 @@ _lib = None
 
 def use_native():
     """CPU-baseline legs of bench.py only: build the oracle with -march=native ON THIS MACHINE (BASELINE.md section 3) and bind that
-    library instead of the portable one.  Must be called before the first lib() call.  Falls back to the portable build if the
-    compiler is unavailable."""
+    library instead of the portable one.  The library is built in a temporary directory, removed once it is loaded, so that the
+    source tree stays untouched (it may be read-only).  Must be called before the first lib() call.  Falls back to the portable
+    build if the compiler is unavailable."""
     global _lib
     assert _lib is None, "use_native() must come before the first oracle call"
-    try:
-        subprocess.check_call(["make", "-B", "-C", os.path.join(ROOT, "oracle"), "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-        _bind(_LIB_NATIVE)
-        return True
-    except (subprocess.CalledProcessError, OSError):
-        return False
+    with tempfile.TemporaryDirectory(prefix="liboracle-") as tmp:
+        so = os.path.join(tmp, "liboracle_native.so")
+        try:
+            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "native", f"NATIVE_LIB={so}"], stdout=subprocess.DEVNULL,
+                                  stderr=subprocess.DEVNULL)
+            _bind(so)  # the loaded mapping outlives the file
+            return True
+        except (subprocess.CalledProcessError, OSError):
+            return False
 
 
 def _bind(path):

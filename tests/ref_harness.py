@@ -1,22 +1,16 @@
-"""Runs the TOP HALF of a reference script (/root/reference/*_talos.py, read at test time — never copied into the repo)
-with `aligator` / `pinocchio` replaced by this package ("switch backends with one import", SURVEY 8b) and the plant /
-robot-data / spline packages stubbed (bullet_robot, example_robot_data, ndcurves, proxsuite are not installable offline).
+"""Runs the TOP HALF of a reference script (`*_talos.py` of a checkout of edantec/MPC_benchmark, passed as `ref_dir` — never
+copied into the repo) with `aligator` / `pinocchio` replaced by this package ("switch backends with one import", SURVEY 8b)
+and the plant / robot-data / spline packages stubbed (bullet_robot, example_robot_data, ndcurves, proxsuite).
 
 The script source is executed up to (excluding) the line `solver.max_iters = 1`, i.e. model construction + setup + cold
 solve (fulldynamic_talos.py:1-405).  `capture=True` replaces SolverProxDDP.setup/run by recorders so the flattening can
-be checked on a machine without GPU.
+be checked on a machine without GPU.  tests/golden/make_golden.py stores what it captures as tests/golden/ref_flat_*.npz.
 """
 import os
 import sys
 import types
 
 import numpy as np
-
-REF = "/root/reference"
-
-
-def available():
-    return os.path.isdir(REF)
 
 
 class _Stop(Exception):
@@ -72,12 +66,12 @@ def _stub_modules():
     return mods
 
 
-def run_top_half(script, capture=True):
+def run_top_half(script, ref_dir, capture=True):
     """Returns (namespace, captured) where captured = list of ('setup'|'run', FlatProblem, xs, us)."""
     import mpc_benchmark_b200 as pkg
     from mpc_benchmark_b200 import flatten
 
-    src = open(os.path.join(REF, script)).read()
+    src = open(os.path.join(ref_dir, script)).read()
     cut = src.index("solver.max_iters = 1")
     src = src[:cut]
     saved = {k: sys.modules.get(k) for k in list(_stub_modules())}
@@ -88,7 +82,7 @@ def run_top_half(script, capture=True):
         sys.modules.update(_stub_modules())
         for m in ("talos_utils", "QP_utils"):
             sys.modules.pop(m, None)
-        sys.path.insert(0, REF)
+        sys.path.insert(0, ref_dir)
         if capture:
             def fake_setup(self, problem):
                 self._check_options()
@@ -103,7 +97,7 @@ def run_top_half(script, capture=True):
             pkg.SolverProxDDP.setup, pkg.SolverProxDDP.run = fake_setup, fake_run
         ns = {"__name__": "__ref_script__"}
         try:
-            exec(compile(src, os.path.join(REF, script), "exec"), ns)
+            exec(compile(src, os.path.join(ref_dir, script), "exec"), ns)
         except _Stop:
             pass
         return ns, captured

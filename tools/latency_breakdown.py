@@ -1,5 +1,5 @@
-import sys, time, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mpc_benchmark_b200 import problems
 from mpc_benchmark_b200.batch import BatchSolver
 prob = problems.full_walk_batch(1, seed=5)
