@@ -4,8 +4,19 @@
 // proportional to the number of instances still working, not to the batch.
 #pragma once
 #include "solver_core.cuh"
+#include <type_traits>
 
 namespace mpcdev {
+
+// f(std::integral_constant<int, KIND>{}) for the runtime model kind: the one place where a kind becomes the template argument
+// of KindTraits and of the kernels
+template <class F> auto dispatch_kind(int kind, F &&f) {
+  switch (kind) {
+  case MPC_KIND_FULL: return f(std::integral_constant<int, MPC_KIND_FULL>{});
+  case MPC_KIND_KINO: return f(std::integral_constant<int, MPC_KIND_KINO>{});
+  default: return f(std::integral_constant<int, MPC_KIND_CENT>{});
+  }
+}
 
 // Backend: reset_counters(), eval(deriv, list, n), decide_eval(list, n, next_eval), riccati(list, n), apply_step(list, n),
 //          decide_ls(list, n, ls_out, next_eval), rollout_ls(list, n, next_eval), read_counters(int[4])
@@ -42,6 +53,14 @@ template <class Backend> int run_loop(Backend &be, const Ws &w, int max_iters, c
     cur ^= 1;
   }
   return launches;
+}
+
+// one instance's solve summary as the C-ABI returns it
+inline mpc_info_t info_of(const InstState &s) {
+  mpc_info_t o;
+  o.prim_infeas = s.prim_infeas; o.dual_infeas = s.dual_infeas; o.traj_cost = s.traj_cost; o.merit = s.merit; o.mu = s.mu; o.alpha = s.alpha;
+  o.ls_evals = s.ls_evals; o.pad_ = 0; o.num_iters = s.num_iters; o.al_iters = s.al_iters; o.conv = s.conv; o.status = s.status;
+  return o;
 }
 
 } // namespace mpcdev

@@ -43,4 +43,14 @@ inline void gait_fill_cfg(const mpc_gait_t &p, int kind, int nsteps, GaitCfg &g)
   g.phases = nullptr; g.urefs = nullptr;
 }
 
+// every robot starts with both soles at the gait's initial placements; mirror (optional, [batch]): robots whose first swing is made with the other foot
+inline std::vector<GaitRobot> gait_init_robots(const mpc_gait_t &p, int batch, const int32_t *mirror) {
+  std::vector<GaitRobot> rs(batch);
+  for (int b = 0; b < batch; b++) {
+    for (int i = 0; i < 12; i++) { rs[b].start_l[i] = rs[b].final_l[i] = rs[b].next_l[i] = p.lf0[i]; rs[b].start_r[i] = rs[b].final_r[i] = rs[b].next_r[i] = p.rf0[i]; }
+    rs[b].mirror = mirror ? (mirror[b] != 0) : 0; rs[b].pad_ = 0;
+  }
+  return rs;
+}
+
 } // namespace mpcdev

@@ -83,6 +83,27 @@ int upload(mpc_qp *h, Slot &s, const double *src, long long stride, int batch, c
   return 0;
 }
 
+// inputs of k_qp_assemble_id for B QPs, carved out of the handle's scratch: M, nle, Jc, gamma, a, forces, cs
+struct AsmScratch {
+  double *M, *nle, *Jc, *gamma, *a, *forces;
+  int32_t *cs;
+  AsmScratch(double *s, size_t B)
+      : M(s), nle(M + B * 784), Jc(nle + B * 28), gamma(Jc + B * 336), a(gamma + B * 12), forces(a + B * 28), cs((int32_t *)(forces + B * 12)) {}
+};
+
+// assemble the whole-body ID QPs from the scratch into the handle's A, b, C, l, which then hold one array per QP
+int assemble_id(mpc_qp *h, const AsmScratch &s, int batch, double mu, double L, double W) {
+  AsmArgs P;
+  P.M = s.M; P.nle = s.nle; P.Jc = s.Jc; P.gamma = s.gamma; P.a = s.a; P.forces = s.forces; P.cs = s.cs; P.mu = mu; P.L = L; P.W = W;
+  P.A = h->A.d; P.b = h->b.d; P.C = h->C.d; P.l = h->l.d; P.batch = batch;
+  k_qp_assemble_id<<<batch, QP_THREADS, 0, h->stream>>>(P);
+  CUQ(cudaGetLastError());
+  h->A.stride = h->A.per; h->b.stride = h->b.per; h->C.stride = h->C.per; h->l.stride = h->l.per;
+  h->A.set = h->b.set = h->C.set = h->l.set = true;
+  h->batch = batch;
+  return 0;
+}
+
 int launch(mpc_qp *h, const QPArgs &P, cudaStream_t stream) {
   if (P.batch <= 0) return 0;
   const int grid = P.batch; // one CTA per QP: QPs take different numbers of Newton steps, the hardware scheduler balances them
@@ -253,25 +274,15 @@ int32_t mpc_qp_assemble_id(mpc_qp_t *h, int32_t batch, const double *M, const do
   if (batch <= 0 || batch > h->max_batch) return fail("mpc_qp_assemble_id: batch out of range");
   CUQ(cudaSetDevice(h->device));
   const size_t B = batch;
-  double *s = h->dscratch;
-  AsmArgs P;
-  double *dM = s; s += B * 784; double *dn = s; s += B * 28; double *dJ = s; s += B * 336; double *dg = s; s += B * 12; double *da = s; s += B * 28;
-  double *df = s; s += B * 12; int32_t *dcs = (int32_t *)s;
-  CUQ(cudaMemcpyAsync(dM, M, 8 * B * 784, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(dn, nle, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(dJ, Jc, 8 * B * 336, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(dg, gamma, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(da, a, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(df, forces, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(dcs, cs, 4 * B * 2, cudaMemcpyHostToDevice, h->stream));
-  P.M = dM; P.nle = dn; P.Jc = dJ; P.gamma = dg; P.a = da; P.forces = df; P.cs = dcs; P.mu = mu; P.L = L; P.W = W;
-  P.A = h->A.d; P.b = h->b.d; P.C = h->C.d; P.l = h->l.d; P.batch = batch;
-  k_qp_assemble_id<<<batch, QP_THREADS, 0, h->stream>>>(P);
-  CUQ(cudaGetLastError());
-  h->A.stride = h->A.per; h->b.stride = h->b.per; h->C.stride = h->C.per; h->l.stride = h->l.per;
-  h->A.set = h->b.set = h->C.set = h->l.set = true;
-  h->batch = batch;
-  return 0;
+  const AsmScratch s(h->dscratch, B);
+  CUQ(cudaMemcpyAsync(s.M, M, 8 * B * 784, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.nle, nle, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.Jc, Jc, 8 * B * 336, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.gamma, gamma, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.a, a, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.forces, forces, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.cs, cs, 4 * B * 2, cudaMemcpyHostToDevice, h->stream));
+  return assemble_id(h, s, batch, mu, L, W);
 }
 
 int32_t mpc_qp_assemble_id_from_state(mpc_qp_t *h, struct mpc_solver *solver, int32_t batch, const double *x, const double *a, const double *forces,
@@ -281,26 +292,16 @@ int32_t mpc_qp_assemble_id_from_state(mpc_qp_t *h, struct mpc_solver *solver, in
   if (batch <= 0 || batch > h->max_batch) return fail("mpc_qp_assemble_id_from_state: batch out of range");
   CUQ(cudaSetDevice(h->device));
   const size_t B = batch;
-  // scratch layout as in mpc_qp_assemble_id (M, nle, Jc, gamma, a, forces, cs); the states go where a / forces do not reach: behind cs
-  double *s = h->dscratch;
-  double *dM = s; s += B * 784; double *dn = s; s += B * 28; double *dJ = s; s += B * 336; double *dg = s; s += B * 12; double *da = s; s += B * 28;
-  double *df = s; s += B * 12; int32_t *dcs = (int32_t *)s;
+  // M, nle, Jc and gamma come from the rigid-body terms of the states (held in dstate with the frame velocities behind them)
+  const AsmScratch s(h->dscratch, B);
   CUQ(cudaMemcpyAsync(h->dstate, x, 8 * B * 57, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(da, a, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(df, forces, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
-  CUQ(cudaMemcpyAsync(dcs, cs, 4 * B * 2, cudaMemcpyHostToDevice, h->stream));
-  if (mpc_rbd_terms_device(solver, batch, (uint64_t)h->dstate, (uint64_t)dM, (uint64_t)dn, (uint64_t)dJ, (uint64_t)dg, (uint64_t)(h->dstate + B * 57), (uint64_t)h->stream) != 0)
+  CUQ(cudaMemcpyAsync(s.a, a, 8 * B * 28, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.forces, forces, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.cs, cs, 4 * B * 2, cudaMemcpyHostToDevice, h->stream));
+  if (mpc_rbd_terms_device(solver, batch, (uint64_t)h->dstate, (uint64_t)s.M, (uint64_t)s.nle, (uint64_t)s.Jc, (uint64_t)s.gamma, (uint64_t)(h->dstate + B * 57), (uint64_t)h->stream) != 0)
     return fail(std::string("mpc_rbd_terms_device: ") + mpc_last_error());
-  k_qp_gamma<<<(batch * 12 + 127) / 128, 128, 0, h->stream>>>(dg, h->dstate + B * 57, dcs, kd, batch);
-  AsmArgs P;
-  P.M = dM; P.nle = dn; P.Jc = dJ; P.gamma = dg; P.a = da; P.forces = df; P.cs = dcs; P.mu = mu; P.L = L; P.W = W;
-  P.A = h->A.d; P.b = h->b.d; P.C = h->C.d; P.l = h->l.d; P.batch = batch;
-  k_qp_assemble_id<<<batch, QP_THREADS, 0, h->stream>>>(P);
-  CUQ(cudaGetLastError());
-  h->A.stride = h->A.per; h->b.stride = h->b.per; h->C.stride = h->C.per; h->l.stride = h->l.per;
-  h->A.set = h->b.set = h->C.set = h->l.set = true;
-  h->batch = batch;
-  return 0;
+  k_qp_gamma<<<(batch * 12 + 127) / 128, 128, 0, h->stream>>>(s.gamma, h->dstate + B * 57, s.cs, kd, batch);
+  return assemble_id(h, s, batch, mu, L, W);
 }
 
 } // extern "C"

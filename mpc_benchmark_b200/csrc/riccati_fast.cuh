@@ -298,10 +298,9 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
   // W_k and [A B]_k (single stage), the first KROWS gain rows and the small per-knot vectors (two stages) go global -> shared by bulk
   // copies into the now dead H / P / G buffers: W / [A B] of knot k + 1 are requested as soon as knot k's mat-vecs are done, gain rows
   // and vectors two knots ahead; everything is bulk-prefetched from HBM into L2 PF knots ahead of the chain dx_k -> du_k -> dx_{k+1}
-#ifndef MPC_RIC_PF
-#define MPC_RIC_PF 1
-#endif
-  constexpr int PF = MPC_RIC_PF; // knots of HBM -> L2 prefetch ahead of the chain (resident instances x PF x 76 KB must stay well inside L2)
+  // knots of HBM -> L2 prefetch ahead of the chain (resident instances x PF x 76 KB must stay well inside L2); distances 2 and 3 read
+  // more from DRAM in the same kernel time
+  constexpr int PF = 1;
   constexpr int FWA = N * LDW + N * NZ;    // W_k | [A B]_k
   constexpr int FX = 4 * N + NZ + 36;      // pt_k, fbar_k, lplus_{k+1}, lam_{k+1}, lxu_k, T6_k
   constexpr int KROWS = ((((ZP * LDH + Lay::un - FWA - 2 * FX) / 2) / NR) & ~1) < S ? ((((ZP * LDH + Lay::un - FWA - 2 * FX) / 2) / NR) & ~1) : (S & ~1);

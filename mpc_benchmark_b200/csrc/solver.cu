@@ -14,7 +14,6 @@
 #include "gait_host.hpp"
 #include <cuda_runtime.h>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -32,30 +31,21 @@ static int fail(const std::string &m) { g_err = m; return 1; }
 // ------------------------------------------------------------------ kernels
 __global__ void k_init(Ws w, const double *xs_in, const double *us_in, int max_iters, int first) { init_instance(w, first + blockIdx.x, xs_in, us_in, max_iters); }
 
-#ifndef MPC_VALUES_CTAS
-#define MPC_VALUES_CTAS 5 /* values-only knots resident per SM */
-#endif
-#ifndef MPC_VALUES_G
-#define MPC_VALUES_G 5 /* of which per CTA */
-#endif
-#ifndef MPC_VALUES_TH
-#define MPC_VALUES_TH 96 /* threads per values-only knot (full / kinodynamic): 5 x 96 in one CTA measured 16 % faster than 2 CTAs of 2 x 128 */
-#endif
 // Evaluation kernel launch shape: G knots per CTA (one group of TH threads each, own shared-memory slice and named barrier).
 // The groups of a CTA start together and run the same instruction stream, which is what keeps the (large, mostly
 // straight-line) evaluation code from being fetched G times per SM: ncu showed 59 % instruction-cache hits and
 // "no instruction" as the second stall reason with one knot per CTA.
 template <int KIND, bool DERIV> struct EvalShape {
   // full-dynamics derivative pass: FOUR knots of 96 threads per SM (same 384 threads / register budget as three of 128; the tangent
-  // matrices live in the L2-resident global scratch, which brings a knot's shared memory under 56 KB)
-  static constexpr int TH = (KIND == MPC_KIND_CENT) ? 32 : ((KIND == MPC_KIND_FULL && DERIV) ? 96 : (DERIV ? 128 : MPC_VALUES_TH));
-  static constexpr int G = (KIND == MPC_KIND_CENT) ? 4 : (DERIV ? ((KIND == MPC_KIND_FULL) ? 4 : 3) : MPC_VALUES_G); // knots per CTA
-  static constexpr int CTAS = (KIND == MPC_KIND_CENT || DERIV) ? 1 : MPC_VALUES_CTAS / MPC_VALUES_G; // CTAs per SM
-  static constexpr size_t raw = (KIND == MPC_KIND_FULL) ? sizeof(FullWsT<DERIV>) : (KIND == MPC_KIND_KINO) ? sizeof(KinoWsT<DERIV>) : sizeof(CentWs);
+  // matrices live in the L2-resident global scratch, which brings a knot's shared memory under 56 KB).  Values-only passes (full /
+  // kinodynamic): five knots of 96 threads in one CTA measured 16 % faster than 2 CTAs of 2 x 128.
+  static constexpr int TH = (KIND == MPC_KIND_CENT) ? 32 : (KIND == MPC_KIND_KINO && DERIV) ? 128 : 96;
+  static constexpr int G = (KIND == MPC_KIND_CENT) ? 4 : DERIV ? ((KIND == MPC_KIND_FULL) ? 4 : 3) : 5; // knots per CTA
+  static constexpr size_t raw = sizeof(typename KindTraits<KIND>::template EvalWs<DERIV>);
   static constexpr size_t slice = (raw + 15) / 16 * 16;
   static_assert(G * slice <= 232448, "evaluation groups exceed the 227 KB opt-in shared memory");
 };
-template <int KIND, bool DERIV> __global__ void __launch_bounds__(EvalShape<KIND, DERIV>::TH * EvalShape<KIND, DERIV>::G, EvalShape<KIND, DERIV>::CTAS)
+template <int KIND, bool DERIV> __global__ void __launch_bounds__(EvalShape<KIND, DERIV>::TH * EvalShape<KIND, DERIV>::G, 1)
 k_eval(Ws w, const int32_t *list, int nitems) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int T1 = w.T + 1;
@@ -113,7 +103,6 @@ __global__ void k_cycle(Ws w, const mpc_knot_t *last) {
   for (int i = threadIdx.x; i < nd; i += blockDim.x) kn[(w.T - 1) * nd + i] = reinterpret_cast<const double *>(last + b)[i];
 }
 
-// fp64 peak micro-benchmark: 8 independent DFMA chains per thread
 // rigid-body terms of the whole-body QPs for `count` states (rbd_terms.cuh): one 128-thread CTA per state
 __global__ void __launch_bounds__(128) k_rbd_terms(const DevModel *model, const double *x, int count, double *M, double *nle, double *Jc, double *dJv, double *vf) {
   extern __shared__ double rbd_smem[];
@@ -141,6 +130,7 @@ __global__ void __launch_bounds__(128) k_feet_of_prediction(Ws w, const DevModel
   PAR_FOR(i, 12) { lf[b * 12 + i] = ws.ofoot[i]; rf[b * 12 + i] = ws.ofoot[12 + i]; }
 }
 
+// fp64 peak micro-benchmark: 8 independent DFMA chains per thread
 __global__ void k_dfma_peak(double *out, int iters) {
   double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
   const double m = 1.0000001, c = 1e-9;
@@ -181,9 +171,7 @@ struct mpc_solver {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_part[2 * 8] = {};
   double *d_k0 = nullptr; // first feedback gains, packed (mpc_run_pipelined)
   InstState *h_st = nullptr; // pinned copy of the per-instance summaries (mpc_run_pipelined)
-  size_t eval_smem = 0, eval_smem_values = 0, ric_smem = 0;
-  int eval_threads = 128, ric_threads = 256, num_sms = 148;
-  bool ric_threads_auto = true;
+  int num_sms = 148;
   int last_launches = 0;
   float last_ms = 0;
   size_t bytes = 0;
@@ -219,28 +207,25 @@ struct CudaBackend {
   void eval(bool d, const int32_t *list, int n) {
     const int nitems = n * (h->w.T + 1);
     mark(d ? 0 : 2);
-    switch (h->w.kind * 2 + (d ? 1 : 0)) {
-    case MPC_KIND_FULL * 2 + 1: launch_eval<MPC_KIND_FULL, true>(h->w, list, nitems, s); break;
-    case MPC_KIND_FULL * 2 + 0: launch_eval<MPC_KIND_FULL, false>(h->w, list, nitems, s); break;
-    case MPC_KIND_KINO * 2 + 1: launch_eval<MPC_KIND_KINO, true>(h->w, list, nitems, s); break;
-    case MPC_KIND_KINO * 2 + 0: launch_eval<MPC_KIND_KINO, false>(h->w, list, nitems, s); break;
-    case MPC_KIND_CENT * 2 + 1: launch_eval<MPC_KIND_CENT, true>(h->w, list, nitems, s); break;
-    default: launch_eval<MPC_KIND_CENT, false>(h->w, list, nitems, s); break;
-    }
+    dispatch_kind(h->w.kind, [&](auto kind) {
+      if (d) launch_eval<decltype(kind)::value, true>(h->w, list, nitems, s);
+      else launch_eval<decltype(kind)::value, false>(h->w, list, nitems, s);
+    });
   }
   void decide_eval(const int32_t *list, int n, int32_t *next_eval) { mark(3); k_decide_eval<<<n, 128, 0, s>>>(h->w, list, next_eval); }
   void riccati(const int32_t *list, int n) {
     mark(1);
-    // full dynamics: two 128-thread instances per SM when the launch fills the GPU; 256 threads per instance when SMs would idle (latency)
-    if (h->w.kind == MPC_KIND_FULL) k_riccati<MPC_KIND_FULL><<<n, (h->ric_threads_auto && n <= h->num_sms) ? 256 : h->ric_threads, h->ric_smem, s>>>(h->w, list);
-    else if (h->w.kind == MPC_KIND_KINO) k_riccati<MPC_KIND_KINO><<<n, h->ric_threads, h->ric_smem, s>>>(h->w, list);
-    else k_riccati<MPC_KIND_CENT><<<n, h->ric_threads, h->ric_smem, s>>>(h->w, list);
+    dispatch_kind(h->w.kind, [&](auto kind) {
+      using K = KindTraits<decltype(kind)::value>;
+      k_riccati<decltype(kind)::value><<<n, K::ric_threads(n, h->num_sms), K::ric_smem, s>>>(h->w, list);
+    });
   }
   void rollout_ls(const int32_t *list, int n, int32_t *next_eval) {
     mark(2);
-    if (h->w.kind == MPC_KIND_FULL) k_rollout_ls<MPC_KIND_FULL><<<n, RolloutShape<MPC_KIND_FULL>::TH, RolloutShape<MPC_KIND_FULL>::smem, s>>>(h->w, list, next_eval);
-    else if (h->w.kind == MPC_KIND_KINO) k_rollout_ls<MPC_KIND_KINO><<<n, RolloutShape<MPC_KIND_KINO>::TH, RolloutShape<MPC_KIND_KINO>::smem, s>>>(h->w, list, next_eval);
-    else k_rollout_ls<MPC_KIND_CENT><<<n, RolloutShape<MPC_KIND_CENT>::TH, RolloutShape<MPC_KIND_CENT>::smem, s>>>(h->w, list, next_eval);
+    dispatch_kind(h->w.kind, [&](auto kind) {
+      using Sh = RolloutShape<decltype(kind)::value>;
+      k_rollout_ls<decltype(kind)::value><<<n, Sh::TH, Sh::smem, s>>>(h->w, list, next_eval);
+    });
     mark(-1);
   }
   void apply_step(const int32_t *list, int n) { mark(3); k_apply_step<<<n, 128, 0, s>>>(h->w, list); }
@@ -253,24 +238,47 @@ struct CudaBackend {
   }
 };
 
+// the SM count (Riccati launch shape) and the dynamic shared memory of the handle's kernels
 static int set_kernel_attrs(mpc_solver *h) {
-  if (h->w.kind == MPC_KIND_FULL) { h->eval_smem = sizeof(FullWsT<true>); h->eval_smem_values = sizeof(FullWsT<false>); h->eval_threads = 128; h->ric_smem = RicFastLayout<56, 22, 78, FULL_NCAP>::total * 8; h->ric_threads = 128; } // two 128-thread instances per SM
-  else if (h->w.kind == MPC_KIND_KINO) { h->eval_smem = sizeof(KinoWsT<true>); h->eval_smem_values = sizeof(KinoWsT<false>); h->eval_threads = 128;
-    h->ric_smem = RicFastLayout<56, 34, 68, KINO_NCAP>::total * 8; h->ric_threads = 256; }
-  else { h->eval_smem = h->eval_smem_values = sizeof(CentWs); h->eval_threads = 32; h->ric_smem = riccati_smem_doubles<9, 12, 34>() * 8; h->ric_threads = 128; }
-  if (const char *e = getenv("MPCB200_RIC_THREADS")) { int t = atoi(e); if (t >= 32 && t <= 256 && (t >= 128 || h->w.kind == MPC_KIND_CENT)) { h->ric_threads = t; h->ric_threads_auto = false; } }
   { int dev = 0, sms = 0; if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && sms > 0) h->num_sms = sms; }
-  static_assert(RicFastLayout<56, 22, 78, FULL_NCAP>::total * 8 <= 232448 && RicFastLayout<56, 34, 68, KINO_NCAP>::total * 8 <= 232448,
-                "Riccati shared memory exceeds the 227 KB opt-in limit");
-#define EVAL_ATTR(KIND, D) CK(cudaFuncSetAttribute(k_eval<KIND, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EvalShape<KIND, D>::G * EvalShape<KIND, D>::slice)))
-  EVAL_ATTR(MPC_KIND_FULL, true); EVAL_ATTR(MPC_KIND_FULL, false); EVAL_ATTR(MPC_KIND_KINO, true); EVAL_ATTR(MPC_KIND_KINO, false);
-  EVAL_ATTR(MPC_KIND_CENT, true); EVAL_ATTR(MPC_KIND_CENT, false);
-#undef EVAL_ATTR
-  CK(cudaFuncSetAttribute(k_rollout_ls<MPC_KIND_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RolloutShape<MPC_KIND_FULL>::smem));
-  CK(cudaFuncSetAttribute(k_rollout_ls<MPC_KIND_KINO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RolloutShape<MPC_KIND_KINO>::smem));
-  CK(cudaFuncSetAttribute(k_rollout_ls<MPC_KIND_CENT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RolloutShape<MPC_KIND_CENT>::smem));
-  CK(cudaFuncSetAttribute(k_riccati<MPC_KIND_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, RicFastLayout<56, 22, 78, FULL_NCAP>::total * 8));
-  CK(cudaFuncSetAttribute(k_riccati<MPC_KIND_KINO>, cudaFuncAttributeMaxDynamicSharedMemorySize, RicFastLayout<56, 34, 68, KINO_NCAP>::total * 8));
+  return dispatch_kind(h->w.kind, [&](auto kind) {
+    constexpr int KIND = decltype(kind)::value;
+    CK(cudaFuncSetAttribute(k_eval<KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EvalShape<KIND, true>::G * EvalShape<KIND, true>::slice)));
+    CK(cudaFuncSetAttribute(k_eval<KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EvalShape<KIND, false>::G * EvalShape<KIND, false>::slice)));
+    CK(cudaFuncSetAttribute(k_rollout_ls<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RolloutShape<KIND>::smem));
+    CK(cudaFuncSetAttribute(k_riccati<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, KindTraits<KIND>::ric_smem));
+    return 0;
+  });
+}
+
+// multipliers of every instance back to zero (a fresh solver.setup())
+static int zero_multipliers(mpc_solver *h, cudaStream_t s) {
+  const Ws &w = h->w;
+  const size_t T1 = w.T + 1;
+  CK(cudaMemsetAsync(w.vs, 0, w.B * T1 * w.nc * 8, s));
+  CK(cudaMemsetAsync(w.lams, 0, w.B * T1 * w.n * 8, s));
+  return 0;
+}
+
+// upload `last` (host, [batch]) and append it to the horizon (k_cycle), on the handle's stream
+static int cycle_knots(mpc_solver *h, const mpc_knot_t *last) {
+  if (!h->d_last) CK(cudaMalloc(&h->d_last, sizeof(mpc_knot_t) * h->w.B)); // owned by the handle, released in mpc_destroy
+  CK(cudaMemcpyAsync(h->d_last, last, sizeof(mpc_knot_t) * h->w.B, cudaMemcpyHostToDevice, h->stream));
+  k_cycle<<<h->w.B, 96, 0, h->stream>>>(h->w, h->d_last);
+  return 0;
+}
+
+// device time of the last run (ev0 -> ev1, ev1 complete) and its per-category split from the marks of CudaBackend
+static int read_run_times(mpc_solver *h) {
+  CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
+  for (int c = 0; c < 4; c++) { h->cat_ms[c] = 0; h->cat_launches[c] = 0; }
+  for (size_t i = 0; i + 1 < h->evcat.size(); i++) {
+    int c = h->evcat[i];
+    if (c < 0) continue;
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, h->evpool[i], h->evpool[i + 1]));
+    h->cat_ms[c] += ms; h->cat_launches[c]++;
+  }
   return 0;
 }
 
@@ -289,18 +297,12 @@ mpc_solver_t *mpc_create(const mpc_robot_t *robot, const mpc_config_t *cfg, int3
   h->device = device;
   const char *err = nullptr;
   if (build_dev_model(robot, cfg, &h->h_model, &err)) { g_err = err; delete h; return nullptr; }
-  Ws &w = h->w;
-  std::memset(&w, 0, sizeof w);
-  w.B = batch; w.T = cfg->T; w.kind = cfg->kind;
-  dims_of_kind(cfg->kind, w.nx, w.n, w.m, w.nc);
-  w.nz = w.n + w.m;
-  w.sc = default_consts(cfg->tol, cfg->mu_init, cfg->rollout);
   // every failure below releases what was created so far through mpc_destroy (all members start null)
   auto bail = [&](const char *what, cudaError_t e) -> mpc_solver_t * { g_err = std::string(what) + ": " + cudaGetErrorString(e); mpc_destroy(h); return nullptr; };
   cudaError_t e;
   if ((e = cudaMalloc(&h->d_model, sizeof(DevModel))) != cudaSuccess) return bail("cudaMalloc(model)", e);
   if ((e = cudaMemcpy(h->d_model, &h->h_model, sizeof(DevModel), cudaMemcpyHostToDevice)) != cudaSuccess) return bail("cudaMemcpy(model)", e);
-  w.model = h->d_model;
+  init_ws(h->w, *cfg, batch, h->d_model);
   if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
   if ((e = cudaEventCreate(&h->ev0)) != cudaSuccess || (e = cudaEventCreate(&h->ev1)) != cudaSuccess) return bail("cudaEventCreate", e);
   if ((e = cudaMallocHost(&h->h_counters, 4 * sizeof(int32_t))) != cudaSuccess) return bail("cudaMallocHost", e);
@@ -351,8 +353,7 @@ int32_t mpc_setup(mpc_solver_t *h, const mpc_knot_t *knots, const mpc_term_t *te
     h->setup_done = true;
   } else {
     // solver.setup() re-creates the workspace: multipliers restart from zero (fulldynamic_talos.py:539)
-    CK(cudaMemsetAsync(w.vs, 0, w.B * T1 * w.nc * 8, h->stream));
-    CK(cudaMemsetAsync(w.lams, 0, w.B * T1 * w.n * 8, h->stream));
+    if (zero_multipliers(h, h->stream)) return 1;
   }
   CK(cudaMemcpyAsync(w.knots, knots, sizeof(mpc_knot_t) * w.B * w.T, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(w.terms, terms, sizeof(mpc_term_t) * w.B, cudaMemcpyHostToDevice, h->stream));
@@ -384,15 +385,12 @@ int32_t mpc_update_terms(mpc_solver_t *h, const mpc_term_t *terms) {
 int32_t mpc_cycle(mpc_solver_t *h, const mpc_knot_t *last) {
   CK(cudaSetDevice(h->device));
   if (!h->setup_done) return fail("mpc_cycle before mpc_setup");
-  if (!h->d_last) CK(cudaMalloc(&h->d_last, sizeof(mpc_knot_t) * h->w.B)); // owned by the handle, released in mpc_destroy
-  CK(cudaMemcpyAsync(h->d_last, last, sizeof(mpc_knot_t) * h->w.B, cudaMemcpyHostToDevice, h->stream));
-  k_cycle<<<h->w.B, 96, 0, h->stream>>>(h->w, h->d_last);
+  if (cycle_knots(h, last)) return 1;
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
-// shift the warm multipliers by `n` knots: vs[k] <- vs[k+n], lams[k] <- lams[k+n], tail zeroed
 // Warm-start shift of the multipliers by n knots (solver.cycleProblem without setup, kinodynamic_talos.py:488).  The constraint
 // multipliers of the RUNNING knots and the co-states of x_1 .. x_T move n knots to the left, the vacated slots repeat the last
 // running knot / the last co-state (as the trajectory warm start repeats its last knot); the terminal constraint's multiplier
@@ -454,20 +452,11 @@ static int run_impl(mpc_solver *h, const double *d_xs, const double *d_us, int m
   CK(cudaGetLastError());
   if (sync_events) {
     CK(cudaEventSynchronize(h->ev1));
-    CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
-    for (int c = 0; c < 4; c++) { h->cat_ms[c] = 0; h->cat_launches[c] = 0; }
-    for (size_t i = 0; i + 1 < h->evcat.size(); i++) {
-      int c = h->evcat[i];
-      if (c < 0) continue;
-      float ms = 0;
-      CK(cudaEventElapsedTime(&ms, h->evpool[i], h->evpool[i + 1]));
-      h->cat_ms[c] += ms; h->cat_launches[c]++;
-    }
+    return read_run_times(h);
   }
   return 0;
 }
 
-static int run_impl(mpc_solver *h, const double *d_xs, const double *d_us, int max_iters, cudaStream_t s, bool sync_events);
 // closed-loop warm start (fulldynamic_talos.py:532-536): xs <- xs[1:] + [xs[-1]], us <- us[1:] + [us[-1]], x0 <- measured state
 // (x_meas, or the model prediction xs[1] when x_meas == nullptr: ideal plant)
 // tail_mode 0: the reference scripts' warm start, us = us[1:] + [us[-1]] (fulldynamic_talos.py:534): the appended knot starts from the previous knot's control.
@@ -502,12 +491,7 @@ int32_t mpc_tick(mpc_solver_t *h, const mpc_knot_t *last, const double *x_meas, 
   CK(cudaSetDevice(h->device));
   if (!h->setup_done) return fail("mpc_tick before mpc_setup");
   Ws &w = h->w;
-  const size_t T1 = w.T + 1;
-  if (last) {
-    if (!h->d_last) CK(cudaMalloc(&h->d_last, sizeof(mpc_knot_t) * w.B));
-    CK(cudaMemcpyAsync(h->d_last, last, sizeof(mpc_knot_t) * w.B, cudaMemcpyHostToDevice, h->stream));
-    k_cycle<<<w.B, 96, 0, h->stream>>>(w, h->d_last);
-  }
+  if (last && cycle_knots(h, last)) return 1;
   double *d_meas = nullptr;
   if (x_meas) {
     if (!h->d_meas) CK(cudaMalloc(&h->d_meas, (size_t)w.B * w.nx * 8));
@@ -516,10 +500,7 @@ int32_t mpc_tick(mpc_solver_t *h, const mpc_knot_t *last, const double *x_meas, 
   }
   k_shift_warmstart<<<w.B, 128, 0, h->stream>>>(w, h->d_xs_in, h->d_us_in, d_meas, h->tail_mode);
   if (keep_multipliers) k_shift_multipliers<<<w.B, 128, 0, h->stream>>>(w, 1);
-  else {
-    CK(cudaMemsetAsync(w.vs, 0, w.B * T1 * w.nc * 8, h->stream));
-    CK(cudaMemsetAsync(w.lams, 0, w.B * T1 * w.n * 8, h->stream));
-  }
+  else if (zero_multipliers(h, h->stream)) return 1;
   CK(cudaGetLastError());
   return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream, true);
 }
@@ -534,12 +515,7 @@ int32_t mpc_set_tail_warmstart(mpc_solver_t *h, int32_t mode) {
 int32_t mpc_reset_multipliers(mpc_solver_t *h, uint64_t stream) {
   CK(cudaSetDevice(h->device));
   if (!h->setup_done) return fail("mpc_reset_multipliers before mpc_setup");
-  Ws &w = h->w;
-  const size_t T1 = w.T + 1;
-  cudaStream_t s = stream ? reinterpret_cast<cudaStream_t>(stream) : h->stream;
-  CK(cudaMemsetAsync(w.vs, 0, w.B * T1 * w.nc * 8, s));
-  CK(cudaMemsetAsync(w.lams, 0, w.B * T1 * w.n * 8, s));
-  return 0;
+  return zero_multipliers(h, stream ? reinterpret_cast<cudaStream_t>(stream) : h->stream);
 }
 
 int32_t mpc_run(mpc_solver_t *h, const double *xs_init, const double *us_init, int32_t max_iters) {
@@ -552,10 +528,16 @@ int32_t mpc_run(mpc_solver_t *h, const double *xs_init, const double *us_init, i
   return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream, true);
 }
 
-// first feedback gain of the instances [first, first + gridDim.x), packed [instance][m][n]
-__global__ void k_pack_k0_part(Ws w, double *K0, int first) {
+// pack what the MPC loop consumes (fulldynamic_talos.py:548-550) of the instances [first, first + gridDim.x): the first feedback
+// gain into K0 [instance][m][n] and the summary into info [instance][8] (either may be null)
+__global__ void k_pack_k0_info(Ws w, double *K0, double *info, int first) {
   const size_t b = first + blockIdx.x, sz = (size_t)w.m * w.n;
-  for (size_t i = threadIdx.x; i < sz; i += blockDim.x) K0[b * sz + i] = w.Kfb[b * (size_t)w.T * sz + i];
+  if (K0) for (size_t i = threadIdx.x; i < sz; i += blockDim.x) K0[b * sz + i] = w.Kfb[b * (size_t)w.T * sz + i];
+  if (info && threadIdx.x == 0) {
+    const InstState &t = w.st[b];
+    double *o = info + b * 8;
+    o[0] = t.prim_infeas; o[1] = t.dual_infeas; o[2] = t.traj_cost; o[3] = t.merit; o[4] = (double)t.num_iters; o[5] = (double)t.conv; o[6] = (double)t.status; o[7] = t.alpha;
+  }
 }
 
 int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *us_init, int32_t max_iters, int32_t parts, double *xs_out,
@@ -598,7 +580,7 @@ int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *
     if (xs_out) CK(cudaMemcpyAsync(xs_out + (size_t)o * sx, w.xs + (size_t)o * sx, (size_t)n * sx * 8, cudaMemcpyDeviceToHost, sc));
     if (us_out) CK(cudaMemcpyAsync(us_out + (size_t)o * su, w.us + (size_t)o * su, (size_t)n * su * 8, cudaMemcpyDeviceToHost, sc));
     if (K0_out) {
-      k_pack_k0_part<<<n, 128, 0, sc>>>(w, h->d_k0, o);
+      k_pack_k0_info<<<n, 128, 0, sc>>>(w, h->d_k0, nullptr, o);
       CK(cudaMemcpyAsync(K0_out + (size_t)o * sk, h->d_k0 + (size_t)o * sk, (size_t)n * sk * 8, cudaMemcpyDeviceToHost, sc));
     }
     if (info_out) CK(cudaMemcpyAsync(h->h_st + o, w.st + o, sizeof(InstState) * n, cudaMemcpyDeviceToHost, sc));
@@ -608,22 +590,9 @@ int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *
   CK(cudaStreamSynchronize(sc));
   CK(cudaEventSynchronize(h->ev1));
   h->last_launches = launches;
-  CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
-  for (int c = 0; c < 4; c++) { h->cat_ms[c] = 0; h->cat_launches[c] = 0; }
-  for (size_t i = 0; i + 1 < h->evcat.size(); i++) {
-    int c = h->evcat[i];
-    if (c < 0) continue;
-    float ms = 0;
-    CK(cudaEventElapsedTime(&ms, h->evpool[i], h->evpool[i + 1]));
-    h->cat_ms[c] += ms; h->cat_launches[c]++;
-  }
+  if (read_run_times(h)) return 1;
   if (info_out)
-    for (int b = 0; b < w.B; b++) {
-      const InstState &t = h->h_st[b];
-      info_out[b].prim_infeas = t.prim_infeas; info_out[b].dual_infeas = t.dual_infeas; info_out[b].traj_cost = t.traj_cost; info_out[b].merit = t.merit;
-      info_out[b].mu = t.mu; info_out[b].alpha = t.alpha; info_out[b].ls_evals = t.ls_evals; info_out[b].pad_ = 0; info_out[b].num_iters = t.num_iters;
-      info_out[b].al_iters = t.al_iters; info_out[b].conv = t.conv; info_out[b].status = t.status;
-    }
+    for (int b = 0; b < w.B; b++) info_out[b] = info_of(h->h_st[b]);
   return 0;
 }
 
@@ -648,11 +617,7 @@ int32_t mpc_get_results(mpc_solver_t *h, double *xs, double *us, double *K, doub
   if (info) { st.resize(w.B); CK(cudaMemcpyAsync(st.data(), w.st, sizeof(InstState) * w.B, cudaMemcpyDeviceToHost, s)); }
   CK(cudaStreamSynchronize(s));
   if (info)
-    for (int b = 0; b < w.B; b++) {
-      const InstState &t = st[b];
-      info[b].prim_infeas = t.prim_infeas; info[b].dual_infeas = t.dual_infeas; info[b].traj_cost = t.traj_cost; info[b].merit = t.merit;
-      info[b].mu = t.mu; info[b].alpha = t.alpha; info[b].ls_evals = t.ls_evals; info[b].pad_ = 0; info[b].num_iters = t.num_iters; info[b].al_iters = t.al_iters; info[b].conv = t.conv; info[b].status = t.status;
-    }
+    for (int b = 0; b < w.B; b++) info[b] = info_of(st[b]);
   return 0;
 }
 
@@ -665,17 +630,7 @@ int32_t mpc_result_ptrs(mpc_solver_t *h, uint64_t *xs, uint64_t *us, uint64_t *K
   return 0;
 }
 
-// pack what the MPC loop consumes (fulldynamic_talos.py:548-550) for a gather over NVLink: xs, us, K0 and the per-instance summary
-__global__ void k_pack_k0_info(Ws w, double *K0, double *info) {
-  const size_t b = blockIdx.x, sz = (size_t)w.m * w.n;
-  if (K0) for (size_t i = threadIdx.x; i < sz; i += blockDim.x) K0[b * sz + i] = w.Kfb[b * (size_t)w.T * sz + i];
-  if (info && threadIdx.x == 0) {
-    const InstState &t = w.st[b];
-    double *o = info + b * 8;
-    o[0] = t.prim_infeas; o[1] = t.dual_infeas; o[2] = t.traj_cost; o[3] = t.merit; o[4] = (double)t.num_iters; o[5] = (double)t.conv; o[6] = (double)t.status; o[7] = t.alpha;
-  }
-}
-
+// xs, us, K0 and the per-instance summary into device buffers, e.g. for a gather over NVLink
 int32_t mpc_export_results_device(mpc_solver_t *h, uint64_t xs_dev, uint64_t us_dev, uint64_t K0_dev, uint64_t info_dev, uint64_t stream) {
   CK(cudaSetDevice(h->device));
   if (!h->setup_done) return fail("mpc_export_results_device before mpc_setup");
@@ -684,7 +639,7 @@ int32_t mpc_export_results_device(mpc_solver_t *h, uint64_t xs_dev, uint64_t us_
   if (xs_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(xs_dev), w.xs, (size_t)w.B * (w.T + 1) * w.nx * 8, cudaMemcpyDeviceToDevice, s));
   if (us_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(us_dev), w.us, (size_t)w.B * w.T * w.m * 8, cudaMemcpyDeviceToDevice, s));
   if (K0_dev || info_dev) {
-    k_pack_k0_info<<<w.B, 128, 0, s>>>(w, reinterpret_cast<double *>(K0_dev), reinterpret_cast<double *>(info_dev));
+    k_pack_k0_info<<<w.B, 128, 0, s>>>(w, reinterpret_cast<double *>(K0_dev), reinterpret_cast<double *>(info_dev), 0);
     CK(cudaGetLastError());
   }
   return 0;
@@ -696,8 +651,7 @@ int32_t mpc_get_stage_data(mpc_solver_t *h, int32_t k, double *xdot, double *con
   Ws &w = h->w;
   if (k < 0 || k >= w.T) return fail("stage index out of range");
   const size_t T1 = w.T + 1;
-  const int nd = (w.kind == MPC_KIND_CENT) ? 9 : 56;
-  if (xdot) CK(cudaMemcpy2D(xdot, nd * 8, w.xdot + (size_t)k * 56, T1 * 56 * 8, nd * 8, w.B, cudaMemcpyDeviceToHost));
+  if (xdot) CK(cudaMemcpy2D(xdot, w.n * 8, w.xdot + (size_t)k * 56, T1 * 56 * 8, w.n * 8, w.B, cudaMemcpyDeviceToHost));
   if (contact_force) CK(cudaMemcpy2D(contact_force, 12 * 8, w.lamc + (size_t)k * 12, T1 * 12 * 8, 12 * 8, w.B, cudaMemcpyDeviceToHost));
   return 0;
 }
@@ -776,53 +730,34 @@ int32_t mpc_debug_gemm_tn(int32_t mt, int32_t nt, int32_t K, const double *A, in
   return 0;
 }
 
-double mpc_measure_fp64_peak(int32_t device) {
+// TFLOP/s of a peak kernel: 8 CTAs of 256 threads per SM, one warm-up launch of warm_iters, best of five timed launches of iters
+// (flop_per_thread: FLOP per thread and iteration)
+static double time_peak(int device, void (*kernel)(double *, int), int warm_iters, int iters, double flop_per_thread) {
   if (cudaSetDevice(device) != cudaSuccess) { g_err = "no CUDA device"; return -1.0; }
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, device);
-  const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 16;
+  const int blocks = prop.multiProcessorCount * 8, threads = 256;
   double *out = nullptr;
   if (cudaMalloc(&out, (size_t)blocks * threads * 8) != cudaSuccess) return -1.0;
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0); cudaEventCreate(&e1);
-  k_dfma_peak<<<blocks, threads>>>(out, 1024);
+  kernel<<<blocks, threads>>>(out, warm_iters);
   float best = 1e30f;
   for (int rep = 0; rep < 5; rep++) {
     cudaEventRecord(e0);
-    k_dfma_peak<<<blocks, threads>>>(out, iters);
+    kernel<<<blocks, threads>>>(out, iters);
     cudaEventRecord(e1);
     cudaEventSynchronize(e1);
     float ms; cudaEventElapsedTime(&ms, e0, e1);
     if (ms < best) best = ms;
   }
   cudaFree(out); cudaEventDestroy(e0); cudaEventDestroy(e1);
-  double flops = 2.0 * 8.0 * (double)iters * blocks * threads;
+  double flops = flop_per_thread * (double)iters * blocks * threads;
   return flops / (best * 1e-3) / 1e12;
 }
 
-double mpc_measure_fp64_peak_dmma(int32_t device) {
-  if (cudaSetDevice(device) != cudaSuccess) { g_err = "no CUDA device"; return -1.0; }
-  cudaDeviceProp prop;
-  cudaGetDeviceProperties(&prop, device);
-  const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 14;
-  double *out = nullptr;
-  if (cudaMalloc(&out, (size_t)blocks * threads * 8) != cudaSuccess) return -1.0;
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
-  k_dmma_peak<<<blocks, threads>>>(out, 256);
-  float best = 1e30f;
-  for (int rep = 0; rep < 5; rep++) {
-    cudaEventRecord(e0);
-    k_dmma_peak<<<blocks, threads>>>(out, iters);
-    cudaEventRecord(e1);
-    cudaEventSynchronize(e1);
-    float ms; cudaEventElapsedTime(&ms, e0, e1);
-    if (ms < best) best = ms;
-  }
-  cudaFree(out); cudaEventDestroy(e0); cudaEventDestroy(e1);
-  double flops = 512.0 * 8.0 * (double)iters * blocks * (threads / 32);
-  return flops / (best * 1e-3) / 1e12;
-}
+double mpc_measure_fp64_peak(int32_t device) { return time_peak(device, k_dfma_peak, 1024, 1 << 16, 2.0 * 8); }
+double mpc_measure_fp64_peak_dmma(int32_t device) { return time_peak(device, k_dmma_peak, 256, 1 << 14, 512.0 * 8 / 32); }
 
 // ---- rigid-body terms in front of the whole-body QPs (include/mpcb200.h)
 int32_t mpc_rbd_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, uint64_t M_dev, uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t vf_dev,
@@ -883,11 +818,7 @@ int32_t mpc_gait_setup(mpc_solver_t *h, const mpc_gait_t *gait, const int32_t *m
     g.urefs = h->d_gait_urefs;
   }
   CK(cudaMemcpy(h->d_gait, &g, sizeof g, cudaMemcpyHostToDevice));
-  std::vector<GaitRobot> rs(w.B);
-  for (int b = 0; b < w.B; b++) {
-    for (int i = 0; i < 12; i++) { rs[b].start_l[i] = rs[b].final_l[i] = rs[b].next_l[i] = gait->lf0[i]; rs[b].start_r[i] = rs[b].final_r[i] = rs[b].next_r[i] = gait->rf0[i]; }
-    rs[b].mirror = mirror ? (mirror[b] != 0) : 0; rs[b].pad_ = 0;
-  }
+  const std::vector<GaitRobot> rs = gait_init_robots(*gait, w.B, mirror);
   CK(cudaMemcpy(h->d_gait_robots, rs.data(), sizeof(GaitRobot) * w.B, cudaMemcpyHostToDevice));
   h->gait_t = 0;
   h->gait_ready = true;

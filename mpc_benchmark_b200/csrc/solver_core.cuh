@@ -16,8 +16,6 @@
 namespace mpcdev {
 
 enum { MODE_EVAL = 0, MODE_STEP = 1, MODE_LS = 2, MODE_DONE = 3 };
-constexpr int KINO_NCAP = 54; // active rows of the kinodynamic Riccati's shared-memory carving; knots with more (up to all 68) solve their KKT out of global scratch
-constexpr int FULL_NCAP = 23; // full dynamics: what fits over the dead P | G buffers (two instances per SM)
 
 struct SolverConst {
   double tol, mu_init;
@@ -264,22 +262,52 @@ HD void decide_ls(const Ws &w, int b, double *red, int32_t *ls_out, int32_t *nex
   }
 }
 
-// ---- one (instance, knot) evaluation; KIND is a compile-time parameter so every model gets its own kernel (registers,
-// shared memory and spills of one stage type do not tax the others).  smem: FullWsT / KinoWsT / CentWs storage.
+// ---- what differs between the model kinds: dimensions, the evaluation workspace and stage functions, the Riccati solver and
+// its launch shape.  KIND is a compile-time parameter so every model gets its own kernels (registers, shared memory and spills
+// of one stage type do not tax the others); the host turns the runtime kind into KIND with dispatch_kind (driver.hpp).
+template <int KIND> struct KindTraits;
+template <> struct KindTraits<MPC_KIND_FULL> {
+  static constexpr int nx = 57, n = 56, m = 22, nc = 78;
+  static constexpr int ncap = 23; // active rows of the Riccati's shared-memory carving: what fits over the dead P | G buffers (two instances per SM)
+  template <bool D> using EvalWs = FullWsT<D>;
+  template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_full_knot<D, ROLL>(md, io, f); }
+  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_full_term<D>(md, io, f); }
+  static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
+  static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
+  // two 128-thread instances per SM when the launch fills the GPU; 256 threads per instance when SMs would idle (latency)
+  static constexpr int ric_threads(int count, int num_sms) { return count <= num_sms ? 256 : 128; }
+};
+template <> struct KindTraits<MPC_KIND_KINO> {
+  static constexpr int nx = 57, n = 56, m = 34, nc = 68;
+  static constexpr int ncap = 54; // knots with more active rows (up to all 68) solve their KKT out of global scratch
+  template <bool D> using EvalWs = KinoWsT<D>;
+  template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_kino_knot<D, ROLL>(md, io, f); }
+  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_kino_term<D>(md, io, f); }
+  static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
+  static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
+  static constexpr int ric_threads(int, int) { return 256; }
+};
+template <> struct KindTraits<MPC_KIND_CENT> {
+  static constexpr int nx = 9, n = 9, m = 12, nc = 34;
+  static constexpr int ncap = nc; // the generic Riccati kernel holds every row in shared memory
+  template <bool D> using EvalWs = CentWs;
+  template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_knot<D, ROLL>(md, io, f); }
+  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_term<D>(md, io, f); }
+  static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, false>(r, smem); }
+  static constexpr int ric_smem = riccati_smem_doubles<n, m, nc>() * 8, ric_scratch = 2; // no global scratch: a token block
+  static constexpr int ric_threads(int, int) { return 128; }
+};
+static_assert(KindTraits<MPC_KIND_FULL>::ric_smem <= 232448 && KindTraits<MPC_KIND_KINO>::ric_smem <= 232448 && KindTraits<MPC_KIND_CENT>::ric_smem <= 232448,
+              "Riccati shared memory exceeds the 227 KB opt-in limit");
+
+// ---- one (instance, knot) evaluation.  smem: KindTraits<KIND>::EvalWs<DERIV> storage.
 template <int KIND, bool DERIV> HD void eval_dispatch(const Ws &w, int b, int k, void *smem) {
+  using K = KindTraits<KIND>;
   const int mode = w.st[b].mode;
   if (mode != (DERIV ? MODE_EVAL : MODE_LS)) return;
   KnotIO io = make_io(w, b, k, !DERIV);
-  if (KIND == MPC_KIND_FULL) {
-    FullWsT<DERIV> &f = *reinterpret_cast<FullWsT<DERIV> *>(smem);
-    if (k < w.T) eval_full_knot<DERIV>(*w.model, io, f); else eval_full_term<DERIV>(*w.model, io, f);
-  } else if (KIND == MPC_KIND_KINO) {
-    KinoWsT<DERIV> &f = *reinterpret_cast<KinoWsT<DERIV> *>(smem);
-    if (k < w.T) eval_kino_knot<DERIV>(*w.model, io, f); else eval_kino_term<DERIV>(*w.model, io, f);
-  } else {
-    CentWs &c = *reinterpret_cast<CentWs *>(smem);
-    if (k < w.T) eval_cent_knot<DERIV>(*w.model, io, c); else eval_cent_term<DERIV>(*w.model, io, c);
-  }
+  auto &f = *reinterpret_cast<typename K::template EvalWs<DERIV> *>(smem);
+  if (k < w.T) K::template knot<DERIV>(*w.model, io, f); else K::template term<DERIV>(*w.model, io, f);
 }
 
 // ---- ROLLOUT_NONLINEAR: one trial point of the fused rollout + linesearch kernel (one CTA = one evaluation group per instance).
@@ -289,6 +317,8 @@ template <int KIND, bool DERIV> HD void eval_dispatch(const Ws &w, int b, int k,
 // and every knot's merit terms land in tscal exactly as in a linear-rollout trial, so decide_ls applies unchanged.
 // xv: >= 64 + 96 + 64 doubles of shared memory next to the evaluation workspace.
 template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void *smem, double *xv) {
+  using K = KindTraits<KIND>;
+  auto &f = *reinterpret_cast<typename K::template EvalWs<false> *>(smem);
   const size_t T1 = (size_t)w.T + 1;
   const int n = w.n, m = w.m, nc = w.nc, nz = w.nz, nx = w.nx, NRk = 1 + n, S = m + nc, T = w.T;
   const int ldw = (KIND == MPC_KIND_CENT) ? nz : ((nz + 7) & ~7);
@@ -330,9 +360,7 @@ template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void
       }
       SYNC();
       KnotIO io = make_io(w, b, k, true);
-      if (KIND == MPC_KIND_FULL) eval_full_term<false>(*w.model, io, *reinterpret_cast<FullWsT<false> *>(smem));
-      else if (KIND == MPC_KIND_KINO) eval_kino_term<false>(*w.model, io, *reinterpret_cast<KinoWsT<false> *>(smem));
-      else eval_cent_term<false>(*w.model, io, *reinterpret_cast<CentWs *>(smem));
+      K::template term<false>(*w.model, io, f);
       SYNC();
       break;
     }
@@ -358,9 +386,7 @@ template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void
     SYNC();
     KnotIO io = make_io(w, b, k, true);
     io.xn = io.x; io.slack = slack; io.xn_out = txs + (size_t)(k + 1) * nx;
-    if (KIND == MPC_KIND_FULL) eval_full_knot<false, true>(*w.model, io, *reinterpret_cast<FullWsT<false> *>(smem));
-    else if (KIND == MPC_KIND_KINO) eval_kino_knot<false, true>(*w.model, io, *reinterpret_cast<KinoWsT<false> *>(smem));
-    else eval_cent_knot<false, true>(*w.model, io, *reinterpret_cast<CentWs *>(smem));
+    K::template knot<false, true>(*w.model, io, f);
     SYNC();
   }
 }
@@ -396,10 +422,7 @@ HD RiccatiIO make_riccati_io(const Ws &w, int b) {
 
 template <int KIND> HD void riccati_dispatch(const Ws &w, int b, double *smem) {
   if (w.st[b].mode != MODE_STEP) return;
-  RiccatiIO r = make_riccati_io(w, b);
-  if (KIND == MPC_KIND_FULL) riccati_instance_fast<56, 22, 78, FULL_NCAP>(r, smem);
-  else if (KIND == MPC_KIND_KINO) riccati_instance_fast<56, 34, 68, KINO_NCAP>(r, smem);
-  else riccati_instance<9, 12, 34, false>(r, smem);
+  KindTraits<KIND>::riccati(make_riccati_io(w, b), smem);
   ONE_THREAD { if (w.overflow[b]) { w.st[b].status = 3; w.st[b].mode = MODE_DONE; w.overflow[b] = 0; } }
   SYNC();
   start_linesearch(w, b);

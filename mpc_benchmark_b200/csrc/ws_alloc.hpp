@@ -1,15 +1,28 @@
 // Workspace layout of one solver handle: every array is [batch][knot][...] row-major fp64 in HBM
 // (results layout of SURVEY 8b: xs [B,T+1,nx], us [B,T,nu], K [B,T,nu,ndx]).
 #pragma once
-#include "solver_core.cuh"
+#include "driver.hpp"
 #include <cstddef>
+#include <cstring>
 
 namespace mpcdev {
 
+// state, tangent, control and constraint dimensions of a model kind (KindTraits)
 inline void dims_of_kind(int kind, int &nx, int &n, int &m, int &nc) {
-  if (kind == MPC_KIND_CENT) { nx = 9; n = 9; m = 12; nc = 34; }
-  else if (kind == MPC_KIND_KINO) { nx = 57; n = 56; m = 34; nc = 68; }
-  else { nx = 57; n = 56; m = 22; nc = 78; }
+  dispatch_kind(kind, [&](auto k) {
+    using K = KindTraits<decltype(k)::value>;
+    nx = K::nx; n = K::n; m = K::m; nc = K::nc;
+  });
+}
+
+// shape and solver constants of a workspace for `batch` instances of cfg's model kind; every array pointer starts null (alloc_ws)
+inline void init_ws(Ws &w, const mpc_config_t &cfg, int batch, const DevModel *model) {
+  std::memset(&w, 0, sizeof w);
+  w.B = batch; w.T = cfg.T; w.kind = cfg.kind;
+  dims_of_kind(cfg.kind, w.nx, w.n, w.m, w.nc);
+  w.nz = w.n + w.m;
+  w.model = model;
+  w.sc = default_consts(cfg.tol, cfg.mu_init, cfg.rollout);
 }
 
 // alloc(bytes) must return zero-initialised memory
@@ -33,7 +46,7 @@ template <class Alloc> size_t alloc_ws(Ws &w, Alloc &&alloc) {
   D(w.gap, B * T * n); D(w.h, B * T1 * nc); D(w.scal, B * T1 * SC_COUNT); D(w.tscal, B * T1 * SC_COUNT);
   D(w.xdot, B * T1 * 56); D(w.lamc, B * T1 * 12);
   D(w.W, B * T * n * ((nz + 7) & ~(size_t)7)); D(w.pt, B * T * n); D(w.K, B * T * (m + nc) * (1 + n)); D(w.Kfb, B * T * m * n); D(w.dphi, B); D(w.phase, 64);
-  w.ric_scratch_stride = (w.kind == MPC_KIND_FULL) ? RicFastLayout<56, 22, 78, FULL_NCAP>::scratch : (w.kind == MPC_KIND_KINO) ? RicFastLayout<56, 34, 68, KINO_NCAP>::scratch : 2;
+  w.ric_scratch_stride = dispatch_kind(w.kind, [](auto kind) { return KindTraits<decltype(kind)::value>::ric_scratch; });
   D(w.ric_scratch, B * w.ric_scratch_stride);
   w.st = (InstState *)alloc(B * sizeof(InstState)); total += B * sizeof(InstState);
   I(w.counters, 4); I(w.lists, 4 * B); I(w.overflow, B);

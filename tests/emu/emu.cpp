@@ -7,7 +7,6 @@
 #include "../../mpc_benchmark_b200/csrc/qp.cuh"
 #include "../../mpc_benchmark_b200/csrc/rbd_terms.cuh"
 #include "../../mpc_benchmark_b200/csrc/gait_host.hpp"
-#include <cstdlib>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -21,25 +20,17 @@ struct EmuBackend {
   EmuBackend() : smem(40000, 0.0) {}
   void reset_counters() { for (int i = 0; i < 4; i++) w.counters[i] = 0; }
   void eval(bool d, const int32_t *list, int n) {
-    for (int i = 0; i < n; i++)
-      for (int k = 0; k <= w.T; k++) {
-        switch (w.kind * 2 + (d ? 1 : 0)) {
-        case MPC_KIND_FULL * 2 + 1: eval_dispatch<MPC_KIND_FULL, true>(w, list[i], k, smem.data()); break;
-        case MPC_KIND_FULL * 2 + 0: eval_dispatch<MPC_KIND_FULL, false>(w, list[i], k, smem.data()); break;
-        case MPC_KIND_KINO * 2 + 1: eval_dispatch<MPC_KIND_KINO, true>(w, list[i], k, smem.data()); break;
-        case MPC_KIND_KINO * 2 + 0: eval_dispatch<MPC_KIND_KINO, false>(w, list[i], k, smem.data()); break;
-        case MPC_KIND_CENT * 2 + 1: eval_dispatch<MPC_KIND_CENT, true>(w, list[i], k, smem.data()); break;
-        default: eval_dispatch<MPC_KIND_CENT, false>(w, list[i], k, smem.data()); break;
+    dispatch_kind(w.kind, [&](auto kind) {
+      for (int i = 0; i < n; i++)
+        for (int k = 0; k <= w.T; k++) {
+          if (d) eval_dispatch<decltype(kind)::value, true>(w, list[i], k, smem.data());
+          else eval_dispatch<decltype(kind)::value, false>(w, list[i], k, smem.data());
         }
-      }
+    });
   }
   void decide_eval(const int32_t *list, int n, int32_t *next_eval) { double red[8]; for (int i = 0; i < n; i++) mpcdev::decide_eval(w, list[i], red, next_eval); }
   void riccati(const int32_t *list, int n) {
-    for (int i = 0; i < n; i++) {
-      if (w.kind == MPC_KIND_FULL) riccati_dispatch<MPC_KIND_FULL>(w, list[i], smem.data());
-      else if (w.kind == MPC_KIND_KINO) riccati_dispatch<MPC_KIND_KINO>(w, list[i], smem.data());
-      else riccati_dispatch<MPC_KIND_CENT>(w, list[i], smem.data());
-    }
+    dispatch_kind(w.kind, [&](auto kind) { for (int i = 0; i < n; i++) riccati_dispatch<decltype(kind)::value>(w, list[i], smem.data()); });
   }
   void apply_step(const int32_t *list, int n) { w.counters[0] = 0; for (int i = 0; i < n; i++) mpcdev::apply_step(w, list[i]); }
   void decide_ls(const int32_t *list, int n, int32_t *ls_out, int32_t *next_eval) {
@@ -48,11 +39,7 @@ struct EmuBackend {
   }
   void rollout_ls(const int32_t *list, int n, int32_t *next_eval) {
     double red[8], xv[256];
-    for (int i = 0; i < n; i++) {
-      if (w.kind == MPC_KIND_FULL) rollout_linesearch<MPC_KIND_FULL>(w, list[i], smem.data(), xv, red, next_eval);
-      else if (w.kind == MPC_KIND_KINO) rollout_linesearch<MPC_KIND_KINO>(w, list[i], smem.data(), xv, red, next_eval);
-      else rollout_linesearch<MPC_KIND_CENT>(w, list[i], smem.data(), xv, red, next_eval);
-    }
+    dispatch_kind(w.kind, [&](auto kind) { for (int i = 0; i < n; i++) rollout_linesearch<decltype(kind)::value>(w, list[i], smem.data(), xv, red, next_eval); });
   }
   void read_counters(int *c) { for (int i = 0; i < 4; i++) c[i] = w.counters[i]; }
 };
@@ -66,10 +53,7 @@ extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, int bat
   if (build_dev_model(rb, cfg, model, &err)) return 1;
   EmuBackend be;
   Ws &w = be.w;
-  std::memset(&w, 0, sizeof w);
-  w.B = batch; w.T = cfg->T; w.kind = cfg->kind;
-  dims_of_kind(cfg->kind, w.nx, w.n, w.m, w.nc);
-  w.nz = w.n + w.m; w.model = model; w.sc = default_consts(cfg->tol, cfg->mu_init, cfg->rollout);
+  init_ws(w, *cfg, batch, model);
   std::vector<void *> allocs;
   alloc_ws(w, [&](size_t bytes) { void *p = calloc(bytes ? bytes : 8, 1); allocs.push_back(p); return p; });
   const size_t T1 = w.T + 1;
@@ -95,9 +79,7 @@ extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, int bat
   if (vs) std::memcpy(vs, w.vs, 8 * batch * T1 * w.nc);
   if (lams) std::memcpy(lams, w.lams, 8 * batch * T1 * w.n);
   for (int b = 0; b < batch; b++) {
-    const InstState &s = w.st[b];
-    if (info) { mpc_info_t &o = info[b]; o.prim_infeas = s.prim_infeas; o.dual_infeas = s.dual_infeas; o.traj_cost = s.traj_cost; o.merit = s.merit; o.mu = s.mu; o.alpha = s.alpha; o.ls_evals = s.ls_evals; o.pad_ = 0;
-      o.num_iters = s.num_iters; o.al_iters = s.al_iters; o.conv = s.conv; o.status = s.status; }
+    if (info) info[b] = info_of(w.st[b]);
     if (stage0) { std::memcpy(stage0 + b * 68, w.xdot + b * T1 * 56, 8 * 56); std::memcpy(stage0 + b * 68 + 56, w.lamc + b * T1 * 12, 8 * 12); }
   }
   for (void *p : allocs) free(p);
@@ -148,11 +130,7 @@ extern "C" int emu_gait(int kind, int T, const mpc_gait_t *gait, int batch, cons
   gait_build_schedule(*gait, T, phases, g);
   g.phases = phases.data();
   g.urefs = urefs;
-  std::vector<GaitRobot> rs(batch);
-  for (int b = 0; b < batch; b++) {
-    for (int i = 0; i < 12; i++) { rs[b].start_l[i] = rs[b].final_l[i] = rs[b].next_l[i] = gait->lf0[i]; rs[b].start_r[i] = rs[b].final_r[i] = rs[b].next_r[i] = gait->rf0[i]; }
-    rs[b].mirror = mirror[b] != 0; rs[b].pad_ = 0;
-  }
+  std::vector<GaitRobot> rs = gait_init_robots(*gait, batch, mirror);
   double sm[16];
   for (int t = 0; t < ticks; t++)
     for (int b = 0; b < batch; b++)

@@ -1,5 +1,4 @@
-"""Warm single-instance centroidal MPC tick latency and its per-category kernel time (GPU box).  MPCB200_RIC_THREADS=32|64|128 selects
-the thread count of the generic Riccati kernel.  usage: python tools/cent_latency.py"""
+"""Warm single-instance centroidal MPC tick latency and its per-category kernel time (GPU box).  usage: python tools/cent_latency.py"""
 import os
 import sys
 import time
@@ -20,4 +19,4 @@ for _ in range(60):
     s.reset_multipliers()
     s.run(warm.xs, warm.us, max_iters=1, gains=False)
     ts.append(1e3 * (time.perf_counter() - t0))
-print("threads", os.environ.get("MPCB200_RIC_THREADS", "default"), "p50 ms", float(np.percentile(ts[5:], 50)), "kernel ms", s.kernel_ms(), "launches", s.last_launches)
+print("p50 ms", float(np.percentile(ts[5:], 50)), "kernel ms", s.kernel_ms(), "launches", s.last_launches)

@@ -18,7 +18,7 @@ def run(name, prob, iters):
 
 
 def main():
-    # MPCB200_RIC_THREADS=128 in the environment forces the two-instances-per-SM launch shape of the full-dynamics Riccati kernel
+    # batch 2 launches the full-dynamics Riccati kernel with 256 threads per instance; batches above the SM count use 128
     run("full walk", problems.full_walk_batch(2, seed=3, T=12), 3)
     cold = problems.full_walk_batch(2, seed=3, T=12)
     cold["x0"] = problems.perturbed_x0(cold["robot"], cold["x0"][0], __import__("numpy").random.default_rng(2), 2)  # many active rows: scratch path
