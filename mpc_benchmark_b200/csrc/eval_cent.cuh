@@ -5,7 +5,7 @@
 // and the CentroidalWrenchConeResidual constraints (centroidal_talos.py:242-245).
 //   x = [c, h_lin, h_ang], u = [f_L, tau_L, f_R, tau_R];  xdot = [h_lin/m; m g + sum f; sum (p_i - c) x f_i + tau_i]
 #pragma once
-#include "eval_full.cuh"
+#include "eval_mb.cuh"
 
 namespace mpcdev {
 

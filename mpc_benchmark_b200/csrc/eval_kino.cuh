@@ -5,9 +5,9 @@
 // FramePlacementResidual x2) and the constraints of :161-171 (joint box, CentroidalWrenchConeResidual + zero LOCAL
 // FrameVelocityResidual per active contact).  u = [w_L(6), w_R(6), a_joint(22)]; the base acceleration solves
 //   A_g[:, :6] a_b = hdot'(q, u) - F_g(q, v, [0; a_j])           (SURVEY App. A5; F_g with a_world = -g, see oracle/rbd.hpp)
-// and its derivatives reuse the world-frame tangent machinery of eval_full.cuh: d F_o / d q_j = s_j x* F_J - (Ic_J c_j + Bc_J w_j).
+// and its derivatives reuse the world-frame tangent machinery of eval_mb.cuh: d F_o / d q_j = s_j x* F_J - (Ic_J c_j + Bc_J w_j).
 #pragma once
-#include "eval_full.cuh"
+#include "eval_mb.cuh"
 
 namespace mpcdev {
 
@@ -272,59 +272,22 @@ template <bool DERIV, bool ROLL = false> HD void eval_kino_knot(const DevModel &
         else { type = 0; hv = w.vl[6 * f + rr - 17]; }
       }
     }
-    int act = 0; double prim = 0;
-    const double vp = vplus_row(type, hv, io.v_prev[r], io.mu, lo, hi, act, prim), dv = vp - io.v[r];
-    w.ctype[r] = type; w.late.hval[r] = hv; w.late.vpl[r] = vp; w.isact[r] = act;
-    w.late.dbr[r] = io.mu * dv;
-    io.h[r] = hv;
-    if (type >= 0) {
-      acc_pen += 0.5 * io.mu * (vp * vp + dv * dv);
-      acc_prim = fmax(acc_prim, fabs(prim));
-      acc_inner = fmax(acc_inner, fabs(io.mu * dv));
-    }
+    mb_row_epilogue(w, io, r, type, hv, lo, hi, io.v, io.v_prev, acc_pen, acc_prim, acc_inner);
   }
-  PAR_FOR(i, FN) {
-    const double gap = w.fbr[i], lp = io.lam_n_prev[i] + gap * rcp_(io.mu), dl = lp - io.lam_n[i]; // fbr = gap here
-    w.lpl[i] = lp;
-    w.fbr[i] = io.mu * dl;
-    acc_pen += 0.5 * io.mu * (lp * lp + dl * dl);
-    acc_prim = fmax(acc_prim, fabs(gap));
-    acc_inner = fmax(acc_inner, fabs(io.mu * dl));
-    acc_cost += 0.5 * cfg.wx[i] * w.estate[i] * w.estate[i];
-  }
+  mb_dynamics_rows(m, w, io, io.lam_n, io.lam_n_prev, acc_cost, acc_pen, acc_prim, acc_inner);
   PAR_FOR(i, KM) { const double e = w.u[i] - kn.u_ref[i]; acc_cost += 0.5 * cfg.wu[i] * e * e; }
   PAR_FOR(i, 6) {
     const double rcd = w.hd[i] + (i < 3 ? m.total_mass * rb.gravity[i] : 0.0);
     acc_cost += 0.5 * (cfg.w_cent[i] * w.rcent[i] * w.rcent[i] + kn.w_lf[i] * w.rpose[i] * w.rpose[i] + kn.w_rf[i] * w.rpose[6 + i] * w.rpose[6 + i] +
                        cfg.w_centder[i] * rcd * rcd);
   }
-  reduce_sum2_max2(acc_cost, acc_pen, acc_prim, acc_inner, w.part, w.part + 16);
-  ONE_THREAD { w.scal[SC_COST] = w.part[16]; w.scal[SC_PEN] = w.part[17]; w.scal[SC_PRIM] = w.part[18]; w.scal[SC_INNER] = w.part[19]; w.scal[SC_DUAL] = 0; }
-  compact_flags(w.isact, KNC, w.act_idx, &w.nca, reinterpret_cast<int32_t *>(w.part));
+  mb_merit_finish<KNC>(w, acc_cost, acc_pen, acc_prim, acc_inner);
   if (!DERIV) { PAR_FOR(i, SC_COUNT) io.scal[i] = w.scal[i]; return; }
 
   // ---- LQ blocks to HBM
-  PAR_FOR(i, KNC) { io.dbar[i] = w.late.dbr[i]; io.vplus[i] = w.late.vpl[i]; io.act_idx[i] = (i < w.nca) ? w.act_idx[i] : -1; }
-  PAR_FOR(i, FN) { io.fbar[i] = w.fbr[i]; io.lplus[i] = w.lpl[i]; }
-  PAR_FOR(i, 36) { io.T6[i] = w.late.T6[i]; io.E6[i] = w.late.E6[i]; }
-  ONE_THREAD io.nca[0] = w.nca;
-  const double dt2 = dt * dt;
+  mb_store_rows<KNC>(w, io);
   PAR_FOR(z, KNZ) {
-    double d6[6], acc = 0;
-    for (int k = 0; k < 6; k++) d6[k] = dt2 * w.X[k * KNZ + z] + ((z == NV + k) ? dt : 0.0);
-    for (int i = 0; i < 6; i++) {
-      double s = (z < 6) ? w.late.P2[6 * i + z] : 0.0;
-      for (int k = 0; k < 6; k++) s += w.late.P1[6 * i + k] * d6[k];
-      io.AB[i * KNZ + z] = s; acc += s * io.lam_n[i];
-    }
-    for (int i = 6; i < NV; i++) {
-      double s = dt2 * w.X[i * KNZ + z] + ((z == NV + i) ? dt : 0.0) + ((z == i) ? 1.0 : 0.0);
-      io.AB[i * KNZ + z] = s; acc += s * io.lam_n[i];
-    }
-    for (int i = 0; i < NV; i++) {
-      double s = dt * w.X[i * KNZ + z] + ((z == NV + i) ? 1.0 : 0.0);
-      io.AB[(NV + i) * KNZ + z] = s; acc += s * io.lam_n[NV + i];
-    }
+    const double acc = mb_ab_column<KNZ>(w, io, z, w.X + z, KNZ, dt, io.lam_n);
     double lz = mb_cost_grad(w, cfg.wx, cfg.w_cent, kn.w_lf, kn.w_rf, z < FN ? z : FN);
     if (z >= FN) lz = cfg.wu[z - FN] * (w.u[z - FN] - kn.u_ref[z - FN]);
     for (int r = 0; r < 6; r++) {
@@ -341,123 +304,15 @@ template <bool DERIV, bool ROLL = false> HD void eval_kino_knot(const DevModel &
     if (z < FN) { if (io.k == 0) gz += io.lam_k[z]; else if (z >= 6) gz -= io.lam_k[z]; }
     w.late.g[z] = gz; io.g[z] = gz;
   }
-  PAR_FOR(j, 6) {
-    double s = 0;
-    for (int i = 0; i < 6; i++) s += w.late.E6[6 * i + j] * io.lam_n[i];
-    io.gE_next[j] = s;
-  }
-  {
-    constexpr int HT = (KNZ + 3) / 4;
-    PAR_FOR(t, HT * HT) {
-      const int ta = t / HT, tb = t % HT;
-      if (tb < ta) continue;
-      const int a0_ = 4 * ta, b0 = 4 * tb;
-      double acc[4][4];
-#pragma unroll
-      for (int i = 0; i < 4; i++)
-#pragma unroll
-        for (int j = 0; j < 4; j++) acc[i][j] = 0.0;
-      auto rank1 = [&](const double *J, int ncols, double wgt) {
-        double va[4], vb[4];
-#pragma unroll
-        for (int i = 0; i < 4; i++) { va[i] = (a0_ + i < ncols) ? wgt * J[a0_ + i] : 0.0; vb[i] = (b0 + i < ncols) ? J[b0 + i] : 0.0; }
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-#pragma unroll
-          for (int j = 0; j < 4; j++) acc[i][j] += va[i] * vb[j];
-      };
-      for (int r = 0; r < 6; r++) if (cfg.w_centder[r] != 0.0) rank1(w.Jcd + r * KNZ, KNZ, cfg.w_centder[r]);
-      if (a0_ < FN) {
-        for (int r = 0; r < 6; r++) if (cfg.w_cent[r] != 0.0) rank1(w.cj.Jcent + r * FN, FN, cfg.w_cent[r]);
-        if (a0_ < NV && b0 < NV)
-          for (int r = 0; r < 6; r++) {
-            if (kn.w_lf[r] != 0.0) rank1(w.cj.Jpose + r * NV, NV, kn.w_lf[r]);
-            if (kn.w_rf[r] != 0.0) rank1(w.cj.Jpose + (6 + r) * NV, NV, kn.w_rf[r]);
-          }
-        if (b0 < 8 && a0_ < 8) for (int r = 0; r < 6; r++) rank1(w.Jls + 6 * r, 6, cfg.wx[r]);
-      }
-#pragma unroll
-      for (int i = 0; i < 4; i++)
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-          const int a = a0_ + i, b = b0 + j;
-          if (a >= KNZ || b >= KNZ || b < a) continue;
-          double hv = acc[i][j];
-          if (a == b) { hv += io.preg; if (a >= FN) hv += cfg.wu[a - FN]; else if (a >= 6) hv += cfg.wx[a]; }
-          io.H[a * KNZ + b] = hv; io.H[b * KNZ + a] = hv;
-        }
-    }
-  }
+  mb_gE_next(w, io, io.lam_n);
+  mb_gn_hessian<KNZ>(w, io, cfg, kn, [&](auto &rank1) { // momentum-derivative cost rows
+    for (int r = 0; r < 6; r++) if (cfg.w_centder[r] != 0.0) rank1(w.Jcd + r * KNZ, KNZ, cfg.w_centder[r]);
+  });
   PAR_FOR(e, w.nca * KNZ) {
     int ai = e / KNZ, z = e % KNZ;
     io.CDact[e] = kino_c_entry(m, w.Cvel, w.act_idx[ai], z);
   }
-  SYNC();
-  PAR_FOR(c, 8) {
-    double dual = 0;
-    for (int z = 6 + c; z < KNZ; z += 8) {
-      if (io.k == 0 && z < FN) continue;
-      dual = fmax(dual, fabs(w.late.g[z]));
-    }
-    w.part[c] = dual;
-  }
-  SYNC();
-  PAR_FOR(i, SC_COUNT) {
-    double v = w.scal[i];
-    if (i == SC_DUAL) for (int c = 0; c < 8; c++) v = fmax(v, w.part[c]);
-    io.scal[i] = v;
-  }
-}
-
-// terminal knot: empty cost (kinodynamic_talos.py:175), CoM equality (kinodynamic_talos.py:176-180,276)
-template <bool DERIV> HD void eval_kino_term(const DevModel &m, const KnotIO &io, KinoWsT<DERIV> &w) {
-  PAR_FOR(i, NQ + NV) w.x[i] = io.x[i];
-  SYNC();
-  mb_kinematics(m, w);
-  const bool has_c = io.tm->has_com_cstr != 0.0;
-  PAR_FOR(r, KNC) {
-    int type = -1; double hv = 0;
-    if (r < 3 && has_c) { type = 0; hv = w.com[r] - io.tm->com_ref[r]; }
-    int act = 0; double prim = 0;
-    double vp = vplus_row(type, hv, io.v_prev[r], io.mu, 0, 0, act, prim);
-    w.ctype[r] = type; w.late.hval[r] = hv; w.late.vpl[r] = vp; w.isact[r] = act; w.late.dbr[r] = io.mu * (vp - io.v[r]); w.late.rowtmp[r] = fabs(prim);
-    io.h[r] = hv;
-  }
-  SYNC();
-  ONE_THREAD {
-    double pen = 0, prim = 0, inner = 0;
-    int nca = 0;
-    for (int r = 0; r < 3; r++) {
-      if (w.ctype[r] < 0) continue;
-      double dv = w.late.vpl[r] - io.v[r];
-      pen += 0.5 * io.mu * (w.late.vpl[r] * w.late.vpl[r] + dv * dv);
-      prim = fmax(prim, w.late.rowtmp[r]); inner = fmax(inner, fabs(w.late.dbr[r]));
-      if (w.isact[r]) w.act_idx[nca++] = r;
-    }
-    w.nca = nca;
-    w.scal[SC_COST] = 0; w.scal[SC_PEN] = pen; w.scal[SC_PRIM] = prim; w.scal[SC_INNER] = inner; w.scal[SC_DUAL] = 0;
-  }
-  SYNC();
-  if (!DERIV) { PAR_FOR(i, SC_COUNT) io.scal[i] = w.scal[i]; return; }
-  PAR_FOR(i, KNC) { io.dbar[i] = w.late.dbr[i]; io.vplus[i] = w.late.vpl[i]; io.act_idx[i] = (i < w.nca) ? w.act_idx[i] : -1; }
-  ONE_THREAD io.nca[0] = w.nca;
-  PAR_FOR(z, KNZ) {
-    io.lxu[z] = 0.0;
-    double gz = 0;
-    if (z < NV && has_c) for (int r = 0; r < 3; r++) gz += io.v[r] * w.U[6 * z + r] * rcp_(w.Ic[0]);
-    if (z >= 6 && z < FN) gz -= io.lam_k[z];
-    w.late.g[z] = gz; io.g[z] = gz;
-  }
-  PAR_FOR(e, KNZ * KNZ) { int a = e / KNZ, b = e % KNZ; io.H[e] = (a == b && a < FN) ? io.preg : 0.0; }
-  PAR_FOR(e, w.nca * KNZ) { int ai = e / KNZ, z = e % KNZ, r = w.act_idx[ai]; io.CDact[e] = (z < NV) ? w.U[6 * z + r] * rcp_(w.Ic[0]) : 0.0; }
-  SYNC();
-  ONE_THREAD {
-    double dual = 0;
-    for (int z = 6; z < FN; z++) dual = fmax(dual, fabs(w.late.g[z]));
-    w.scal[SC_DUAL] = dual;
-  }
-  SYNC();
-  PAR_FOR(i, SC_COUNT) io.scal[i] = w.scal[i];
+  mb_dual_scal<KNZ>(w, io);
 }
 
 } // namespace mpcdev

@@ -5,10 +5,10 @@
 //   Jc     = pin.getFrameJacobian(..., LOCAL) of both sole frames    [12][nv]
 //   dJv    = pin.getFrameJacobianTimeVariation(..., LOCAL) @ v       [12]   (spatial acceleration of the frame at zero joint acceleration)
 //   vf     = pin.getFrameVelocity(...)  (LOCAL: linear, angular)     [2][6]
-// One group of threads per state, on the kinematics / composite-inertia phases of the evaluation kernel (eval_full.cuh:
-// mb_kinematics and the bias-force phase of eval_full_knot), world-frame formulation, everything in the group's shared memory.
+// One group of threads per state, on the kinematics / composite-inertia phases of the evaluation kernel
+// (mb_kinematics and the bias-force phase of eval_full_knot), world-frame formulation, everything in the group's shared memory.
 #pragma once
-#include "eval_full.cuh"
+#include "eval_mb.cuh"
 
 namespace mpcdev {
 

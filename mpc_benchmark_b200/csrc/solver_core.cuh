@@ -271,7 +271,7 @@ template <> struct KindTraits<MPC_KIND_FULL> {
   static constexpr int ncap = 23; // active rows of the Riccati's shared-memory carving: what fits over the dead P | G buffers (two instances per SM)
   template <bool D> using EvalWs = FullWsT<D>;
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_full_knot<D, ROLL>(md, io, f); }
-  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_full_term<D>(md, io, f); }
+  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_mb_term<D, true, FNZ, FNC>(md, io, f); }
   static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
   static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
   // two 128-thread instances per SM when the launch fills the GPU; 256 threads per instance when SMs would idle (latency)
@@ -282,7 +282,7 @@ template <> struct KindTraits<MPC_KIND_KINO> {
   static constexpr int ncap = 54; // knots with more active rows (up to all 68) solve their KKT out of global scratch
   template <bool D> using EvalWs = KinoWsT<D>;
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_kino_knot<D, ROLL>(md, io, f); }
-  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_kino_term<D>(md, io, f); }
+  template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_mb_term<D, false, KNZ, KNC>(md, io, f); }
   static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
   static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
   static constexpr int ric_threads(int, int) { return 256; }
