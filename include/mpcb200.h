@@ -210,6 +210,19 @@ int32_t mpc_debug_phases(mpc_solver_t *h, double *out64);
 int32_t mpc_rbd_terms(mpc_solver_t *h, int32_t count, const double *x, double *M, double *nle, double *Jc, double *dJv, double *vf);
 int32_t mpc_rbd_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, uint64_t M_dev, uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev,
                              uint64_t vf_dev, uint64_t stream);
+/* The same M, nle, Jc, dJv plus the task terms of the IKID QP (IKIDSolver_f6, QP_utils.py:666-675,684,690) for `count` states:
+ *   Ag [count][6][nv]      data.Ag, centroidal momentum matrix about the CoM, world axes, linear rows then angular rows;
+ *   dAgv [count][6]        data.dAg @ v: rate of the centroidal momentum at zero joint acceleration, gravity EXCLUDED;
+ *   Jang [count][2][3][nv] angular rows of the LOCAL frame Jacobian of the two frames (frame_body[f], frame_place[f]: parent body
+ *                          in [0, nb) and placement in it, R row-major then p), in the caller's order (the IKID QP: base, then torso);
+ *   dJang [count][2][3]    angular part of those frames' LOCAL acceleration at zero joint acceleration (dJ v).
+ * The LOCAL frame matches the sole Jacobians; which frame the reference uses for the base / torso rows (QP_utils.py:666-675) is
+ * UNPINNED.  Host arrays (any output may be NULL) / device pointers + stream (asynchronous).  Not available for MPC_KIND_CENT. */
+int32_t mpc_ikid_terms(mpc_solver_t *h, int32_t count, const double *x, const int32_t frame_body[2], const double frame_place[2][12], double *M,
+                       double *nle, double *Jc, double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang);
+int32_t mpc_ikid_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, const int32_t frame_body[2], const double frame_place[2][12],
+                              uint64_t M_dev, uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t Ag_dev, uint64_t dAgv_dev,
+                              uint64_t Jang_dev, uint64_t dJang_dev, uint64_t stream);
 /* ---- Device-side gait / swing-foot reference generation (SURVEY 8f row f-4).  Replaces, per MPC tick and for the whole batch, the
  * Python bookkeeping of the reference loops: update_timings (talos_utils.py:350-373), footTrajectory.updateTrajectory
  * (talos_utils.py:187-327), the per-stage setReference / contact_poses writes and the stage entering the horizon

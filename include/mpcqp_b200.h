@@ -102,6 +102,22 @@ struct mpc_solver;
 int32_t mpc_qp_assemble_id_from_state(mpc_qp_t *h, struct mpc_solver *solver, int32_t batch, const double *x, const double *a, const double *forces,
                                       const int32_t *cs, double mu, double L, double W, double kd);
 
+/* The whole IKID QP of the reference (IKIDSolver_f6.computeMatrice, QP_utils.py:666-738; n 62, n_eq 40, n_in 18, box constraints)
+ * assembled on the device from MEASURED STATES: x [batch][57] host -> M, nle, Jc, dJv and the task terms (mpc_ikid_terms_device of
+ * `solver`, a libmpcb200 solver handle created for the same robot; frame_body / frame_place name the base and torso frames, whose
+ * LOCAL angular Jacobians are used — the reference's choice of frame there is unpinned) -> the cost
+ *   H[:28,:28] = w0 I + w1 (JL'JL + JR'JR) + w2 Ag'Ag + w3 (Jb'Jb + Jt'Jt),  H[28:40,28:40] = w4 I,  zeros elsewhere,
+ *   g[:28] from the PD task errors, the gains, dJv, dAgv and dH (QP_utils.py:684-691),
+ * and A, b, C, l as mpc_qp_assemble_id with a = 0 and gamma = dJv on the active contacts (no Baumgarte term).
+ * task [batch][98]: q_diff 28, dq_diff 28, LF 6, dLF 6, RF 6, dRF 6, base 3, dbase 3, torso 3, dtorso 3, dH 6 (the argument order of
+ * IKIDSolver_f6.solve); forces [batch][12]; cs [batch][2]; weights [5]; gains [1658], shared: Kp_q, Kd_q (28 x 28), Kp_f, Kd_f (6 x 6),
+ * Kp_b, Kd_b (3 x 3), row-major general matrices.  Afterwards H, g, A, b, C, l hold one array per QP; u, l_box, u_box stay as uploaded.
+ * Uploads 167 doubles + 8 bytes per robot (+ the gains once per call) instead of the 5,106 doubles of the host-side cost.
+ * The first call allocates a scratch for the task terms and gains, freed by mpc_qp_destroy. */
+int32_t mpc_qp_assemble_ikid_from_state(mpc_qp_t *h, struct mpc_solver *solver, int32_t batch, const double *x, const double *task,
+                                        const double *forces, const int32_t *cs, const double weights[5], const double *gains,
+                                        const int32_t frame_body[2], const double frame_place[2][12], double mu, double L, double W);
+
 #ifdef __cplusplus
 }
 #endif

@@ -17,7 +17,8 @@ EXPORTS = [
     "mpc_run", "mpc_run_pipelined", "mpc_run_device", "mpc_tick", "mpc_get_results", "mpc_export_results_device", "mpc_result_ptrs", "mpc_get_stage_data", "mpc_last_launches", "mpc_last_device_ms",
     "mpc_get_feedback", "mpc_last_kernel_ms", "mpc_last_kernel_launches", "mpc_set_profiling",
     "mpc_qp_create", "mpc_qp_destroy", "mpc_qp_last_error", "mpc_qp_default_settings", "mpc_qp_update", "mpc_qp_solve", "mpc_qp_solve_device",
-    "mpc_qp_last_device_ms", "mpc_qp_abi_sizeof", "mpc_qp_assemble_id", "mpc_qp_debug_phases", "mpc_qp_assemble_id_from_state", "mpc_rbd_terms", "mpc_rbd_terms_device", "mpc_gait_setup", "mpc_gait_tick", "mpc_get_knots", "mpc_set_tail_warmstart",
+    "mpc_qp_last_device_ms", "mpc_qp_abi_sizeof", "mpc_qp_assemble_id", "mpc_qp_debug_phases", "mpc_qp_assemble_id_from_state", "mpc_rbd_terms", "mpc_rbd_terms_device",
+    "mpc_ikid_terms", "mpc_ikid_terms_device", "mpc_qp_assemble_ikid_from_state", "mpc_gait_setup", "mpc_gait_tick", "mpc_get_knots", "mpc_set_tail_warmstart",
     "mpc_reset_multipliers", "mpc_debug_lq", "mpc_debug_gemm_tn", "mpc_debug_phases", "mpc_workspace_bytes", "mpc_abi_sizeof", "mpc_measure_fp64_peak", "mpc_measure_fp64_peak_dmma",
 ]
 
@@ -87,6 +88,9 @@ def lib():
         L.mpc_qp_assemble_id_from_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, dp, dp, dp, i32p] + [C.c_double] * 4
         L.mpc_rbd_terms.argtypes = [C.c_void_p, C.c_int32] + [dp] * 6
         L.mpc_rbd_terms_device.argtypes = [C.c_void_p, C.c_int32] + [u64] * 7
+        L.mpc_ikid_terms.argtypes = [C.c_void_p, C.c_int32, dp, i32p, dp] + [dp] * 8
+        L.mpc_ikid_terms_device.argtypes = [C.c_void_p, C.c_int32, u64, i32p, dp] + [u64] * 9
+        L.mpc_qp_assemble_ikid_from_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, dp, dp, dp, i32p, dp, dp, i32p, dp] + [C.c_double] * 3
         L.mpc_gait_setup.argtypes = [C.c_void_p, C.POINTER(_abi.Gait), i32p, dp]
         L.mpc_gait_tick.argtypes = [C.c_void_p, dp, dp]
         L.mpc_get_knots.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]

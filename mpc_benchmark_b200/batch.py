@@ -9,6 +9,7 @@ import ctypes as C
 import numpy as np
 
 from . import _abi, _native
+from .qp_utils import RBDTermsIKID
 
 
 class BatchResults:
@@ -199,6 +200,21 @@ class BatchSolver:
         o = dict(M=np.zeros((B, 28, 28)), nle=np.zeros((B, 28)), Jc=np.zeros((B, 12, 28)), dJv=np.zeros((B, 12)), vf=np.zeros((B, 2, 6)))
         _native.check(_native.lib().mpc_rbd_terms(self._h, B, _native.ptr(x), *[_native.ptr(o[k]) for k in ("M", "nle", "Jc", "dJv", "vf")]), "mpc_rbd_terms")
         return o
+
+    def ikid_terms(self, x, frames):
+        """Rigid-body terms and task terms of the IKID QP (IKIDSolver_f6, QP_utils.py:666-675) for the states x [count][nx]:
+        (M, qp_utils.RBDTermsIKID).  frames = ((body, placement 12), (body, placement 12)) of the base and torso frames, whose LOCAL
+        angular Jacobians and dJ v are returned.  Uses only the handle's robot model."""
+        x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, 57)
+        B = x.shape[0]
+        fb = np.ascontiguousarray([f[0] for f in frames], dtype=np.int32)
+        fp = np.ascontiguousarray([f[1] for f in frames], dtype=np.float64).reshape(2, 12)
+        o = dict(M=np.zeros((B, 28, 28)), nle=np.zeros((B, 28)), Jc=np.zeros((B, 12, 28)), dJv=np.zeros((B, 12)), Ag=np.zeros((B, 6, 28)),
+                 dAgv=np.zeros((B, 6)), Jang=np.zeros((B, 2, 3, 28)), dJang=np.zeros((B, 2, 3)))
+        _native.check(_native.lib().mpc_ikid_terms(self._h, B, _native.ptr(x), fb.ctypes.data_as(C.POINTER(C.c_int32)), _native.ptr(fp),
+                                                   *[_native.ptr(o[k]) for k in ("M", "nle", "Jc", "dJv", "Ag", "dAgv", "Jang", "dJang")]), "mpc_ikid_terms")
+        return o["M"], RBDTermsIKID(nle=o["nle"], Jc=o["Jc"], dJv=o["dJv"], J_base=o["Jang"][:, 0], dJv_base=o["dJang"][:, 0], J_torso=o["Jang"][:, 1],
+                                    dJv_torso=o["dJang"][:, 1], Ag=o["Ag"], dAgv=o["dAgv"])
 
     def feedback(self, k=0):
         """results.controlFeedbacks()[k] for every instance: [batch, nu, ndx]."""

@@ -35,6 +35,22 @@ __global__ void __launch_bounds__(QP_THREADS) k_qp_assemble_id(const AsmArgs P) 
                        P.A + (size_t)i * 2480, P.b + i * 40, P.C + (size_t)i * 1116, P.l + i * 18);
 }
 
+struct IkidAsmArgs {
+  const double *M, *nle, *Jc, *dJv, *Ag, *dAgv, *Jang, *dJang, *task, *forces, *gains;
+  const int32_t *cs;
+  double wt[5], mu, L, W;
+  double *H, *g, *A, *b, *C, *l;
+  int batch;
+};
+__global__ void __launch_bounds__(QP_THREADS) k_qp_assemble_ikid(const IkidAsmArgs P) {
+  __shared__ double sm[24 * 28 + 24 + 12 + 28];
+  const int i = blockIdx.x;
+  if (i >= P.batch) return;
+  qp_assemble_ikid_group(P.M + i * 784, P.nle + i * 28, P.Jc + i * 336, P.dJv + i * 12, P.Ag + i * 168, P.dAgv + i * 6, P.Jang + i * 168, P.dJang + i * 6,
+                         P.task + i * 98, P.forces + i * 12, P.cs + i * 2, P.wt, P.gains, P.mu, P.L, P.W, sm, P.H + (size_t)i * 3844, P.g + i * 62,
+                         P.A + (size_t)i * 2480, P.b + i * 40, P.C + (size_t)i * 1116, P.l + i * 18);
+}
+
 // gamma = (dJ v + kd (v_lin + v_ang) on the linear rows) of the active contacts (QP_utils.py:524-528), in place over dJv
 __global__ void k_qp_gamma(double *dJv, const double *vf, const int32_t *cs, double kd, int batch) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -62,6 +78,7 @@ struct mpc_qp {
   int n, ne, ni, box, nz, max_batch, device, batch = 0;
   Slot H, g, A, b, C, l, u, lb, ub;
   double *dx = nullptr, *dy = nullptr, *dz = nullptr, *dscratch = nullptr, *dstate = nullptr; // dstate: [B][57] states + [B][12] frame velocities
+  double *dikid = nullptr; // IKID assembly only, allocated by its first call: gains [1658] + [B][98] task errors + [B] task terms (IkidScratch)
   mpc_qp_info_t *dinfo = nullptr;
   long long *dphase = nullptr; // instrumented builds only
   cudaStream_t stream = nullptr;
@@ -104,6 +121,13 @@ int assemble_id(mpc_qp *h, const AsmScratch &s, int batch, double mu, double L, 
   return 0;
 }
 
+// the IKID assembly's inputs beyond AsmScratch, for B QPs: the shared gains, then per QP the task errors and the task terms
+constexpr size_t IKID_GAINS = 2 * 784 + 2 * 36 + 2 * 9, IKID_PER = 98 + 168 + 6 + 168 + 6;
+struct IkidScratch {
+  double *gains, *task, *Ag, *dAgv, *Jang, *dJang;
+  IkidScratch(double *s, size_t B) : gains(s), task(gains + IKID_GAINS), Ag(task + B * 98), dAgv(Ag + B * 168), Jang(dAgv + B * 6), dJang(Jang + B * 168) {}
+};
+
 int launch(mpc_qp *h, const QPArgs &P, cudaStream_t stream) {
   if (P.batch <= 0) return 0;
   const int grid = P.batch; // one CTA per QP: QPs take different numbers of Newton steps, the hardware scheduler balances them
@@ -132,7 +156,7 @@ void mpc_qp_destroy(mpc_qp_t *h) {
   if (!h) return;
   cudaSetDevice(h->device);
   for (Slot *s : {&h->H, &h->g, &h->A, &h->b, &h->C, &h->l, &h->u, &h->lb, &h->ub}) cudaFree(s->d);
-  cudaFree(h->dphase); cudaFree(h->dstate);
+  cudaFree(h->dphase); cudaFree(h->dstate); cudaFree(h->dikid);
   cudaFree(h->dx); cudaFree(h->dy); cudaFree(h->dz); cudaFree(h->dinfo); cudaFree(h->dscratch);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
@@ -302,6 +326,42 @@ int32_t mpc_qp_assemble_id_from_state(mpc_qp_t *h, struct mpc_solver *solver, in
     return fail(std::string("mpc_rbd_terms_device: ") + mpc_last_error());
   k_qp_gamma<<<(batch * 12 + 127) / 128, 128, 0, h->stream>>>(s.gamma, h->dstate + B * 57, s.cs, kd, batch);
   return assemble_id(h, s, batch, mu, L, W);
+}
+
+int32_t mpc_qp_assemble_ikid_from_state(mpc_qp_t *h, struct mpc_solver *solver, int32_t batch, const double *x, const double *task, const double *forces,
+                                        const int32_t *cs, const double weights[5], const double *gains, const int32_t frame_body[2],
+                                        const double frame_place[2][12], double mu, double L, double W) {
+  if (!h || !solver) return fail("null handle");
+  if (!x || !task || !forces || !cs || !weights || !gains || !frame_body || !frame_place) return fail("mpc_qp_assemble_ikid_from_state: null argument");
+  if (h->n != 62 || h->ne != 40 || h->ni != 18 || !h->box)
+    return fail("mpc_qp_assemble_ikid_from_state: handle is not the IKID shape (n 62, n_eq 40, n_in 18, box constraints)");
+  if (batch <= 0 || batch > h->max_batch) return fail("mpc_qp_assemble_ikid_from_state: batch out of range");
+  CUQ(cudaSetDevice(h->device));
+  if (!h->dikid && cudaMalloc(&h->dikid, 8 * (IKID_GAINS + (size_t)h->max_batch * IKID_PER)) != cudaSuccess)
+    return fail("mpc_qp_assemble_ikid_from_state: cudaMalloc of the IKID scratch failed");
+  const size_t B = batch;
+  // M, nle, Jc and dJv (in the gamma slot) come from the rigid-body terms of the states, the task terms go to the IKID scratch
+  const AsmScratch s(h->dscratch, B);
+  const IkidScratch k(h->dikid, B);
+  CUQ(cudaMemcpyAsync(h->dstate, x, 8 * B * 57, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(k.task, task, 8 * B * 98, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(k.gains, gains, 8 * IKID_GAINS, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.forces, forces, 8 * B * 12, cudaMemcpyHostToDevice, h->stream));
+  CUQ(cudaMemcpyAsync(s.cs, cs, 4 * B * 2, cudaMemcpyHostToDevice, h->stream));
+  if (mpc_ikid_terms_device(solver, batch, (uint64_t)h->dstate, frame_body, frame_place, (uint64_t)s.M, (uint64_t)s.nle, (uint64_t)s.Jc, (uint64_t)s.gamma,
+                            (uint64_t)k.Ag, (uint64_t)k.dAgv, (uint64_t)k.Jang, (uint64_t)k.dJang, (uint64_t)h->stream) != 0)
+    return fail(std::string("mpc_ikid_terms_device: ") + mpc_last_error());
+  IkidAsmArgs P;
+  P.M = s.M; P.nle = s.nle; P.Jc = s.Jc; P.dJv = s.gamma; P.Ag = k.Ag; P.dAgv = k.dAgv; P.Jang = k.Jang; P.dJang = k.dJang; P.task = k.task;
+  P.forces = s.forces; P.gains = k.gains; P.cs = s.cs;
+  for (int i = 0; i < 5; i++) P.wt[i] = weights[i];
+  P.mu = mu; P.L = L; P.W = W;
+  P.H = h->H.d; P.g = h->g.d; P.A = h->A.d; P.b = h->b.d; P.C = h->C.d; P.l = h->l.d; P.batch = batch;
+  k_qp_assemble_ikid<<<batch, QP_THREADS, 0, h->stream>>>(P);
+  CUQ(cudaGetLastError());
+  for (Slot *sl : {&h->H, &h->g, &h->A, &h->b, &h->C, &h->l}) { sl->stride = sl->per; sl->set = true; }
+  h->batch = batch;
+  return 0;
 }
 
 } // extern "C"

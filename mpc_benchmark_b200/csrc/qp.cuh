@@ -525,4 +525,68 @@ HD void qp_assemble_id_group(const double *M, const double *nle, const double *J
   }
 }
 
+// IKIDSolver_f6.computeMatrice (QP_utils.py:677-738) for one instance, nv = 28, two 6-D contacts: fills H [62][62], g [62] and, through
+// qp_assemble_id_group with a = 0 and gamma = dJv on the active contacts, A, b, C, l.  Inputs per instance: M, nle, Jc, dJv, Ag [6][28],
+// dAgv [6], Jang [2][3][28] (base, torso), dJang [2][3], task [98] (q_diff 28, dq_diff 28, LF 6, dLF 6, RF 6, dRF 6, base 3, dbase 3,
+// torso 3, dtorso 3, dH 6), forces, cs; shared: weights [5], gains [1658] (Kp_q, Kd_q 28 x 28, Kp_f, Kd_f 6 x 6, Kp_b, Kd_b 3 x 3, row-major).
+// sm: 24 * 28 + 24 + 12 + 28 doubles of the group's shared memory.
+//   H[:28,:28] = w0 I + w1 (JL'JL + JR'JR) + w2 Ag'Ag + w3 (Jb'Jb + Jt'Jt),   H[28:40,28:40] = w4 I,   zeros elsewhere
+//   g[:28] = -w0 (Kp_q q_diff + Kd_q dq_diff) + sum_k w_k r_k' J_k over the task rows J_k = (JL, JR, Ag, Jb, Jt) with
+//            r = dJv_L - Kp_f LF - Kd_f dLF,  dJv_R - Kp_f RF - Kd_f dRF,  dAgv - dH,  dJv_b - Kp_b base - Kd_b dbase,  same for the torso
+HD void qp_assemble_ikid_group(const double *M, const double *nle, const double *Jc, const double *dJv, const double *Ag, const double *dAgv, const double *Jang,
+                               const double *dJang, const double *task, const double *forces, const int32_t *cs, const double *wt, const double *gains,
+                               double mu, double L, double W, double *sm, double *H, double *g, double *A, double *b, double *C, double *l) {
+  constexpr int nv = 28, n = 62, NR = 24;
+  const double *Kpq = gains, *Kdq = Kpq + nv * nv, *Kpf = Kdq + nv * nv, *Kdf = Kpf + 36, *Kpb = Kdf + 36, *Kdb = Kpb + 9;
+  double *J = sm, *r = J + NR * nv, *gamma = r + NR, *a = gamma + 12; // task rows JL, JR, Ag, Jb, Jt; their residuals; gamma; a = 0
+  PAR_FOR(e, NR * nv) {
+    const int k = e / nv, c = e % nv;
+    J[e] = k < 12 ? Jc[e] : k < 18 ? Ag[(k - 12) * nv + c] : Jang[(k - 18) * nv + c];
+  }
+  PAR_FOR(k, NR) {
+    double s;
+    if (k < 12) { // contact rows: K_f is 6 x 6 over the rows of one foot
+      const int f = k / 6, i = k % 6;
+      const double *e = task + 56 + 12 * f, *de = e + 6;
+      s = dJv[k];
+      for (int j = 0; j < 6; j++) s -= Kpf[6 * i + j] * e[j] + Kdf[6 * i + j] * de[j];
+    } else if (k < 18) s = dAgv[k - 12] - task[92 + k - 12];
+    else { // base / torso rows: K_b is 3 x 3
+      const int f = (k - 18) / 3, i = (k - 18) % 3;
+      const double *e = task + 80 + 6 * f, *de = e + 3;
+      s = dJang[k - 18];
+      for (int j = 0; j < 3; j++) s -= Kpb[3 * i + j] * e[j] + Kdb[3 * i + j] * de[j];
+    }
+    r[k] = s;
+  }
+  PAR_FOR(k, 12) gamma[k] = cs[k / 6] ? dJv[k] : 0.0;
+  PAR_FOR(j, nv) a[j] = 0.0;
+  SYNC();
+  PAR_FOR(e, n * n) {
+    const int i = e / n, j = e % n;
+    double v = 0;
+    if (i < nv && j < nv) {
+      double s1 = 0, s2 = 0, s3 = 0;
+      for (int k = 0; k < 12; k++) s1 += J[k * nv + i] * J[k * nv + j];
+      for (int k = 12; k < 18; k++) s2 += J[k * nv + i] * J[k * nv + j];
+      for (int k = 18; k < NR; k++) s3 += J[k * nv + i] * J[k * nv + j];
+      v = (i == j ? wt[0] : 0.0) + wt[1] * s1 + wt[2] * s2 + wt[3] * s3;
+    } else if (i == j && i >= nv && i < nv + 12) v = wt[4];
+    H[e] = v;
+  }
+  PAR_FOR(i, n) {
+    double v = 0;
+    if (i < nv) {
+      double p = 0, s1 = 0, s2 = 0, s3 = 0;
+      for (int j = 0; j < nv; j++) p += Kpq[i * nv + j] * task[j] + Kdq[i * nv + j] * task[nv + j];
+      for (int k = 0; k < 12; k++) s1 += r[k] * J[k * nv + i];
+      for (int k = 12; k < 18; k++) s2 += r[k] * J[k * nv + i];
+      for (int k = 18; k < NR; k++) s3 += r[k] * J[k * nv + i];
+      v = -wt[0] * p + wt[1] * s1 + wt[2] * s2 + wt[3] * s3;
+    }
+    g[i] = v;
+  }
+  qp_assemble_id_group(M, nle, Jc, gamma, a, forces, cs, mu, L, W, A, b, C, l);
+}
+
 } // namespace mpcdev

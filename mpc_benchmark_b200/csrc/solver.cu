@@ -112,6 +112,21 @@ __global__ void __launch_bounds__(128) k_rbd_terms(const DevModel *model, const 
   rbd_terms_group(*model, x + (size_t)i * (NQ + NV), w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV, dJv + (size_t)i * 12, vf + (size_t)i * 12);
 }
 
+// the same terms plus the IKID QP's task terms (ikid_terms_group) of two frames for `count` states, one 128-thread CTA per state
+struct IkidFrames {
+  int32_t body[2];
+  double place[24];
+};
+__global__ void __launch_bounds__(128) k_ikid_terms(const DevModel *model, const double *x, int count, const IkidFrames fr, double *M, double *nle, double *Jc,
+                                                    double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
+  extern __shared__ double rbd_smem[];
+  const int i = blockIdx.x;
+  if (i >= count) return;
+  FullWsT<false> &w = *reinterpret_cast<FullWsT<false> *>(rbd_smem);
+  ikid_terms_group(*model, x + (size_t)i * (NQ + NV), fr.body, fr.place, w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV,
+                   dJv + (size_t)i * 12, Ag + (size_t)i * 6 * NV, dAgv + (size_t)i * 6, Jang + (size_t)i * 6 * NV, dJang + (size_t)i * 6);
+}
+
 // device-side gait bookkeeping (gait.cuh): one 128-thread CTA per robot rewrites its T knots and terminal block
 __global__ void __launch_bounds__(128) k_gait_tick(Ws w, const GaitCfg *g, GaitRobot *robots, int t, const double *lf, const double *rf) {
   __shared__ double sm[16];
@@ -787,6 +802,49 @@ int32_t mpc_rbd_terms(mpc_solver_t *h, int32_t count, const double *x, double *M
   auto back = [&](double *dst, const double *src, size_t n) { if (!rc && dst && cudaMemcpyAsync(dst, src, 8 * B * n, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) rc = fail("D2H failed"); };
   back(M, dM, NV * NV); back(nle, dn, NV); back(Jc, dJ, 12 * NV); back(dJv, dd, 12); back(vf, dv, 12);
   if (cudaStreamSynchronize(h->stream) != cudaSuccess && !rc) rc = fail("mpc_rbd_terms: kernel failed");
+  cudaFree(d);
+  return rc;
+}
+
+int32_t mpc_ikid_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, const int32_t frame_body[2], const double frame_place[2][12], uint64_t M_dev,
+                              uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t Ag_dev, uint64_t dAgv_dev, uint64_t Jang_dev, uint64_t dJang_dev,
+                              uint64_t stream) {
+  if (!h || !frame_body || !frame_place) return fail("null handle / frames");
+  if (h->w.kind == MPC_KIND_CENT) return fail("mpc_ikid_terms: the centroidal model has no rigid-body tree");
+  if (count <= 0) return fail("mpc_ikid_terms: count out of range");
+  if (frame_body[0] < 0 || frame_body[0] >= NB || frame_body[1] < 0 || frame_body[1] >= NB) return fail("mpc_ikid_terms: frame body out of range [0, nb)");
+  CK(cudaSetDevice(h->device));
+  IkidFrames fr;
+  for (int f = 0; f < 2; f++) {
+    fr.body[f] = frame_body[f];
+    for (int i = 0; i < 12; i++) fr.place[12 * f + i] = frame_place[f][i];
+  }
+  const size_t smem = sizeof(FullWsT<false>);
+  CK(cudaFuncSetAttribute(k_ikid_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_ikid_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->d_model, (const double *)x_dev, count, fr, (double *)M_dev, (double *)nle_dev,
+                                                                                   (double *)Jc_dev, (double *)dJv_dev, (double *)Ag_dev, (double *)dAgv_dev,
+                                                                                   (double *)Jang_dev, (double *)dJang_dev);
+  CK(cudaGetLastError());
+  return 0;
+}
+int32_t mpc_ikid_terms(mpc_solver_t *h, int32_t count, const double *x, const int32_t frame_body[2], const double frame_place[2][12], double *M, double *nle,
+                       double *Jc, double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
+  if (!h) return fail("null handle");
+  if (count <= 0) return fail("mpc_ikid_terms: count out of range");
+  CK(cudaSetDevice(h->device));
+  const size_t B = count, per = (NQ + NV) + NV * NV + NV + 12 * NV + 12 + 6 * NV + 6 + 6 * NV + 6;
+  double *d = nullptr;
+  CK(cudaMalloc(&d, 8 * B * per));
+  double *dx = d, *dM = dx + B * (NQ + NV), *dn = dM + B * NV * NV, *dJ = dn + B * NV, *dd = dJ + B * 12 * NV, *dA = dd + B * 12, *dAv = dA + B * 6 * NV,
+         *dJa = dAv + B * 6, *dJav = dJa + B * 6 * NV;
+  int rc = 0;
+  if (cudaMemcpyAsync(dx, x, 8 * B * (NQ + NV), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) rc = fail("H2D of the states failed");
+  if (!rc) rc = mpc_ikid_terms_device(h, count, (uint64_t)dx, frame_body, frame_place, (uint64_t)dM, (uint64_t)dn, (uint64_t)dJ, (uint64_t)dd, (uint64_t)dA,
+                                      (uint64_t)dAv, (uint64_t)dJa, (uint64_t)dJav, 0);
+  auto back = [&](double *dst, const double *src, size_t n) { if (!rc && dst && cudaMemcpyAsync(dst, src, 8 * B * n, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) rc = fail("D2H failed"); };
+  back(M, dM, NV * NV); back(nle, dn, NV); back(Jc, dJ, 12 * NV); back(dJv, dd, 12);
+  back(Ag, dA, 6 * NV); back(dAgv, dAv, 6); back(Jang, dJa, 6 * NV); back(dJang, dJav, 6);
+  if (cudaStreamSynchronize(h->stream) != cudaSuccess && !rc) rc = fail("mpc_ikid_terms: kernel failed");
   cudaFree(d);
   return rc;
 }

@@ -205,6 +205,25 @@ class BatchQP:
         if rc != 0:
             raise _native.NativeError(f"mpc_qp_assemble_id_from_state failed: {lib.mpc_qp_last_error().decode()}")
 
+    def assemble_ikid_from_state(self, solver, x, task, forces, cs, weights, gains, frames, mu, L, W):
+        """The whole IKID QP (IKIDSolver_f6.computeMatrice, QP_utils.py:666-738) from MEASURED STATES x [batch][57]: rigid-body and task
+        terms on the device by `solver` (a batch.BatchSolver of the same robot), then H, g, A, b, C, l.  task [batch][98] packs the PD
+        errors in the argument order of IKIDSolver_f6.solve; gains [1658] packs Kp_q, Kd_q, Kp_f, Kd_f, Kp_b, Kd_b row-major;
+        frames = ((body, placement 12), (body, placement 12)) of the base and torso frames."""
+        B = self.batch
+        f = lambda v, per: np.ascontiguousarray(np.broadcast_to(np.asarray(v, float).reshape(-1, per), (B, per)))  # noqa: E731
+        xs, tk, ff = f(x, 57), f(task, 98), f(forces, 12)
+        cs = np.ascontiguousarray(np.broadcast_to(np.asarray(cs).reshape(-1, 2), (B, 2)), dtype=np.int32)
+        wt, gn = np.ascontiguousarray(weights, float).reshape(5), np.ascontiguousarray(gains, float).reshape(1658)
+        fb = np.ascontiguousarray([fr[0] for fr in frames], dtype=np.int32)
+        fp = np.ascontiguousarray([fr[1] for fr in frames], dtype=np.float64).reshape(2, 12)
+        i32p = C.POINTER(C.c_int32)
+        lib = _native.lib()
+        rc = lib.mpc_qp_assemble_ikid_from_state(self._handle(), solver._h, B, _native.ptr(xs), _native.ptr(tk), _native.ptr(ff), cs.ctypes.data_as(i32p),
+                                                 _native.ptr(wt), _native.ptr(gn), fb.ctypes.data_as(i32p), _native.ptr(fp), float(mu), float(L), float(W))
+        if rc != 0:
+            raise _native.NativeError(f"mpc_qp_assemble_ikid_from_state failed: {lib.mpc_qp_last_error().decode()}")
+
 
 class QP(BatchQP):
     """proxsuite.proxqp.dense.QP(n, n_eq, n_in[, box_constraints], dense_backend=...): one QP (a batch of one)."""

@@ -4,7 +4,8 @@ kinodynamic_talos.py:408-445) on the CUDA QP solver (proxqp.BatchQP -> libmpcb20
 Same constructor arguments, same `solve(...)` return values (new accelerations, new contact forces, joint torques), with a leading
 batch axis on every array.  The reference reads M, nle, the LOCAL contact Jacobians, dJ v and the frame velocities out of a
 `pinocchio.Data`; here they are passed as arrays (`RBDTerms`, produced by whatever plays pinocchio's part: the fixture generator
-in tests/, a user's own pinocchio, ...), because the rigid-body library is not part of this row.
+in tests/, a user's own pinocchio, ...).  Both classes also have `solve_from_state`, which computes those terms on the device from the
+measured states (the kernels of csrc/rbd_terms.cuh) and assembles the whole QP there.
 """
 from dataclasses import dataclass
 
@@ -100,7 +101,8 @@ class IKIDSolver_f6:
     """Batched mirror of QP_utils.py:584-768 (inverse kinematics + dynamics QP, 6-D contact wrenches, torque box constraints):
     the cost `H, g` is assembled on the host with batched numpy exactly as QP_utils.py:677-691 writes it, the constraint blocks by
     the same CUDA assembly kernel as IDSolver_ulim (they coincide with a = 0 and gamma = dJ v: QP_utils.py:693-721), the solve runs
-    on the batched CUDA QP solver with box constraints."""
+    on the batched CUDA QP solver with box constraints.  `solve_from_state` builds the same QP, cost included, on the device from the
+    measured states."""
 
     def __init__(self, model, weights, K_gains, nk, mu, L, W, contact_ids, base_id, torso_id, force_size, verbose=False, batch=1, device=0):
         if force_size != 6 or nk != 2 or model.nv != 28:
@@ -164,3 +166,31 @@ class IKIDSolver_f6:
         new_forces = np.asarray(forces, float).reshape(self.batch, nf) + x[:, nv:nv + nf]
         torque = x[:, nv + nf:]
         return anew, new_forces, torque
+
+    def _frames(self):
+        """(parent body, placement 12) of the base and torso frames named by base_id / torso_id."""
+        return [(self.model.frames[i].parentJoint - 1, self.model.frames[i].placement.to12()) for i in (self.base_id, self.torso_id)]
+
+    def _packed_gains(self):
+        """K_gains packed as the device assembly reads them: Kp_q, Kd_q (nv x nv), Kp_f, Kd_f (6 x 6), Kp_b, Kd_b (3 x 3), row-major."""
+        K, nv = self.K_gains, self.model.nv
+        return np.concatenate([np.broadcast_to(np.asarray(k, float), (m, m)).ravel() for k, m in
+                               ((K[0][0], nv), (K[0][1], nv), (K[1][0], 6), (K[1][1], 6), (K[3][0], 3), (K[3][1], 3))])
+
+    def solve_from_state(self, solver, x_measured, cs, q_diff, dq_diff, LF_diff, dLF_diff, RF_diff, dRF_diff, base_diff, dbase_diff, torso_diff,
+                         dtorso_diff, forces, dH):
+        """centroidal_talos.py:435-445 in one call for the whole batch: the pinocchio step (crba, nonLinearEffects, the contact, base and
+        torso frame Jacobians with their time variation, the centroidal momentum matrix and dAg v at the MEASURED states x_measured
+        [batch][57]) runs on the device through `solver` (a kinodynamic or full-dynamics batch.BatchSolver of the same robot), then the
+        whole cost and constraint assembly and the QP.  Only x, the task errors, forces and cs are uploaded per robot.  Returns what
+        `solve` returns.  The base / torso rows use the LOCAL frame."""
+        B = self.batch
+        f = lambda a, per: np.broadcast_to(np.asarray(a, float).reshape(-1, per), (B, per))  # noqa: E731
+        nv = self.model.nv
+        task = np.concatenate([f(q_diff, nv), f(dq_diff, nv), f(LF_diff, 6), f(dLF_diff, 6), f(RF_diff, 6), f(dRF_diff, 6), f(base_diff, 3), f(dbase_diff, 3),
+                               f(torso_diff, 3), f(dtorso_diff, 3), f(dH, 6)], axis=1)
+        self.qp.assemble_ikid_from_state(solver, x_measured, task, forces, cs, self.weights, self._packed_gains(), self._frames(), self.mu, self.L, self.W)
+        self.qp.solve()
+        nf = self.force_size * self.nk
+        x = self.qp.results.x
+        return x[:, :nv], np.asarray(forces, float).reshape(B, nf) + x[:, nv:nv + nf], x[:, nv + nf:]
