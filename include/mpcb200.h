@@ -78,7 +78,8 @@ typedef struct mpc_config {
   int32_t max_iters;
   int32_t force_initial_condition;
   int32_t rollout;              /* solver.rollout_type (full:381): 0 = ROLLOUT_LINEAR (every reference script), 1 = ROLLOUT_NONLINEAR */
-  int32_t pad_;
+  int32_t lq_legs;              /* LQ solve: 0 or 1 = serial Riccati sweep; 2..min(16, T) = time-parallel solve over that many horizon legs
+                                   (same step and gains up to rounding, lower single-instance latency; DESIGN section 5) */
 } mpc_config_t;
 
 /* Per-knot parameter block (one per instance per knot). */

@@ -64,7 +64,7 @@ class Config(C.Structure):
         ("max_iters", i32),
         ("force_initial_condition", i32),
         ("rollout", i32),
-        ("pad_", i32),
+        ("lq_legs", i32),
     ]
 
 

@@ -506,6 +506,8 @@ class SolverProxDDP:
         self.force_initial_condition = True
         self.ldlt_algo_choice = 0
         self.num_threads = 1
+        # horizon legs of the time-parallel LQ solve (0 = serial).  Independent of linear_solver_choice, which stays recorded only.
+        self.lq_legs = 0
         self.device = device
         self.results, self.workspace = Results(), Workspace(self)
         self._bs, self._sig, self._T, self._flat = None, None, 0, None
@@ -529,7 +531,7 @@ class SolverProxDDP:
 
         self._check_options()
         flat = flatten.flatten_problem(problem, tol=self.target_tol, mu_init=self.mu_init, max_iters=self.max_iters,
-                                       rollout=int(self.rollout_type == ROLLOUT_NONLINEAR))
+                                       rollout=int(self.rollout_type == ROLLOUT_NONLINEAR), lq_legs=self.lq_legs)
         sig = (flat.cfg.kind, flat.cfg.T)
         if self._bs is None or sig != self._sig:
             if self._bs is not None:
@@ -552,7 +554,7 @@ class SolverProxDDP:
             raise RuntimeError("SolverProxDDP.run: call setup(problem) first")
         self._check_options()
         flat = flatten.flatten_problem(problem, tol=self.target_tol, mu_init=self.mu_init, max_iters=self.max_iters,
-                                       rollout=int(self.rollout_type == ROLLOUT_NONLINEAR))
+                                       rollout=int(self.rollout_type == ROLLOUT_NONLINEAR), lq_legs=self.lq_legs)
         if (flat.cfg.kind, flat.cfg.T) != self._sig:
             raise RuntimeError("problem structure changed since setup(); call setup(problem) again")
         bs = self._bs

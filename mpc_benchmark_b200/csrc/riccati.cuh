@@ -72,6 +72,10 @@ struct RiccatiIO {
   int32_t *overflow;     // set to 1 when a knot has more active rows than the kernel's shared-memory capacity
   double *scratch;       // per-instance global block for the KKT buffers of knots whose active rows exceed the shared-memory carving
   double *phase_out;     // optional 16 per-phase cycle counters (MPC_PHASE_TIMING builds), else nullptr
+  // SEEDED solves (one leg of the time-parallel solve, riccati_par.cuh): knots [k0, k1) only, backward from the value function
+  // (seedP, seedp) at k1 (nullptr: the terminal knot, k1 = T), forward from dx0 at k0
+  int k0, k1;
+  const double *seedP, *seedp, *dx0;
 };
 
 template <int N, int M, int NC> constexpr int riccati_smem_doubles() {
@@ -83,9 +87,13 @@ template <int N, int M, int NC> constexpr int riccati_smem_doubles() {
 
 // Backward + forward sweep for one instance.  ws: riccati_smem_doubles<N,M,NC>() doubles of shared memory.
 // LIE6: the first 6 state coordinates live on SE(3) (E-normalisation by T6); false for vector-space models (centroidal: T6 = I)
-template <int N, int M, int NC, bool LIE6 = true> HD void riccati_instance(const RiccatiIO &io, double *ws) {
+// SEEDED: solve the knots [io.k0, io.k1) only (see RiccatiIO).  dxs / dlams of knot k0 are written by leg 0 only, the terminal knot's
+// rows by the last leg only; dphi receives the leg's partial.
+template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void riccati_instance(const RiccatiIO &io, double *ws) {
   constexpr int NZ = N + M, NR = 1 + N, S = M + NC;
   const int T = io.T;
+  const int K0 = SEEDED ? io.k0 : 0, K1 = SEEDED ? io.k1 : T;
+  const bool seeded = SEEDED && io.seedP != nullptr, last = !SEEDED || K1 == T;
   const double mu = io.mu, mu_d = io.mu_d;
   // ---- carve shared memory
   double *H = ws;                       // NZ*NZ; its [0:N,0:N] block carries the value-function Hessian between knots
@@ -98,7 +106,11 @@ template <int N, int M, int NC, bool LIE6 = true> HD void riccati_instance(const
   double *p = vec, *pt = p + NZ, *gh = pt + NZ, *fb = gh + NZ, *tmp = fb + NZ, *dx = tmp + NZ, *z = dx + NZ, *dl = z + NZ;
   double *T6 = dl + NZ, *dbr = T6 + 36, *dva = dbr + NC, *red = dva + NC, *dinv = red + 512;
   // ---- terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C' d/mu
-  {
+  if (seeded) {
+    PAR_FOR(e, N * N) H[(e / N) * NZ + e % N] = io.seedP[e];
+    PAR_FOR(i, N) p[i] = io.seedp[i];
+    SYNC();
+  } else {
     const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ;
     const int nca = io.nca[T];
     const double *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
@@ -116,7 +128,7 @@ template <int N, int M, int NC, bool LIE6 = true> HD void riccati_instance(const
     }
     SYNC();
   }
-  for (int k = T - 1; k >= 0; k--) {
+  for (int k = K1 - 1; k >= K0; k--) {
     const double *gAB = io.AB + (size_t)k * N * NZ, *gH = io.H + (size_t)k * NZ * NZ;
     const int nca = io.nca[k];
     if (k >= 2) { // the loads below are on the knot's critical path: pull the blocks of knot k - 2 from HBM into L2 now
@@ -221,9 +233,11 @@ template <int N, int M, int NC, bool LIE6 = true> HD void riccati_instance(const
   }
   // ---- forward sweep, dx0 = 0 (force_initial_condition, fulldynamic_talos.py:384)
   double acc = 0.0; // per-thread partial of the merit directional derivative
-  PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
+  if (SEEDED) {
+    PAR_FOR(i, N) { dx[i] = io.dx0[i]; if (K0 == 0) { io.dxs[i] = io.dx0[i]; io.dlams[i] = -p[i]; } }
+  } else PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
   SYNC();
-  for (int k = 0; k <= T; k++) {
+  for (int k = K0; k <= (last ? T : K1 - 1); k++) {
     const int nca = io.nca[k];
     const int32_t *ai = io.act_idx + (size_t)k * NC;
     const double *gdb = io.dbar + (size_t)k * NC, *gvp = io.vplus + (size_t)k * NC, *gv = io.v + (size_t)k * NC;

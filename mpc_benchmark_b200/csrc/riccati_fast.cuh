@@ -57,11 +57,14 @@ template <int N, int M, int NC, int NCAP = NC> struct RicFastLayout {
   static constexpr int total = ZP * LDH + un + vecs;
 };
 
-template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(const RiccatiIO &io, double *ws) {
+// SEEDED: one leg [io.k0, io.k1) of the time-parallel solve, as riccati_instance<..., SEEDED> (riccati.cuh)
+template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void riccati_instance_fast(const RiccatiIO &io, double *ws) {
   using Lay = RicFastLayout<N, M, NC, NCAP>;
   constexpr int NZ = Lay::NZ, NR = Lay::NR, S = Lay::S, ZP = Lay::ZP, LDN = Lay::LDN, LDH = Lay::LDH, LDW = Lay::LDW, LDZ = Lay::LDZ, NBLK = Lay::NBLK, MR = Lay::MR, LDR = Lay::LDR;
   static_assert(N % 8 == 0, "fast Riccati needs n % 8 == 0");
   const int T = io.T;
+  const int K0 = SEEDED ? io.k0 : 0, K1 = SEEDED ? io.k1 : T;
+  const bool seeded = SEEDED && io.seedP != nullptr, last = !SEEDED || K1 == T;
   const double mu = io.mu, mu_d = io.mu_d;
   PHASE_DECL;
   // ---- carve shared memory
@@ -78,7 +81,11 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
   // ---- zero the padding of H once; terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C' d/mu
   PAR_FOR(e, ZP * LDH) H[e] = 0.0;
   SYNC();
-  {
+  if (seeded) {
+    PAR_FOR(e, N * N) H[(e / N) * LDH + e % N] = io.seedP[e];
+    PAR_FOR(i, N) p[i] = io.seedp[i];
+    SYNC();
+  } else {
     const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ;
     const int nca = io.nca[T];
     const double *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
@@ -111,15 +118,15 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
   auto prefetch_knot = [&](int kk) {
     ONE_THREAD { PREFETCH_L2(io.AB + (size_t)kk * N * NZ, N * NZ * 8); PREFETCH_L2(io.H + (size_t)kk * NZ * NZ, NZ * NZ * 8); }
   };
-  if (T > 0) { stage_small(T - 1); prefetch_knot(T - 1); }
-  for (int k = T - 1; k >= 0; k--) {
+  if (K1 > K0) { stage_small(K1 - 1); prefetch_knot(K1 - 1); }
+  for (int k = K1 - 1; k >= K0; k--) {
     const double *gH = io.H + (size_t)k * NZ * NZ, *gAB = io.AB + (size_t)k * N * NZ;
     double *gW = io.W + (size_t)k * N * LDW;
     const int nca = io.nca[k];
-    if (k > 0) prefetch_knot(k - 1);
+    if (k > K0) prefetch_knot(k - 1);
     // 1. ONE pass over the value Hessian left in H by the previous knot: P <- T' H T (E normalisation: T = blockdiag(T6, I)
     //    touches the 6 base rows / columns only), G <- I + mu_d P, and the normalised gradient tmp <- T' p
-    MBAR_WAIT(mbar + 2, (T - 1 - k) & 1); // T6 and fbar of this knot (issued one knot ahead)
+    MBAR_WAIT(mbar + 2, (K1 - 1 - k) & 1); // T6 and fbar of this knot (issued one knot ahead)
     PHASE(21);
     PAR_FOR(e, N * N) { // rows / columns >= 6: a plain copy — the value update mirrors its upper blocks, H is symmetric up to rounding inside the diagonal blocks
       const int i = e / N, j = e % N;
@@ -160,7 +167,7 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
     matvec_rows(P, LDN, N, N, fb, tmp, pv);
     SYNC();
     PAR_FOR(i, N) PV[8 * i] = pv[i];
-    if (k > 0) stage_small(k - 1); // T6 and fbar of this knot are consumed
+    if (k > K0) stage_small(k - 1); // T6 and fbar of this knot are consumed
     PHASE(1);
     // 2. G = chol(I + mu_d P)
     chol_mma<NBLK>(G, LDN, dinv_s);
@@ -170,7 +177,7 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
     PHASE(4);
     // 4. W = Pt [A B] into shared memory (for the Hessian update) and straight from the accumulators to HBM (for the forward
     //    sweep); pt rides in the first padding column of W, so [A B]' pt falls out of the Hessian update
-    MBAR_WAIT(mbar + 3, (T - 1 - k) & 1); // [A B]_k
+    MBAR_WAIT(mbar + 3, (K1 - 1 - k) & 1); // [A B]_k
     mma_tn_g<N, false, false>(NBLK, ZP / 8, P, LDN, N, ABs, LDZ, ZP, Ws, LDZ, nullptr, 0, 0, 0, false, gW, LDW, ZP);
     PHASE(17);
     PAR_FOR(i, N) { const double v = PV[8 * i]; pt[i] = v; Ws[i * LDZ + NZ] = v; gW[i * LDW + NZ] = v; io.pt[(size_t)k * N + i] = v; }
@@ -283,10 +290,13 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
   // ---- forward sweep, dx0 = 0 (force_initial_condition, fulldynamic_talos.py:384)
   PHASE(13);
   double acc = 0.0;
-  PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
+  if (SEEDED) {
+    PAR_FOR(i, N) { dx[i] = io.dx0[i]; if (K0 == 0) { io.dxs[i] = io.dx0[i]; io.dlams[i] = -p[i]; } }
+  } else PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
   // everything that does not depend on the sequential chain is done for all knots at once: default multiplier steps
   // dv = dbar / mu of the inactive rows and their part of the directional derivative
-  PAR_FOR(e, (T + 1) * NC) {
+  PAR_FOR(e_, ((last ? T + 1 : K1) - K0) * NC) {
+    const int e = K0 * NC + e_;
     const int kk = e / NC, r = e % NC, na = io.nca[kk];
     const int32_t *ak = io.act_idx + (size_t)kk * NC;
     const double db = io.dbar[e];
@@ -326,8 +336,8 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
   };
   auto stage_kx = [&](int kk) {
     ONE_THREAD {
-      double *bk = ws + FWA + (kk & 1) * FKX, *bx = bk + KROWS * NR;
-      unsigned long long *bar = mbar + 4 + (kk & 1);
+      double *bk = ws + FWA + ((kk - K0) & 1) * FKX, *bx = bk + KROWS * NR;
+      unsigned long long *bar = mbar + 4 + ((kk - K0) & 1);
       int rows = M + io.nca[kk];
       if (rows > KROWS) rows = KROWS;
       rows = (rows + 1) & ~1; // whole 16-byte units (an extra row stays inside this knot's gain block)
@@ -343,15 +353,15 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
     }
   };
   SYNC();
-  for (int kk = 0; kk < PF && kk < T; kk++) prefetch_fwd(kk);
-  if (T > 0) { stage_kx(0); stage_wa(0); }
-  if (T > 1) stage_kx(1);
-  for (int k = 0; k < T; k++) {
+  for (int kk = K0; kk < K0 + PF && kk < K1; kk++) prefetch_fwd(kk);
+  if (K1 > K0) { stage_kx(K0); stage_wa(K0); }
+  if (K1 > K0 + 1) stage_kx(K0 + 1);
+  for (int k = K0; k < K1; k++) {
     const int nca = io.nca[k];
-    if (k + PF < T) prefetch_fwd(k + PF);
-    const double *sW = ws, *sAB = ws + N * LDW, *sK = ws + FWA + (k & 1) * FKX, *sX = sK + KROWS * NR;
+    if (k + PF < K1) prefetch_fwd(k + PF);
+    const double *sW = ws, *sAB = ws + N * LDW, *sK = ws + FWA + ((k - K0) & 1) * FKX, *sX = sK + KROWS * NR;
     const double *gK = io.K + (size_t)k * S * NR;
-    MBAR_WAIT(mbar + 4 + (k & 1), (k >> 1) & 1); // gain rows and vectors of knot k (each barrier is used every other knot)
+    MBAR_WAIT(mbar + 4 + ((k - K0) & 1), ((k - K0) >> 1) & 1); // gain rows and vectors of knot k (each barrier is used every other knot)
     // du, dv of the active rows: RA rows per warp at a time (independent reduction chains), columns over lanes
     constexpr int RA = 3;
     for (int base = WARP_ID * RA; base < M + nca; base += NWARPS * RA) {
@@ -390,7 +400,7 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
       }
     }
     PAR_FOR(i, NZ) acc += sX[4 * N + i] * z[i];
-    MBAR_WAIT(mbar + 6, k & 1); // W_k, [A B]_k
+    MBAR_WAIT(mbar + 6, (k - K0) & 1); // W_k, [A B]_k
     // dlam_{k+1} = pt + W z ; tmp = A dx + B du + fbar - mu_d dlam : RB rows per warp at a time
     constexpr int RB = 7;
     for (int base = WARP_ID * RB; base < N; base += NWARPS * RB) {
@@ -418,7 +428,7 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
       }
     }
     SYNC();
-    if (k + 1 < T) stage_wa(k + 1); // the W / [A B] stage is free
+    if (k + 1 < K1) stage_wa(k + 1); // the W / [A B] stage is free
     PAR_FOR(i, N) {
       double v;
       if (i < 6) { v = 0; for (int l = 0; l < 6; l++) v += sX[4 * N + NZ + 6 * i + l] * tmp[l]; } else v = tmp[i];
@@ -426,9 +436,9 @@ template <int N, int M, int NC, int NCAP = NC> HD void riccati_instance_fast(con
     }
     PHASE(20);
     SYNC();
-    if (k + 2 < T) stage_kx(k + 2); // this knot's gain / vector stage is free
+    if (k + 2 < K1) stage_kx(k + 2); // this knot's gain / vector stage is free
   }
-  { // terminal knot: dv of the active terminal rows and the terminal cost gradient
+  if (last) { // terminal knot: dv of the active terminal rows and the terminal cost gradient
     const int nca = io.nca[T];
     const int32_t *ai = io.act_idx + (size_t)T * NC;
     const double *gdb = io.dbar + (size_t)T * NC, *gvp = io.vplus + (size_t)T * NC, *gv = io.v + (size_t)T * NC;

@@ -81,6 +81,20 @@ template <int KIND> __global__ void __launch_bounds__(256) k_riccati(Ws w, const
   riccati_dispatch<KIND>(w, list[blockIdx.x], reinterpret_cast<double *>(smem_raw));
 }
 
+// time-parallel LQ solve (lq_legs >= 2, riccati_par.cuh): A and C one CTA per (instance, leg), B and D one CTA per instance
+template <int KIND> __global__ void __launch_bounds__(256) k_ric_par_legs(Ws w, LegWs lw, const int32_t *list) {
+  ric_par_legs<KIND>(w, lw, list[blockIdx.x / lw.L], blockIdx.x % lw.L);
+}
+template <int KIND> __global__ void __launch_bounds__(256) k_ric_par_consensus(Ws w, LegWs lw, const int32_t *list) {
+  __shared__ double sh[64];
+  ric_par_consensus<KIND>(w, lw, list[blockIdx.x], sh);
+}
+template <int KIND> __global__ void __launch_bounds__(256) k_ric_par_resolve(Ws w, LegWs lw, const int32_t *list) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  ric_par_resolve<KIND>(w, lw, list[blockIdx.x / lw.L], blockIdx.x % lw.L, reinterpret_cast<double *>(smem_raw));
+}
+template <int KIND> __global__ void k_ric_par_finish(Ws w, LegWs lw, const int32_t *list) { ric_par_finish<KIND>(w, lw, list[blockIdx.x]); }
+
 __global__ void k_apply_step(Ws w, const int32_t *list) {
   if (blockIdx.x == 0 && threadIdx.x == 0) w.counters[0] = 0; // next linesearch list starts empty
   apply_step(w, list[blockIdx.x]);
@@ -205,6 +219,11 @@ struct mpc_solver {
   int gait_t = 0;
   bool gait_ready = false;
   int tail_mode = 0; // warm start of the knot appended by mpc_tick (mpc_set_tail_warmstart)
+  // time-parallel LQ solve: legs requested by the configuration (0 / 1: serial) and the per-(instance, leg) blocks, allocated on
+  // first need for lw.L legs
+  int lq_legs = 0;
+  LegWs lw{};
+  size_t leg_bytes = 0;
 };
 
 struct CudaBackend {
@@ -231,8 +250,14 @@ struct CudaBackend {
   void riccati(const int32_t *list, int n) {
     mark(1);
     dispatch_kind(h->w.kind, [&](auto kind) {
-      using K = KindTraits<decltype(kind)::value>;
-      k_riccati<decltype(kind)::value><<<n, K::ric_threads(n, h->num_sms), K::ric_smem, s>>>(h->w, list);
+      constexpr int KIND = decltype(kind)::value;
+      using K = KindTraits<KIND>;
+      if (h->lq_legs < 2) { k_riccati<KIND><<<n, K::ric_threads(n, h->num_sms), K::ric_smem, s>>>(h->w, list); return; }
+      const LegWs &lw = h->lw;
+      k_ric_par_legs<KIND><<<n * lw.L, 256, 0, s>>>(h->w, lw, list);
+      k_ric_par_consensus<KIND><<<n, 256, 0, s>>>(h->w, lw, list);
+      k_ric_par_resolve<KIND><<<n * lw.L, K::ric_threads(n * lw.L, h->num_sms), K::ric_smem, s>>>(h->w, lw, list);
+      k_ric_par_finish<KIND><<<n, 32, 0, s>>>(h->w, lw, list);
     });
   }
   void rollout_ls(const int32_t *list, int n, int32_t *next_eval) {
@@ -262,6 +287,7 @@ static int set_kernel_attrs(mpc_solver *h) {
     CK(cudaFuncSetAttribute(k_eval<KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EvalShape<KIND, false>::G * EvalShape<KIND, false>::slice)));
     CK(cudaFuncSetAttribute(k_rollout_ls<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RolloutShape<KIND>::smem));
     CK(cudaFuncSetAttribute(k_riccati<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, KindTraits<KIND>::ric_smem));
+    CK(cudaFuncSetAttribute(k_ric_par_resolve<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, KindTraits<KIND>::ric_smem));
     return 0;
   });
 }
@@ -301,15 +327,40 @@ extern "C" {
 
 const char *mpc_last_error(void) { return g_err.c_str(); }
 
+// lq_legs: 0 / 1 serial, else 2 .. min(16, T) legs
+static const char *check_lq_legs(const mpc_config_t *cfg) {
+  if (cfg->lq_legs < 0) return "lq_legs must not be negative";
+  if (cfg->lq_legs > 16) return "lq_legs must be at most 16";
+  if (cfg->lq_legs > cfg->T) return "lq_legs must not exceed the horizon T";
+  return nullptr;
+}
+// the per-(instance, leg) blocks of the time-parallel LQ solve for the handle's lq_legs (allocated before the first run that needs them)
+static int ensure_leg_ws(mpc_solver *h) {
+  if (h->lq_legs < 2 || h->lw.L == h->lq_legs) return 0;
+  free_leg_ws(h->lw, [](void *p) { cudaFree(p); });
+  h->leg_bytes = 0;
+  bool ok = true;
+  const size_t bytes = alloc_leg_ws(h->w, h->lw, h->lq_legs, [&](size_t b) -> void * {
+    void *p = nullptr;
+    if (!ok || cudaMalloc(&p, b ? b : 8) != cudaSuccess) { ok = false; return nullptr; }
+    return p;
+  });
+  if (!ok) { free_leg_ws(h->lw, [](void *p) { cudaFree(p); }); return fail("cudaMalloc(lq_legs workspace) failed: batch x lq_legs too large for this GPU"); }
+  h->leg_bytes = bytes;
+  return 0;
+}
+
 mpc_solver_t *mpc_create(const mpc_robot_t *robot, const mpc_config_t *cfg, int32_t batch, int32_t device) {
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { g_err = "no CUDA device: libmpcb200 has no CPU fallback"; return nullptr; }
   if (!robot || !cfg) { g_err = "mpc_create: null robot / config"; return nullptr; }
   if (cfg->kind != MPC_KIND_FULL && cfg->kind != MPC_KIND_CENT && cfg->kind != MPC_KIND_KINO) { g_err = "unknown model kind"; return nullptr; }
   if (batch <= 0 || cfg->T <= 0) { g_err = "mpc_create: batch and horizon must be positive"; return nullptr; }
+  if (const char *le = check_lq_legs(cfg)) { g_err = std::string("mpc_create: ") + le; return nullptr; }
   if (cudaSetDevice(device) != cudaSuccess) { g_err = "cudaSetDevice failed"; return nullptr; }
   mpc_solver *h = new mpc_solver;
   h->device = device;
+  h->lq_legs = cfg->lq_legs;
   const char *err = nullptr;
   if (build_dev_model(robot, cfg, &h->h_model, &err)) { g_err = err; delete h; return nullptr; }
   // every failure below releases what was created so far through mpc_destroy (all members start null)
@@ -330,6 +381,7 @@ void mpc_destroy(mpc_solver_t *h) {
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (void *p : h->allocs) cudaFree(p);
+  free_leg_ws(h->lw, [](void *p) { cudaFree(p); });
   for (cudaEvent_t e : h->evpool) cudaEventDestroy(e);
   if (h->d_xs_in) cudaFree(h->d_xs_in);
   if (h->d_us_in) cudaFree(h->d_us_in);
@@ -437,8 +489,10 @@ int32_t mpc_shift_multipliers(mpc_solver_t *h, int32_t n) {
 int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_config_t *cfg) {
   CK(cudaSetDevice(h->device));
   if (cfg->kind != h->w.kind || cfg->T != h->w.T) return fail("mpc_reconfigure: kind / horizon must not change");
+  if (const char *le = check_lq_legs(cfg)) return fail(std::string("mpc_reconfigure: ") + le);
   const char *err = nullptr;
   if (build_dev_model(robot, cfg, &h->h_model, &err)) return fail(err);
+  h->lq_legs = cfg->lq_legs;
   h->w.sc = default_consts(cfg->tol, cfg->mu_init, cfg->rollout);
   CK(cudaMemcpyAsync(h->d_model, &h->h_model, sizeof(DevModel), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
@@ -455,6 +509,7 @@ int32_t mpc_set_x0(mpc_solver_t *h, const double *x0) {
 
 static int run_impl(mpc_solver *h, const double *d_xs, const double *d_us, int max_iters, cudaStream_t s, bool sync_events) {
   if (!h->setup_done) return fail("mpc_run before mpc_setup");
+  if (ensure_leg_ws(h)) return 1;
   CK(cudaEventRecord(h->ev0, s));
   h->evcat.clear();
   CudaBackend be{h, s};
@@ -559,6 +614,7 @@ int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *
                           double *us_out, double *K0_out, mpc_info_t *info_out) {
   CK(cudaSetDevice(h->device));
   if (!h->setup_done) return fail("mpc_run_pipelined before mpc_setup");
+  if (ensure_leg_ws(h)) return 1;
   Ws &w = h->w;
   const size_t T1 = w.T + 1, sx = T1 * w.nx, su = (size_t)w.T * w.m, sk = (size_t)w.m * w.n;
   if (parts < 1) parts = 1;
@@ -687,7 +743,7 @@ int32_t mpc_get_feedback(mpc_solver_t *h, int32_t k, double *K) {
   return 0;
 }
 double mpc_last_device_ms(mpc_solver_t *h) { return h->last_ms; }
-uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return h->bytes; }
+uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return h->bytes + h->leg_bytes; }
 // per-phase cycle counters of the Riccati kernel for instance 0 (all zero unless built with -DMPC_PHASE_TIMING)
 int32_t mpc_debug_phases(mpc_solver_t *h, double *out64) {
   CK(cudaSetDevice(h->device));

@@ -12,6 +12,7 @@
 #include "eval_kino.cuh"
 #include "riccati.cuh"
 #include "riccati_fast.cuh"
+#include "riccati_par.cuh"
 
 namespace mpcdev {
 
@@ -273,6 +274,8 @@ template <> struct KindTraits<MPC_KIND_FULL> {
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_full_knot<D, ROLL>(md, io, f); }
   template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_mb_term<D, true, FNZ, FNC>(md, io, f); }
   static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
+  static HD void riccati_seeded(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap, true>(r, smem); }
+  static constexpr bool lie6 = true;
   static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
   // two 128-thread instances per SM when the launch fills the GPU; 256 threads per instance when SMs would idle (latency)
   static constexpr int ric_threads(int count, int num_sms) { return count <= num_sms ? 256 : 128; }
@@ -284,6 +287,8 @@ template <> struct KindTraits<MPC_KIND_KINO> {
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_kino_knot<D, ROLL>(md, io, f); }
   template <bool D> static HD void term(const DevModel &md, const KnotIO &io, EvalWs<D> &f) { eval_mb_term<D, false, KNZ, KNC>(md, io, f); }
   static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap>(r, smem); }
+  static HD void riccati_seeded(const RiccatiIO &r, double *smem) { riccati_instance_fast<n, m, nc, ncap, true>(r, smem); }
+  static constexpr bool lie6 = true;
   static constexpr int ric_smem = RicFastLayout<n, m, nc, ncap>::total * 8, ric_scratch = RicFastLayout<n, m, nc, ncap>::scratch;
   static constexpr int ric_threads(int, int) { return 256; }
 };
@@ -294,6 +299,8 @@ template <> struct KindTraits<MPC_KIND_CENT> {
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_knot<D, ROLL>(md, io, f); }
   template <bool D> static HD void term(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_term<D>(md, io, f); }
   static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, false>(r, smem); }
+  static HD void riccati_seeded(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, false, true>(r, smem); }
+  static constexpr bool lie6 = false;
   static constexpr int ric_smem = riccati_smem_doubles<n, m, nc>() * 8, ric_scratch = 2; // no global scratch: a token block
   static constexpr int ric_threads(int, int) { return 128; }
 };
@@ -424,6 +431,61 @@ template <int KIND> HD void riccati_dispatch(const Ws &w, int b, double *smem) {
   if (w.st[b].mode != MODE_STEP) return;
   KindTraits<KIND>::riccati(make_riccati_io(w, b), smem);
   ONE_THREAD { if (w.overflow[b]) { w.st[b].status = 3; w.st[b].mode = MODE_DONE; w.overflow[b] = 0; } }
+  SYNC();
+  start_linesearch(w, b);
+}
+
+// ---- time-parallel LQ solve (riccati_par.cuh), lq_legs = L >= 2: per-(instance, leg) blocks, indexed b * L + j
+struct LegWs {
+  int L;
+  double *sum, *ws, *buf, *scratch; // LegLayout::sum / ::ws / ::buf and KindTraits::ric_scratch doubles per (instance, leg)
+};
+template <int KIND> struct LegDims {
+  using K = KindTraits<KIND>;
+  using Lay = LegLayout<K::n, K::m, K::nc>;
+};
+// phase A: leg j of instance b
+template <int KIND> HD void ric_par_legs(const Ws &w, const LegWs &lw, int b, int j) {
+  using K = KindTraits<KIND>;
+  using Lay = typename LegDims<KIND>::Lay;
+  if (w.st[b].mode != MODE_STEP) return;
+  const size_t i = (size_t)b * lw.L + j;
+  ric_leg_param<K::n, K::m, K::nc, K::lie6>(make_riccati_io(w, b), leg_start(w.T, lw.L, j), leg_start(w.T, lw.L, j + 1), j + 1 == lw.L, lw.ws + i * Lay::ws,
+                                             lw.sum + i * Lay::sum);
+}
+// phase B: the boundaries of instance b.  sh: >= n doubles of shared memory
+template <int KIND> HD void ric_par_consensus(const Ws &w, const LegWs &lw, int b, double *sh) {
+  using K = KindTraits<KIND>;
+  using Lay = typename LegDims<KIND>::Lay;
+  if (w.st[b].mode != MODE_STEP) return;
+  const size_t i = (size_t)b * lw.L;
+  ric_consensus<K::n, K::m, K::nc>(lw.L, lw.sum + i * Lay::sum, Lay::sum, lw.buf + i * Lay::buf, Lay::buf, sh);
+}
+// phase C: exact re-solve of leg j of instance b with the model's Riccati kernel.  smem: KindTraits::ric_smem bytes
+template <int KIND> HD void ric_par_resolve(const Ws &w, const LegWs &lw, int b, int j, double *smem) {
+  using K = KindTraits<KIND>;
+  using Lay = typename LegDims<KIND>::Lay;
+  if (w.st[b].mode != MODE_STEP) return;
+  const size_t i = (size_t)b * lw.L + j;
+  double *bf = lw.buf + i * Lay::buf;
+  RiccatiIO r = make_riccati_io(w, b);
+  r.k0 = leg_start(w.T, lw.L, j); r.k1 = leg_start(w.T, lw.L, j + 1);
+  r.seedP = (j + 1 < lw.L) ? bf : nullptr; r.seedp = bf + Lay::off_seedp; r.dx0 = bf + Lay::off_x;
+  r.dphi = bf + Lay::off_dphi;
+  r.scratch = lw.scratch + i * K::ric_scratch;
+  r.phase_out = (b == 0 && j == 0) ? w.phase : nullptr;
+  K::riccati_seeded(r, smem);
+}
+// phase D: the legs' merit derivative partials in leg order, then what riccati_dispatch does after the serial kernel
+template <int KIND> HD void ric_par_finish(const Ws &w, const LegWs &lw, int b) {
+  using Lay = typename LegDims<KIND>::Lay;
+  if (w.st[b].mode != MODE_STEP) return;
+  ONE_THREAD {
+    double s = 0;
+    for (int j = 0; j < lw.L; j++) s += lw.buf[((size_t)b * lw.L + j) * Lay::buf + Lay::off_dphi];
+    w.dphi[b] = s;
+    if (w.overflow[b]) { w.st[b].status = 3; w.st[b].mode = MODE_DONE; w.overflow[b] = 0; }
+  }
   SYNC();
   start_linesearch(w, b);
 }

@@ -60,4 +60,23 @@ template <class Free> void free_ws(Ws &w, Free &&fr) {
   for (void *p : ptrs) if (p) fr(p);
 }
 
+// the time-parallel LQ solve's per-(instance, leg) blocks for `legs` legs (lq_legs >= 2), allocated on first need; returns bytes
+template <class Alloc> size_t alloc_leg_ws(const Ws &w, LegWs &lw, int legs, Alloc &&alloc) {
+  size_t sz[4];
+  dispatch_kind(w.kind, [&](auto k) {
+    using Lay = typename LegDims<decltype(k)::value>::Lay;
+    sz[0] = Lay::sum; sz[1] = Lay::ws; sz[2] = Lay::buf; sz[3] = KindTraits<decltype(k)::value>::ric_scratch;
+  });
+  const size_t n = (size_t)w.B * legs;
+  double **p[4] = {&lw.sum, &lw.ws, &lw.buf, &lw.scratch};
+  size_t total = 0;
+  for (int i = 0; i < 4; i++) { *p[i] = (double *)alloc(n * sz[i] * 8); total += n * sz[i] * 8; }
+  lw.L = legs;
+  return total;
+}
+template <class Free> void free_leg_ws(LegWs &lw, Free &&fr) {
+  for (double *p : {lw.sum, lw.ws, lw.buf, lw.scratch}) if (p) fr(p);
+  lw = LegWs{};
+}
+
 } // namespace mpcdev

@@ -412,8 +412,9 @@ def _flatten_kino(problem, tol, mu_init, max_iters):
     return FlatProblem(rb, c, knots, terms, np.array(problem.x0_init, float).reshape(1, -1))
 
 
-def flatten_problem(problem, tol, mu_init, max_iters, rollout=0):
-    """rollout: solver.rollout_type (0 = ROLLOUT_LINEAR, fulldynamic_talos.py:381; 1 = ROLLOUT_NONLINEAR)."""
+def flatten_problem(problem, tol, mu_init, max_iters, rollout=0, lq_legs=0):
+    """rollout: solver.rollout_type (0 = ROLLOUT_LINEAR, fulldynamic_talos.py:381; 1 = ROLLOUT_NONLINEAR).
+    lq_legs: 0 or 1 = serial LQ solve, 2..min(16, T) = time-parallel LQ solve over that many horizon legs (mpc_config_t.lq_legs)."""
     if not problem.stages:
         raise ValueError("TrajOptProblem has no stages")
     ode = problem.stages[0].dynamics.differential_dynamics
@@ -426,4 +427,5 @@ def flatten_problem(problem, tol, mu_init, max_iters, rollout=0):
     else:
         raise NotImplementedError(f"unsupported dynamics {type(ode).__name__}")
     flat.cfg.rollout = int(rollout)
+    flat.cfg.lq_legs = int(lq_legs)
     return flat
