@@ -69,7 +69,6 @@ struct RiccatiIO {
   double *Kfb;           // [T][M][N]        controlFeedbacks()
   double *dxs, *dus, *dvs, *dlams; // [T+1][N], [T][M], [T+1][NC], [T+1][N]
   double *dphi;          // scalar
-  int32_t *overflow;     // set to 1 when a knot has more active rows than the kernel's shared-memory capacity
   double *scratch;       // per-instance global block for the KKT buffers of knots whose active rows exceed the shared-memory carving
   double *phase_out;     // optional 16 per-phase cycle counters (MPC_PHASE_TIMING builds), else nullptr
   // SEEDED solves (one leg of the time-parallel solve, riccati_par.cuh): knots [k0, k1) only, backward from the value function
@@ -77,6 +76,89 @@ struct RiccatiIO {
   int k0, k1;
   const double *seedP, *seedp, *dx0;
 };
+
+// ------------------------------------------------------------------ steps shared by the Riccati kernels (riccati_instance,
+// riccati_instance_fast, ric_leg_param); they differ only in leading dimensions and buffer placement
+// terminal value function: P = H_T[xx] + C'C/mu (leading dimension ldp), p = g_T[x] + C'd/mu (stride ps)
+template <int N, int M, int NC> HD void ric_terminal_value(const RiccatiIO &io, double *P, int ldp, double *p, int ps) {
+  constexpr int NZ = N + M;
+  const int T = io.T;
+  const double mu = io.mu;
+  const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ;
+  const int nca = io.nca[T];
+  const double *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
+  const int32_t *ai = io.act_idx + (size_t)T * NC;
+  PAR_FOR(e, N * N) {
+    int i = e / N, j = e % N;
+    double s = HT[i * NZ + j];
+    for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * CT[r * NZ + j] / mu;
+    P[i * ldp + j] = s;
+  }
+  PAR_FOR(i, N) {
+    double s = gT[i];
+    for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * dT[ai[r]] / mu;
+    p[i * ps] = s;
+  }
+}
+
+// value function the backward sweep starts from: the seed (RiccatiIO::seedP) of a seeded leg, else the terminal value function
+template <int N, int M, int NC> HD void ric_start_value(const RiccatiIO &io, bool seeded, double *P, int ldp, double *p) {
+  if (seeded) {
+    PAR_FOR(e, N * N) P[(e / N) * ldp + e % N] = io.seedP[e];
+    PAR_FOR(i, N) p[i] = io.seedp[i];
+    SYNC();
+  } else {
+    ric_terminal_value<N, M, NC>(io, P, ldp, p, 1);
+    SYNC();
+  }
+}
+
+// KKT by block elimination, after Z (M rows, leading dimension ldz) <- R^-1 [gh_u (na columns) | Sh' (N) | D' (nca)], nk = na + N:
+// Schur complement Sg = mu I + D Z_D;  right-hand side Kv = [dbar | 0 | C] - D Z[:, 0:nk] (nca x nk).  CD: the active rows (NZ wide).
+// THETA: na may exceed 1 (the co-state columns of ric_leg_param); the serial kernels pass na = 1
+template <int N, int M, bool THETA = false>
+HD void ric_kkt_schur(int nca, int na, int nk, double mu, const double *CD, const double *dbr, const double *Z, int ldz, double *Sg, double *Kv) {
+  constexpr int NZ = N + M;
+  PAR_FOR(e, nca * nca) {
+    int r = e / nca, c = e % nca;
+    double s = (r == c) ? mu : 0.0;
+    for (int l = 0; l < M; l++) s += CD[r * NZ + N + l] * Z[l * ldz + nk + c];
+    Sg[e] = s;
+  }
+  PAR_FOR(e, nca * nk) {
+    int r = e / nk, c = e % nk;
+    double s = (c == 0) ? dbr[r] : ((THETA && c < na) ? 0.0 : CD[r * NZ + c - na]);
+    for (int l = 0; l < M; l++) s -= CD[r * NZ + N + l] * Z[l * ldz + c];
+    Kv[e] = s;
+  }
+  SYNC();
+}
+// ... then, once Kv <- Sg^-1 Kv:  [ku | Ku] = -Z0 - Z_D Kv  (into Z0's place)
+template <int M> HD void ric_kkt_ku(int nca, int nk, double *Z, int ldz, const double *Kv) {
+  PAR_FOR(e, M * nk) {
+    int i = e / nk, c = e % nk;
+    double s = -Z[i * ldz + c];
+    for (int r = 0; r < nca; r++) s -= Z[i * ldz + nk + r] * Kv[r * nk + c];
+    Z[i * ldz + c] = s;
+  }
+  SYNC();
+}
+
+// store the gains of knot k: rows 0..M-1 = [ku | Ku] (and Ku into Kfb), rows M.. = [kv | Kv] (active rows, compact)
+template <int N, int M, int NC> HD void ric_store_gains(const RiccatiIO &io, int k, const double *Z, int ldz, const double *Kv, int nca) {
+  constexpr int NR = 1 + N, S = M + NC;
+  double *gK = io.K + (size_t)k * S * NR;
+  PAR_FOR(e, M * NR) { int i = e / NR, c = e % NR; double v = Z[i * ldz + c]; gK[e] = v; if (c > 0) io.Kfb[((size_t)k * M + i) * N + c - 1] = v; }
+  PAR_FOR(e, nca * NR) gK[M * NR + e] = Kv[e];
+}
+
+// forward sweep start: dx = dx0 of a SEEDED leg, else 0 (force_initial_condition, fulldynamic_talos.py:384); knot k0 = 0 also writes
+// dxs_0 and dlams_0 = -p
+template <int N, bool SEEDED> HD void ric_forward_start(const RiccatiIO &io, int K0, const double *p, double *dx) {
+  if (SEEDED) {
+    PAR_FOR(i, N) { dx[i] = io.dx0[i]; if (K0 == 0) { io.dxs[i] = io.dx0[i]; io.dlams[i] = -p[i]; } }
+  } else PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
+}
 
 template <int N, int M, int NC> constexpr int riccati_smem_doubles() {
   constexpr int NZ = N + M, NR = 1 + N;
@@ -105,29 +187,7 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
   double *vec = U0 + (phase1 > phase2 ? phase1 : phase2);
   double *p = vec, *pt = p + NZ, *gh = pt + NZ, *fb = gh + NZ, *tmp = fb + NZ, *dx = tmp + NZ, *z = dx + NZ, *dl = z + NZ;
   double *T6 = dl + NZ, *dbr = T6 + 36, *dva = dbr + NC, *red = dva + NC, *dinv = red + 512;
-  // ---- terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C' d/mu
-  if (seeded) {
-    PAR_FOR(e, N * N) H[(e / N) * NZ + e % N] = io.seedP[e];
-    PAR_FOR(i, N) p[i] = io.seedp[i];
-    SYNC();
-  } else {
-    const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ;
-    const int nca = io.nca[T];
-    const double *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
-    const int32_t *ai = io.act_idx + (size_t)T * NC;
-    PAR_FOR(e, N * N) {
-      int i = e / N, j = e % N;
-      double s = HT[i * NZ + j];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * CT[r * NZ + j] / mu;
-      H[i * NZ + j] = s;
-    }
-    PAR_FOR(i, N) {
-      double s = gT[i];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * dT[ai[r]] / mu;
-      p[i] = s;
-    }
-    SYNC();
-  }
+  ric_start_value<N, M, NC>(io, seeded, H, NZ, p);
   for (int k = K1 - 1; k >= K0; k--) {
     const double *gAB = io.AB + (size_t)k * N * NZ, *gH = io.H + (size_t)k * NZ * NZ;
     const int nca = io.nca[k];
@@ -189,33 +249,10 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
       chol_blocked(Rh, M, M, dinv);
       trsm_blocked(Rh, M, M, dinv, Z, ncol, ncol);
     }
-    // Schur complement Sg = mu I + D Z_D ; right-hand side Kv = [dbar | C] - D [Z_r | Z_S]
-    PAR_FOR(e, nca * nca) {
-      int r = e / nca, c = e % nca;
-      double s = (r == c) ? mu : 0.0;
-      for (int l = 0; l < M; l++) s += CD[r * NZ + N + l] * Z[l * ncol + NR + c];
-      Sg[e] = s;
-    }
-    PAR_FOR(e, nca * NR) {
-      int r = e / NR, c = e % NR;
-      double s = (c == 0) ? dbr[r] : CD[r * NZ + c - 1];
-      for (int l = 0; l < M; l++) s -= CD[r * NZ + N + l] * Z[l * ncol + c];
-      Kv[e] = s;
-    }
-    SYNC();
+    ric_kkt_schur<N, M>(nca, 1, NR, mu, CD, dbr, Z, ncol, Sg, Kv);
     if (nca > 0) { chol_blocked(Sg, nca, nca, dinv); trsm_blocked(Sg, nca, nca, dinv, Kv, NR, NR); }
-    // Ku = -Z0 - Z_D Kv  (into Z0's place)
-    PAR_FOR(e, M * NR) {
-      int i = e / NR, c = e % NR;
-      double s = -Z[i * ncol + c];
-      for (int r = 0; r < nca; r++) s -= Z[i * ncol + NR + r] * Kv[r * NR + c];
-      Z[i * ncol + c] = s;
-    }
-    SYNC();
-    // store gains: rows 0..M-1 = [ku | Ku], rows M.. = [kv | Kv] (active rows, compact)
-    double *gK = io.K + (size_t)k * S * NR;
-    PAR_FOR(e, M * NR) { int i = e / NR, c = e % NR; double v = Z[i * ncol + c]; gK[e] = v; if (c > 0) io.Kfb[((size_t)k * M + i) * N + c - 1] = v; }
-    PAR_FOR(e, nca * NR) gK[M * NR + e] = Kv[e];
+    ric_kkt_ku<M>(nca, NR, Z, ncol, Kv);
+    ric_store_gains<N, M, NC>(io, k, Z, ncol, Kv, nca);
     // 5. P = Qh + Sh Ku + C' Kv, p = qh + Sh ku + C' kv : in place in H[0:N,0:N] / p, then symmetrise
     PAR_FOR(e, N * NR) {
       int i = e / NR, c = e % NR;
@@ -233,9 +270,7 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
   }
   // ---- forward sweep, dx0 = 0 (force_initial_condition, fulldynamic_talos.py:384)
   double acc = 0.0; // per-thread partial of the merit directional derivative
-  if (SEEDED) {
-    PAR_FOR(i, N) { dx[i] = io.dx0[i]; if (K0 == 0) { io.dxs[i] = io.dx0[i]; io.dlams[i] = -p[i]; } }
-  } else PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
+  ric_forward_start<N, SEEDED>(io, K0, p, dx);
   SYNC();
   for (int k = K0; k <= (last ? T : K1 - 1); k++) {
     const int nca = io.nca[k];

@@ -81,28 +81,7 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
   // ---- zero the padding of H once; terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C' d/mu
   PAR_FOR(e, ZP * LDH) H[e] = 0.0;
   SYNC();
-  if (seeded) {
-    PAR_FOR(e, N * N) H[(e / N) * LDH + e % N] = io.seedP[e];
-    PAR_FOR(i, N) p[i] = io.seedp[i];
-    SYNC();
-  } else {
-    const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ;
-    const int nca = io.nca[T];
-    const double *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
-    const int32_t *ai = io.act_idx + (size_t)T * NC;
-    PAR_FOR(e, N * N) {
-      int i = e / N, j = e % N;
-      double s = HT[i * NZ + j];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * CT[r * NZ + j] / mu;
-      H[i * LDH + j] = s;
-    }
-    PAR_FOR(i, N) {
-      double s = gT[i];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * dT[ai[r]] / mu;
-      p[i] = s;
-    }
-    SYNC();
-  }
+  ric_start_value<N, M, NC>(io, seeded, H, LDH, p);
   // T6 and fbar of a knot arrive by bulk copies one knot ahead (mbar[2]); [A B]_k streams into the H buffer once the value Hessian
   // has been taken out of it (mbar[3]); [A B]_k and H_k are bulk-prefetched into L2 one knot ahead (H_k is read from there as
   // the initial value of the Hessian update's accumulators).
@@ -218,32 +197,12 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     PHASE(7);
     trsm_mma<MR / 8>(Rh, LDR, dinv, Z, ldz, ldz / 8, nullptr, 0, ldz / 8);
     PHASE(8);
-    PAR_FOR(e, nca * nca) {
-      int r = e / nca, c = e % nca;
-      double s = (r == c) ? mu : 0.0;
-      for (int l = 0; l < M; l++) s += CD[r * NZ + N + l] * Z[l * ldz + NR + c];
-      Sg[e] = s;
-    }
-    PAR_FOR(e, nca * NR) {
-      int r = e / NR, c = e % NR;
-      double s = (c == 0) ? dbr[r] : CD[r * NZ + c - 1];
-      for (int l = 0; l < M; l++) s -= CD[r * NZ + N + l] * Z[l * ldz + c];
-      Kv[e] = s;
-    }
-    SYNC();
+    ric_kkt_schur<N, M>(nca, 1, NR, mu, CD, dbr, Z, ldz, Sg, Kv);
     PHASE(9);
     if (nca > 0) { chol_blocked(Sg, nca, nca, dinv); trsm_blocked(Sg, nca, nca, dinv, Kv, NR, NR); }
     PHASE(10);
-    PAR_FOR(e, M * NR) {
-      int i = e / NR, c = e % NR;
-      double s = -Z[i * ldz + c];
-      for (int r = 0; r < nca; r++) s -= Z[i * ldz + NR + r] * Kv[r * NR + c];
-      Z[i * ldz + c] = s;
-    }
-    SYNC();
-    double *gK = io.K + (size_t)k * S * NR;
-    PAR_FOR(e, M * NR) { int i = e / NR, c = e % NR; double v = Z[i * ldz + c]; gK[e] = v; if (c > 0) io.Kfb[((size_t)k * M + i) * N + c - 1] = v; }
-    PAR_FOR(e, nca * NR) gK[M * NR + e] = Kv[e];
+    ric_kkt_ku<M>(nca, NR, Z, ldz, Kv);
+    ric_store_gains<N, M, NC>(io, k, Z, ldz, Kv, nca);
     PHASE(11);
     // 9. P = Qh + Sh Ku + C' Kv, p = qh + Sh ku + C' kv : in place in H[0:N,0:N] / p.
     //    Sh Ku = H[N:, 0:N]' Z[:, 1:] runs on the DMMA pipe (K = MP, zero rows beyond M); the active-row part is usually empty.
@@ -290,9 +249,7 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
   // ---- forward sweep, dx0 = 0 (force_initial_condition, fulldynamic_talos.py:384)
   PHASE(13);
   double acc = 0.0;
-  if (SEEDED) {
-    PAR_FOR(i, N) { dx[i] = io.dx0[i]; if (K0 == 0) { io.dxs[i] = io.dx0[i]; io.dlams[i] = -p[i]; } }
-  } else PAR_FOR(i, N) { dx[i] = 0.0; io.dxs[i] = 0.0; io.dlams[i] = -p[i]; }
+  ric_forward_start<N, SEEDED>(io, K0, p, dx);
   // everything that does not depend on the sequential chain is done for all knots at once: default multiplier steps
   // dv = dbar / mu of the inactive rows and their part of the directional derivative
   PAR_FOR(e_, ((last ? T + 1 : K1) - K0) * NC) {

@@ -49,21 +49,8 @@ template <int N, int M, int NC, bool LIE6> HD void ric_leg_param(const RiccatiIO
   double *G = ws, *Pt = G + N * N, *Pn = Pt + N * N, *ptl = Pn + N * N, *tpa = ptl + N * NA, *AB = tpa + N * NA, *W = AB + N * NZ, *Hh = W + N * NZ;
   double *gh = Hh + NZ * NZ, *Z = gh + NZ * NA, *Rh = Z + M * NK, *CD = Rh + M * M, *Sg = CD + NC * NZ, *Kv = Sg + NC * NC, *dinv = Kv + NC * (NA + N);
   double *T6 = dinv + 64 * Lay::NB, *fb = T6 + 36, *dbr = fb + N; // ptl, gh, Kv: stride na / na / nk
-  if (last) { // terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C'd/mu
-    const int T = io.T, nca = io.nca[T];
-    const double *HT = io.H + (size_t)T * NZ * NZ, *gT = io.g + (size_t)T * NZ, *CT = io.CDact + (size_t)T * NC * NZ, *dT = io.dbar + (size_t)T * NC;
-    const int32_t *ai = io.act_idx + (size_t)T * NC;
-    PAR_FOR(e, N * N) {
-      const int i = e / N, j = e % N;
-      double s = HT[i * NZ + j];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * CT[r * NZ + j] / mu;
-      VP[e] = s;
-    }
-    PAR_FOR(i, N) {
-      double s = gT[i];
-      for (int r = 0; r < nca; r++) s += CT[r * NZ + i] * dT[ai[r]] / mu;
-      pa[i * NA] = s;
-    }
+  if (last) {
+    ric_terminal_value<N, M, NC>(io, VP, N, pa, NA);
   } else {
     PAR_FOR(e, N * N) { VP[e] = 0.0; Psi[e] = 0.0; }
     PAR_FOR(e, N * NA) pa[e] = ((e % NA) == 1 + e / NA) ? 1.0 : 0.0;
@@ -127,27 +114,9 @@ template <int N, int M, int NC, bool LIE6> HD void ric_leg_param(const RiccatiIO
     SYNC();
     chol_blocked(Rh, M, M, dinv);
     trsm_blocked(Rh, M, M, dinv, Z, ncol, ncol);
-    PAR_FOR(e, nca * nca) {
-      const int r = e / nca, c = e % nca;
-      double s = (r == c) ? mu : 0.0;
-      for (int l = 0; l < M; l++) s += CD[r * NZ + N + l] * Z[l * ncol + nk + c];
-      Sg[e] = s;
-    }
-    PAR_FOR(e, nca * nk) {
-      const int r = e / nk, c = e % nk;
-      double s = (c == 0) ? dbr[r] : (c < na ? 0.0 : CD[r * NZ + c - na]);
-      for (int l = 0; l < M; l++) s -= CD[r * NZ + N + l] * Z[l * ncol + c];
-      Kv[e] = s;
-    }
-    SYNC();
+    ric_kkt_schur<N, M, true>(nca, na, nk, mu, CD, dbr, Z, ncol, Sg, Kv);
     if (nca > 0) { chol_blocked(Sg, nca, nca, dinv); trsm_blocked(Sg, nca, nca, dinv, Kv, nk, nk); }
-    PAR_FOR(e, M * nk) { // [ku | Ku_theta | Ku] = -Z - Z_D Kv
-      const int i = e / nk, c = e % nk;
-      double s = -Z[i * ncol + c];
-      for (int r = 0; r < nca; r++) s -= Z[i * ncol + nk + r] * Kv[r * nk + c];
-      Z[i * ncol + c] = s;
-    }
-    SYNC();
+    ric_kkt_ku<M>(nca, nk, Z, ncol, Kv); // [ku | Ku_theta | Ku]
     PAR_FOR(e, nt * nt) { const int a = e / nt, b = e % nt; double u = 0; for (int i = 0; i < M; i++) u += gh[(N + i) * na + 1 + a] * Z[i * ncol + 1 + b]; Psi[a * N + b] += u; }
     PAR_FOR(a, nt) { double t = 0; for (int i = 0; i < M; i++) t += gh[(N + i) * na + 1 + a] * Z[i * ncol]; psi[a] += t; }
     // 5. P = Qh + Sh Ku + C'Kv (symmetrised);  [p | Pi] = gh_x + Sh [ku | Ku_theta] + C'[kv | Kv_theta]

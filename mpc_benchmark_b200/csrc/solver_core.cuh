@@ -59,7 +59,6 @@ struct Ws {
   double *ric_scratch; size_t ric_scratch_stride; // per-instance scratch of the Riccati kernel (doubles per instance)
   InstState *st;
   int32_t *counters; // [0] instances still in MODE_LS (next ls list), [2] instances to evaluate in the next pass
-  int32_t *overflow; // [B] Riccati active-row overflow flags
   double *phase;     // 16 doubles: per-phase cycle counters of instance 0 (MPC_PHASE_TIMING builds)
   int32_t *lists;    // [4][B] compacted instance lists: 0,1 = evaluation lists (double-buffered), 2,3 = linesearch lists
 };
@@ -423,15 +422,12 @@ HD RiccatiIO make_riccati_io(const Ws &w, int b) {
   r.dxs = w.dxs + b * T1 * w.n; r.dus = w.dus + b * T * w.m; r.dvs = w.dvs + b * T1 * w.nc; r.dlams = w.dlams + b * T1 * w.n;
   r.dphi = w.dphi + b;
   r.phase_out = (b == 0) ? w.phase : nullptr;
-  r.overflow = w.overflow + b;
   return r;
 }
 
 template <int KIND> HD void riccati_dispatch(const Ws &w, int b, double *smem) {
   if (w.st[b].mode != MODE_STEP) return;
   KindTraits<KIND>::riccati(make_riccati_io(w, b), smem);
-  ONE_THREAD { if (w.overflow[b]) { w.st[b].status = 3; w.st[b].mode = MODE_DONE; w.overflow[b] = 0; } }
-  SYNC();
   start_linesearch(w, b);
 }
 
@@ -484,7 +480,6 @@ template <int KIND> HD void ric_par_finish(const Ws &w, const LegWs &lw, int b) 
     double s = 0;
     for (int j = 0; j < lw.L; j++) s += lw.buf[((size_t)b * lw.L + j) * Lay::buf + Lay::off_dphi];
     w.dphi[b] = s;
-    if (w.overflow[b]) { w.st[b].status = 3; w.st[b].mode = MODE_DONE; w.overflow[b] = 0; }
   }
   SYNC();
   start_linesearch(w, b);

@@ -49,14 +49,14 @@ template <class Alloc> size_t alloc_ws(Ws &w, Alloc &&alloc) {
   w.ric_scratch_stride = dispatch_kind(w.kind, [](auto kind) { return KindTraits<decltype(kind)::value>::ric_scratch; });
   D(w.ric_scratch, B * w.ric_scratch_stride);
   w.st = (InstState *)alloc(B * sizeof(InstState)); total += B * sizeof(InstState);
-  I(w.counters, 4); I(w.lists, 4 * B); I(w.overflow, B);
+  I(w.counters, 4); I(w.lists, 4 * B);
   return total;
 }
 
 template <class Free> void free_ws(Ws &w, Free &&fr) {
   void *ptrs[] = {w.knots, w.terms, w.x0, w.xs, w.us, w.vs, w.lams, w.vs_prev, w.lams_prev, w.txs, w.tus, w.tvs, w.tlams, w.dxs, w.dus, w.dvs,
                   w.dlams, w.AB, w.H, w.lxu, w.g, w.T6, w.E6, w.gE, w.fbar, w.dbar, w.vplus, w.lplus, w.CDact, w.nca, w.act_idx, w.gap, w.h,
-                  w.scal, w.tscal, w.xdot, w.lamc, w.W, w.pt, w.K, w.Kfb, w.dphi, w.ric_scratch, w.phase, w.st, w.counters, w.lists, w.overflow};
+                  w.scal, w.tscal, w.xdot, w.lamc, w.W, w.pt, w.K, w.Kfb, w.dphi, w.ric_scratch, w.phase, w.st, w.counters, w.lists};
   for (void *p : ptrs) if (p) fr(p);
 }
 

@@ -3,6 +3,7 @@
 // PARITY UNPINNED against upstream Aligator/Pinocchio (absent from /root/reference, README.md:10-18).
 #include "proxddp.hpp"
 #include "qp.hpp"
+#include "riccati_par.hpp"
 #include <cstdio>
 #include <omp.h>
 
@@ -171,10 +172,10 @@ void orc_eval_knot(const mpc_robot_t *rb, const mpc_config_t *cfg, const mpc_kno
 
 // ---- proximal Riccati on dense caller data (all knots share sizes). Layouts as mpc_riccati_dense (mpcb200.h).
 // H [T][nz][nz], g [T][nz], AB [T][n][nz], f [T][n], CD [T][nc][nz], d [T][nc], HT [n][n], gT [n]
-// E6 [T][36] or NULL; CT [nct][n], dT [nct] or NULL
-void orc_riccati(int n, int m, int nc, int T, double mu_d, double mu, const double *H, const double *g, const double *AB, const double *f,
-                 const double *CD, const double *dd, const double *E6, const double *HT, const double *gT, const double *CT, const double *dT,
-                 int nct, double *dxs, double *dus, double *dvs, double *dlams, double *K) {
+// E6 [T][36] or NULL; CT [nct][n], dT [nct] or NULL.  legs >= 2: the leg-parallel solve (riccati_par.hpp), else the serial one
+static void riccati_dense(int n, int m, int nc, int T, double mu_d, double mu, const double *H, const double *g, const double *AB, const double *f,
+                          const double *CD, const double *dd, const double *E6, const double *HT, const double *gT, const double *CT, const double *dT,
+                          int nct, int legs, double *dxs, double *dus, double *dvs, double *dlams, double *K) {
   int nz = n + m;
   std::vector<std::vector<double>> A(T), B(T), C(T), D(T);
   std::vector<LQKnot> kn(T);
@@ -186,11 +187,22 @@ void orc_riccati(int n, int m, int nc, int T, double mu_d, double mu, const doub
              C[k].data(), D[k].data(), dd + (size_t)k * nc};
   }
   LQSolution sol;
-  riccati_solve(n, m, nc, T, kn.data(), HT, n, gT, CT, dT, nct, mu_d, mu, sol);
+  if (legs >= 2) riccati_solve_par(n, m, nc, T, kn.data(), HT, n, gT, CT, dT, nct, mu_d, mu, legs, sol);
+  else riccati_solve(n, m, nc, T, kn.data(), HT, n, gT, CT, dT, nct, mu_d, mu, sol);
   std::copy(sol.dxs.begin(), sol.dxs.end(), dxs); std::copy(sol.dus.begin(), sol.dus.end(), dus);
   if (dvs) std::copy(sol.dvs.begin(), sol.dvs.end(), dvs);
   if (dlams) std::copy(sol.dlams.begin(), sol.dlams.end(), dlams);
   if (K) std::copy(sol.K.begin(), sol.K.end(), K);
+}
+void orc_riccati(int n, int m, int nc, int T, double mu_d, double mu, const double *H, const double *g, const double *AB, const double *f,
+                 const double *CD, const double *dd, const double *E6, const double *HT, const double *gT, const double *CT, const double *dT,
+                 int nct, double *dxs, double *dus, double *dvs, double *dlams, double *K) {
+  riccati_dense(n, m, nc, T, mu_d, mu, H, g, AB, f, CD, dd, E6, HT, gT, CT, dT, nct, 0, dxs, dus, dvs, dlams, K);
+}
+void orc_riccati_par(int n, int m, int nc, int T, double mu_d, double mu, const double *H, const double *g, const double *AB, const double *f,
+                     const double *CD, const double *dd, const double *E6, const double *HT, const double *gT, const double *CT, const double *dT,
+                     int nct, int legs, double *dxs, double *dus, double *dvs, double *dlams, double *K) {
+  riccati_dense(n, m, nc, T, mu_d, mu, H, g, AB, f, CD, dd, E6, HT, gT, CT, dT, nct, legs, dxs, dus, dvs, dlams, K);
 }
 
 // ---- ProxDDP: batch of instances, OpenMP over instances (knot_threads > 1: over knots, batch serial)
@@ -304,5 +316,38 @@ void orc_qp_assemble_id(int batch, const double *M, const double *nle, const dou
   for (int i = 0; i < batch; i++)
     qp_assemble_id(M + i * 784, nle + i * 28, Jc + i * 336, gamma + i * 12, a + i * 28, forces + i * 12, cs + i * 2, mu, L, W, A + i * 2480, b + i * 40,
                    C + i * 1116, l + i * 18);
+}
+
+// ---- IKID task terms (IKIDSolver_f6) on the oracle's own rigid-body code (rbd.hpp), not on the kernels' composite formulation.
+// Ag [6][NV] (centroidal_derivatives), dAgv [6] (centroidal_rate at qdd = 0, gravity excluded), the angular rows of the LOCAL Jacobians
+// of two frames Jang [2][3][NV] and their dJ v [2][3] column by column from forward_kin, plus the frame placements oMf [2][12].
+// Any output may be NULL.
+void orc_ikid_terms(const mpc_robot_t *rb, const double *x, const int *frame_body, const double *frame_place, double *Ag, double *dAgv,
+                    double *Jang, double *dJang, double *oMf) {
+  Tree tr(rb);
+  static Kin<double> k;
+  forward_kin<double>(tr, x, x + NQ, k);
+  double dhq[6 * NV], ag[6 * NV];
+  centroidal_derivatives(tr, k, dhq, ag);
+  if (Ag) for (int i = 0; i < 6 * NV; i++) Ag[i] = ag[i];
+  // centroidal_rate folds gravity in as a_world = -g: remove its wrench at the CoM, [m (-g); 0]
+  V6<double> F = centroidal_rate<double>(tr, k, x + NQ, nullptr);
+  if (dAgv) for (int i = 0; i < 6; i++) dAgv[i] = F[i] + (i < 3 ? k.mass * rb->gravity[i] : 0.0);
+  V6<double> a[NB];
+  body_accels<double>(tr, k, x + NQ, nullptr, false, a);
+  for (int f = 0; f < 2; f++) {
+    const int b = frame_body[f];
+    SE3<double> Mf = mul(k.oM[b], se3_cast<double>(frame_place + 12 * f));
+    for (int j = 0; j < NV; j++) {
+      V6<double> col = tr.anc[body_of_dof(j)][b] ? actinv_motion(Mf, k.S[j]) : zero6<double>();
+      if (Jang) for (int r = 0; r < 3; r++) Jang[(3 * f + r) * NV + j] = col[3 + r];
+    }
+    V6<double> acc = actinv_motion(Mf, a[b]);
+    if (dJang) for (int r = 0; r < 3; r++) dJang[3 * f + r] = acc[3 + r];
+    if (oMf) {
+      for (int i = 0; i < 9; i++) oMf[12 * f + i] = Mf.R[i];
+      for (int i = 0; i < 3; i++) oMf[12 * f + 9 + i] = Mf.p[i];
+    }
+  }
 }
 }

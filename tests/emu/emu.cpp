@@ -16,6 +16,7 @@ using namespace mpcdev;
 
 struct EmuBackend {
   Ws w;
+  LegWs lw{}; // allocated for cfg.lq_legs >= 2: the time-parallel LQ solve (riccati_par.cuh)
   std::vector<double> smem;
   EmuBackend() : smem(40000, 0.0) {}
   void reset_counters() { for (int i = 0; i < 4; i++) w.counters[i] = 0; }
@@ -30,7 +31,16 @@ struct EmuBackend {
   }
   void decide_eval(const int32_t *list, int n, int32_t *next_eval) { double red[8]; for (int i = 0; i < n; i++) mpcdev::decide_eval(w, list[i], red, next_eval); }
   void riccati(const int32_t *list, int n) {
-    dispatch_kind(w.kind, [&](auto kind) { for (int i = 0; i < n; i++) riccati_dispatch<decltype(kind)::value>(w, list[i], smem.data()); });
+    dispatch_kind(w.kind, [&](auto kind) {
+      constexpr int KIND = decltype(kind)::value;
+      if (lw.L < 2) { for (int i = 0; i < n; i++) riccati_dispatch<KIND>(w, list[i], smem.data()); return; }
+      // the four phases as the CUDA backend launches them: A and C over every (instance, leg), B and D over every instance
+      double sh[64];
+      for (int e = 0; e < n * lw.L; e++) ric_par_legs<KIND>(w, lw, list[e / lw.L], e % lw.L);
+      for (int i = 0; i < n; i++) ric_par_consensus<KIND>(w, lw, list[i], sh);
+      for (int e = 0; e < n * lw.L; e++) ric_par_resolve<KIND>(w, lw, list[e / lw.L], e % lw.L, smem.data());
+      for (int i = 0; i < n; i++) ric_par_finish<KIND>(w, lw, list[i]);
+    });
   }
   void apply_step(const int32_t *list, int n) { w.counters[0] = 0; for (int i = 0; i < n; i++) mpcdev::apply_step(w, list[i]); }
   void decide_ls(const int32_t *list, int n, int32_t *ls_out, int32_t *next_eval) {
@@ -55,7 +65,9 @@ extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, int bat
   Ws &w = be.w;
   init_ws(w, *cfg, batch, model);
   std::vector<void *> allocs;
-  alloc_ws(w, [&](size_t bytes) { void *p = calloc(bytes ? bytes : 8, 1); allocs.push_back(p); return p; });
+  auto calloc_ = [&](size_t bytes) { void *p = calloc(bytes ? bytes : 8, 1); allocs.push_back(p); return p; };
+  alloc_ws(w, calloc_);
+  if (cfg->lq_legs >= 2) alloc_leg_ws(w, be.lw, cfg->lq_legs, calloc_);
   const size_t T1 = w.T + 1;
   std::memcpy(w.knots, knots, sizeof(mpc_knot_t) * batch * w.T);
   std::memcpy(w.terms, terms, sizeof(mpc_term_t) * batch);
@@ -117,6 +129,31 @@ extern "C" int emu_rbd_terms(const mpc_robot_t *rb, const mpc_config_t *cfg, int
     rbd_terms_group(*model, x + (size_t)i * 57, w, M + (size_t)i * 784, nle + (size_t)i * 28, Jc + (size_t)i * 336, dJv + (size_t)i * 12, vf + (size_t)i * 12);
   delete model;
   return 0;
+}
+
+// ---- IKID task terms (k_ikid_terms) of `count` states, serial
+extern "C" int emu_ikid_terms(const mpc_robot_t *rb, const mpc_config_t *cfg, int count, const double *x, const int32_t *frame_body, const double *frame_place,
+                              double *M, double *nle, double *Jc, double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
+  DevModel *model = new DevModel;
+  const char *err = nullptr;
+  if (build_dev_model(rb, cfg, model, &err)) { delete model; return 1; }
+  std::vector<double> smem(sizeof(FullWsT<false>) / 8 + 8, 0.0);
+  FullWsT<false> &w = *reinterpret_cast<FullWsT<false> *>(smem.data());
+  for (int i = 0; i < count; i++)
+    ikid_terms_group(*model, x + (size_t)i * 57, frame_body, frame_place, w, M + (size_t)i * 784, nle + (size_t)i * 28, Jc + (size_t)i * 336, dJv + (size_t)i * 12,
+                     Ag + (size_t)i * 168, dAgv + (size_t)i * 6, Jang + (size_t)i * 168, dJang + (size_t)i * 6);
+  delete model;
+  return 0;
+}
+// k_qp_assemble_ikid, serial
+extern "C" void emu_qp_assemble_ikid(int batch, const double *M, const double *nle, const double *Jc, const double *dJv, const double *Ag, const double *dAgv,
+                                     const double *Jang, const double *dJang, const double *task, const double *forces, const int32_t *cs, const double *weights,
+                                     const double *gains, double mu, double L, double W, double *H, double *g, double *A, double *b, double *C, double *l) {
+  double sm[24 * 28 + 24 + 12 + 28];
+  for (int i = 0; i < batch; i++)
+    qp_assemble_ikid_group(M + i * 784, nle + i * 28, Jc + i * 336, dJv + i * 12, Ag + i * 168, dAgv + i * 6, Jang + i * 168, dJang + i * 6, task + i * 98,
+                           forces + i * 12, cs + i * 2, weights, gains, mu, L, W, sm, H + (size_t)i * 3844, g + i * 62, A + (size_t)i * 2480, b + i * 40,
+                           C + (size_t)i * 1116, l + i * 18);
 }
 
 // ---- device gait generator (gait.cuh) run serially: `ticks` ticks of `batch` robots; lf / rf [ticks][batch][12] measured sole placements;

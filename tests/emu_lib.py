@@ -86,6 +86,32 @@ def rbd_terms(rb, cfg, x):
     return o
 
 
+def ikid_terms(rb, cfg, x, frame_body, frame_place):
+    """ikid_terms_group (csrc/rbd_terms.cuh) run serially: dict(M, nle, Jc, dJv, Ag, dAgv, Jang [count][2][3][28], dJang [count][2][3])
+    for the states x [count][57] and the frames (frame_body[f], frame_place[f])."""
+    x = np.ascontiguousarray(x, float).reshape(-1, 57)
+    B = x.shape[0]
+    o = dict(M=np.zeros((B, 28, 28)), nle=np.zeros((B, 28)), Jc=np.zeros((B, 12, 28)), dJv=np.zeros((B, 12)), Ag=np.zeros((B, 6, 28)), dAgv=np.zeros((B, 6)),
+             Jang=np.zeros((B, 2, 3, 28)), dJang=np.zeros((B, 2, 3)))
+    fb, fp = np.ascontiguousarray(frame_body, np.int32), np.ascontiguousarray(frame_place, float).reshape(24)
+    rc = lib().emu_ikid_terms(C.byref(rb), C.byref(cfg), B, _p(x), fb.ctypes.data_as(C.POINTER(C.c_int32)), _p(fp),
+                              *[_p(o[k]) for k in ("M", "nle", "Jc", "dJv", "Ag", "dAgv", "Jang", "dJang")])
+    assert rc == 0
+    return o
+
+
+def qp_assemble_ikid(M, nle, Jc, dJv, Ag, dAgv, Jang, dJang, task, forces, cs, weights, gains, mu, L, W):
+    """qp_assemble_ikid_group (csrc/qp.cuh) run serially: (H, g, A, b, C, l) of the IKID QPs; gains packed [1658]."""
+    batch = np.asarray(M).reshape(-1, 28, 28).shape[0]
+    H, g = np.zeros((batch, 62, 62)), np.zeros((batch, 62))
+    A, b, Cm, l = np.zeros((batch, 40, 62)), np.zeros((batch, 40)), np.zeros((batch, 18, 62)), np.zeros((batch, 18))
+    cs = np.ascontiguousarray(cs, np.int32)
+    f = lambda v: _p(np.ascontiguousarray(v, float))  # noqa: E731
+    lib().emu_qp_assemble_ikid(batch, f(M), f(nle), f(Jc), f(dJv), f(Ag), f(dAgv), f(Jang), f(dJang), f(task), f(forces), cs.ctypes.data_as(C.POINTER(C.c_int32)),
+                               f(weights), f(gains), C.c_double(mu), C.c_double(L), C.c_double(W), _p(H), _p(g), _p(A), _p(b), _p(Cm), _p(l))
+    return H, g, A, b, Cm, l
+
+
 def gait(kind, T, g, mirror, urefs, lf, rf):
     """csrc/gait.cuh run serially: lf / rf [ticks][batch][12] -> (knots [ticks][batch * T], terms [ticks][batch])."""
     lf, rf = np.ascontiguousarray(lf, float), np.ascontiguousarray(rf, float)

@@ -162,6 +162,16 @@ def riccati(n, m, nc, T, mu_d, mu, H, g, AB, f, CD, d, E6, HT, gT, CT=None, dT=N
     return o
 
 
+def riccati_par(n, m, nc, T, mu_d, mu, H, g, AB, f, CD, d, E6, HT, gT, CT=None, dT=None, legs=2):
+    """The leg-parallel LQ solve (oracle/riccati_par.hpp) over `legs` legs; the same outputs as riccati."""
+    nct = 0 if CT is None else CT.shape[0]
+    s = m + nc
+    o = dict(dxs=np.zeros((T + 1, n)), dus=np.zeros((T, m)), dvs=np.zeros((T + 1, nc)), dlams=np.zeros((T + 1, n)), K=np.zeros((T, s, 1 + n)))
+    lib().orc_riccati_par(n, m, nc, T, C.c_double(mu_d), C.c_double(mu), _p(H), _p(g), _p(AB), _p(f), _p(CD), _p(d), _p(E6), _p(HT), _p(gT),
+                          _p(CT), _p(dT), nct, int(legs), _p(o["dxs"]), _p(o["dus"]), _p(o["dvs"]), _p(o["dlams"]), _p(o["K"]))
+    return o
+
+
 def solve(prob, max_iters=None, inst_threads=1, knot_threads=1, vs=None, lams=None, xs=None, us=None):
     """Run the oracle ProxDDP on a problem dict from mpc_benchmark_b200.problems."""
     cfg = prob["cfg"]
@@ -179,6 +189,18 @@ def solve(prob, max_iters=None, inst_threads=1, knot_threads=1, vs=None, lams=No
                     _p(xs), _p(us), _p(K), _p(vs), _p(lams), info, _p(stage0), int(cfg.max_iters if max_iters is None else max_iters),
                     int(inst_threads), int(knot_threads))
     return dict(xs=xs, us=us, K=K, vs=vs, lams=lams, info=info, stage0=stage0)
+
+
+def ikid_terms(rb, x, frame_body, frame_place):
+    """IKID task terms for the states x [count][57]: dict(Ag [count][6][28], dAgv [count][6], Jang [count][2][3][28], dJang [count][2][3],
+    oMf [count][2][12]) of the frames (frame_body[f], frame_place[f])."""
+    x = np.ascontiguousarray(x, float).reshape(-1, 57)
+    B = x.shape[0]
+    o = dict(Ag=np.zeros((B, 6, 28)), dAgv=np.zeros((B, 6)), Jang=np.zeros((B, 2, 3, 28)), dJang=np.zeros((B, 2, 3)), oMf=np.zeros((B, 2, 12)))
+    fb, fp = np.ascontiguousarray(frame_body, np.int32), np.ascontiguousarray(frame_place, float).reshape(24)
+    for i in range(B):
+        lib().orc_ikid_terms(C.byref(rb), _p(x[i]), fb.ctypes.data_as(C.POINTER(C.c_int32)), _p(fp), *[_p(o[k][i]) for k in ("Ag", "dAgv", "Jang", "dJang", "oMf")])
+    return o
 
 
 # ---- dense QP oracle (oracle/qp.hpp; SURVEY 8f row f-3)

@@ -2,14 +2,15 @@
 csrc/rbd_terms.cuh (ikid_terms_group: Ag, dAg v, LOCAL angular Jacobians of the base / torso frames and their dJ v), the cost and
 constraint assembly of csrc/qp.cuh (qp_assemble_ikid_group) and `IKIDSolver_f6.solve_from_state`.
 
-CPU (`-m "not gpu"`): the oracle's task terms (tests/ikid/ikid_oracle.cpp, on oracle/rbd.hpp) against central differences, the base-frame known answer, and the kernel sources run
-serially under the host emulation (tests/ikid/ikid_emu.cpp) against the oracle and the literal cost formulas.  GPU (`-m gpu`): the device path against the
+CPU (`-m "not gpu"`): the oracle's task terms (orc_ikid_terms in oracle/capi.cpp, on oracle/rbd.hpp) against central differences, the base-frame known answer, and the kernel sources run
+serially under the host emulation (tests/emu/emu.cpp) against the oracle and the literal cost formulas.  GPU (`-m gpu`): the device path against the
 emulation, the oracle and the host-assembled `solve`."""
 import numpy as np
 import pytest
 from scipy.spatial.transform import Rotation
 
-import ikid_lib
+import emu_lib
+import oracle_lib
 
 from test_qp import FIXTURE, FOOT_L, FOOT_W, MU, _ikid_reference_cost
 
@@ -49,7 +50,7 @@ def _states(n_random=4, seed=3):
 def test_oracle_ikid_terms_match_central_differences(oracle, setup):
     rb, fb, fp = setup["robot"], setup["fb"], setup["fp"]
     for x in _states():
-        o = ikid_lib.oracle_ikid_terms(rb, x, fb, fp)
+        o = oracle_lib.ikid_terms(rb, x, fb, fp)
         Ag, dAgv, Jang, dJang = o["Ag"][0], o["dAgv"][0], o["Jang"][0], o["dJang"][0]
         hg = lambda xx: oracle.kinematics(rb, xx)["hg"]  # noqa: E731
         # Ag = d h_g / d v: h_g is linear in v, so the difference is exact up to rounding
@@ -68,7 +69,7 @@ def test_oracle_ikid_terms_match_central_differences(oracle, setup):
         fd = (hg(along(t)) - hg(along(-t))) / (2 * t)
         assert np.abs(fd - dAgv).max() < 1e-6 * max(1.0, np.abs(dAgv).max())
         # angular Jacobian columns: log3(R(q)' R(q + h e_j)) / h, central
-        R = lambda xx: ikid_lib.oracle_ikid_terms(rb, xx, fb, fp)["oMf"][0, :, :9].reshape(2, 3, 3)  # noqa: E731
+        R = lambda xx: oracle_lib.ikid_terms(rb, xx, fb, fp)["oMf"][0, :, :9].reshape(2, 3, 3)  # noqa: E731
         R0, h = R(x), 1e-6
         for j in range(NV):
             e = np.zeros(2 * NV)
@@ -78,7 +79,7 @@ def test_oracle_ikid_terms_match_central_differences(oracle, setup):
                 col = (Rotation.from_matrix(R0[f].T @ Rp[f]).as_rotvec() - Rotation.from_matrix(R0[f].T @ Rm[f]).as_rotvec()) / (2 * h)
                 assert np.abs(col - Jang[f, :, j]).max() < 1e-7
         # dJ v = d/dt (Jang(q + t v) v)
-        Jv = lambda t: ikid_lib.oracle_ikid_terms(rb, along(t), fb, fp)["Jang"][0] @ v  # noqa: E731
+        Jv = lambda t: oracle_lib.ikid_terms(rb, along(t), fb, fp)["Jang"][0] @ v  # noqa: E731
         fd = (Jv(t) - Jv(-t)) / (2 * t)
         assert np.abs(fd - dJang).max() < 1e-6 * max(1.0, np.abs(dJang).max())
 
@@ -88,8 +89,8 @@ def test_base_frame_known_answer(setup):
     x = _states()
     expect = np.zeros((3, NV))
     expect[:, 3:6] = np.eye(3)
-    for o in (ikid_lib.oracle_ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]),
-              ikid_lib.emu_ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])):
+    for o in (oracle_lib.ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]),
+              emu_lib.ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])):
         Jb = o["Jang"][:, 0]
         assert not Jb[:, :, :3].any() and not Jb[:, :, 6:].any()  # exact zeros off the angular base columns
         assert np.abs(Jb - expect).max() < 1e-15  # R' R e_j: identity to rounding
@@ -103,11 +104,9 @@ def _check_against_oracle(o, ref):
 
 
 def test_emulated_ikid_terms_match_oracle_and_rbd_terms(setup):
-    import emu_lib
-
     x = _states()
-    e = ikid_lib.emu_ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])
-    _check_against_oracle(e, ikid_lib.oracle_ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]))
+    e = emu_lib.ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])
+    _check_against_oracle(e, oracle_lib.ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]))
     r = emu_lib.rbd_terms(setup["robot"], setup["cfg"], x)
     for k in ("M", "nle", "Jc", "dJv"):
         assert np.array_equal(e[k], r[k]), k
@@ -118,7 +117,7 @@ def test_emulated_sole_frame_rows_equal_contact_jacobian(setup):
     rb = setup["robot"]
     x = _states()
     fp = np.array([rb.foot_place[0][:], rb.foot_place[1][:]])
-    e = ikid_lib.emu_ikid_terms(rb, setup["cfg"], x, [rb.foot_body[0], rb.foot_body[1]], fp)
+    e = emu_lib.ikid_terms(rb, setup["cfg"], x, [rb.foot_body[0], rb.foot_body[1]], fp)
     Jc = e["Jc"].reshape(-1, 2, 6, NV)
     assert np.array_equal(e["Jang"], Jc[:, :, 3:])
     assert np.abs(e["dJang"] - e["dJv"].reshape(-1, 2, 6)[:, :, 3:]).max() < 1e-15
@@ -164,14 +163,12 @@ def _with_terms(t, o):
 
 
 def test_emulated_ikid_assembly_matches_reference_formulas(setup):
-    import emu_lib
-
     B = 24
     t = _task_inputs(B)
-    o = ikid_lib.emu_ikid_terms(setup["robot"], setup["cfg"], t["x"], setup["fb"], setup["fp"])
+    o = emu_lib.ikid_terms(setup["robot"], setup["cfg"], t["x"], setup["fb"], setup["fp"])
     t = _with_terms(t, o)
-    H, g, A, b, Cm, l = ikid_lib.emu_qp_assemble_ikid(o["M"], o["nle"], o["Jc"], o["dJv"], o["Ag"], o["dAgv"], o["Jang"], o["dJang"], _task(t, B), t["forces"],
-                                                 t["cs"], t["weights"], _pack(t["K_gains"]), MU, FOOT_L, FOOT_W)
+    H, g, A, b, Cm, l = emu_lib.qp_assemble_ikid(o["M"], o["nle"], o["Jc"], o["dJv"], o["Ag"], o["dAgv"], o["Jang"], o["dJang"], _task(t, B), t["forces"],
+                                             t["cs"], t["weights"], _pack(t["K_gains"]), MU, FOOT_L, FOOT_W)
     for i in range(B):
         Hr, gr = _ikid_reference_cost(t, i)
         assert np.abs(H[i, :28, :28] - Hr).max() <= 1e-12 * np.abs(Hr).max()
@@ -216,8 +213,8 @@ def test_gpu_ikid_terms_match_emulation_and_oracle(setup, device_solver):
     M, rbd = device_solver.ikid_terms(x, list(zip(setup["fb"], setup["fp"])))
     d = dict(M=M, nle=rbd.nle, Jc=rbd.Jc, dJv=rbd.dJv, Ag=rbd.Ag, dAgv=rbd.dAgv, Jang=np.stack([rbd.J_base, rbd.J_torso], 1),
              dJang=np.stack([rbd.dJv_base, rbd.dJv_torso], 1))
-    e = ikid_lib.emu_ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])
-    _check_against_oracle(d, ikid_lib.oracle_ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]))
+    e = emu_lib.ikid_terms(setup["robot"], setup["cfg"], x, setup["fb"], setup["fp"])
+    _check_against_oracle(d, oracle_lib.ikid_terms(setup["robot"], x, setup["fb"], setup["fp"]))
     _check_against_oracle(d, e)
     r = device_solver.rbd_terms(x)
     for k in ("M", "nle", "Jc", "dJv"):

@@ -5,7 +5,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-import lqpar_lib
+import emu_lib
 from mpc_benchmark_b200 import _abi, _native, problems
 from test_lq import dense_kkt_solution, random_lq
 
@@ -32,7 +32,7 @@ def test_oracle_legs_match_serial_and_dense_kkt(oracle, n, m, nc, T, mu, legs):
     a = list(args)
     a[12] = E6
     o = oracle.riccati(*a)
-    p = lqpar_lib.riccati_par(*a, legs=L)
+    p = oracle.riccati_par(*a, legs=L)
     dxs, dus, dvs, dls, dvT = dense_kkt_solution(*a)
     assert not np.allclose(args[12].reshape(-1, 6, 6)[0], -np.eye(6))  # E6 != -I
     sc = max(1.0, np.abs(dxs).max(), np.abs(dus).max())
@@ -60,9 +60,15 @@ def _emu_case(kind, batch):
 @pytest.mark.parametrize("rollout", [0, 1])
 def test_emulated_solver_legs_match_serial(kind, rollout):
     prob = _emu_case(kind, 2)
-    ref = lqpar_lib.emu_solve(prob, 0, max_iters=3, rollout=rollout)
+
+    def solve(legs):
+        cfg = _abi.Config.from_buffer_copy(prob["cfg"])
+        cfg.lq_legs, cfg.rollout = legs, rollout
+        return emu_lib.solve(dict(prob, cfg=cfg), max_iters=3)
+
+    ref = solve(0)
     for L in (2, 4, 8):
-        r = lqpar_lib.emu_solve(prob, L, max_iters=3, rollout=rollout)
+        r = solve(L)
         assert [(i.num_iters, i.status, i.ls_evals) for i in r["info"]] == [(i.num_iters, i.status, i.ls_evals) for i in ref["info"]], L
         for k in ("xs", "us", "vs", "lams"):
             assert rel(r[k], ref[k]) < EMU_TOL, (L, k, rel(r[k], ref[k]))
