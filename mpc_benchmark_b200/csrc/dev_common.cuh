@@ -34,9 +34,6 @@
 #define PREFETCH_L2(ptr, bytes) ((void)0)
 #define PREFETCH_LINES(ptr, bytes) ((void)0)
 #define LDCG(p) (*(p))
-#define LANE_ID 0
-#define LANE_IS(r) true
-#define PRELOADED(v, e) (e)
 #define BULK_G2S(dst, src, bytes, bar) do { for (size_t i_ = 0; i_ < (size_t)(bytes) / 8; i_++) (dst)[i_] = (src)[i_]; } while (0)
 struct double2 { double x, y; };
 inline double2 make_double2(double x, double y) { return double2{x, y}; }
@@ -86,11 +83,6 @@ inline double2 make_double2(double x, double y) { return double2{x, y}; }
 #define LDCG(p) __ldcg(p)
 // the same for blocks without 16-byte alignment: one prefetch.global.L2 per 128-byte line, spread over the threads of the group
 #define PREFETCH_LINES(ptr, bytes) do { const char *p_ = reinterpret_cast<const char *>(ptr); for (int o_ = threadIdx.x * 128; o_ < (int)(bytes); o_ += blockDim.x * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(p_ + o_)); } while (0)
-#define LANE_ID ((int)(threadIdx.x & 31))
-// "lane r finishes row r" after a butterfly reduction: values the finishing lane needs are loaded before the reduction
-// (PRELOADED: the early copy on the device; the host emulation has one "lane" that finishes every row and loads on the spot)
-#define LANE_IS(r) ((int)(threadIdx.x & 31) == (r))
-#define PRELOADED(v, e) (v)
 #endif
 
 namespace mpcdev {
@@ -106,7 +98,8 @@ __device__ __forceinline__ double warp_sum(double v) {
 
 // Reciprocal / square root without the library routines' special-case code (hardware seed + two Newton steps, <= 2 ulp).  The
 // library versions cost a single-lane dependency chain 80-130 cycles and dozens of (partly predicated) instructions per call; the
-// serial sections of the kernels (pivot chains, Lie-group routines) are made of exactly such calls (tools/ubench/lat.cu, diag.cu).
+// serial sections of the kernels (pivot chains, Lie-group routines) are made of exactly such calls (tools/ubench/lat.cu, diag.cu):
+// in a pivot chain rcp_ costs 56 cycles of dependent latency against 83 for a division.
 // Arguments are positive and in the normal range at every call site; NaN / non-positive inputs still propagate as NaN.
 #ifdef MPC_HOST_EMU
 inline double rcp_(double a) { return 1.0 / a; }
@@ -426,66 +419,6 @@ HD void compact_flags(const int32_t *flags, int n, int32_t *idx, int32_t *count,
 // In-place lower Cholesky of A (n x n, ld) by 8-wide panels.  Dinv receives the inverses of the diagonal blocks (8 x 8
 // lower, row-major, 64 doubles per panel), which turn the triangular solves below into small GEMMs.
 constexpr int CB = 8;
-#ifdef MPC_HOST_EMU
-inline double rsqrt(double x) { return 1.0 / sqrt(x); }
-#endif
-// 1/sqrt(a) without the slow-path handling of the library routine: fp32 seed + two Newton steps in fp64 (<= 2 ulp).
-HD double fast_rsqrt(double a) {
-#ifdef MPC_HOST_EMU
-  return 1.0 / sqrt(a);
-#else
-  if (a > 1e-30 && a < 1e30) {
-    double y = (double)rsqrtf((float)a); // ~22 bits; two Newton steps -> full fp64
-    double t = a * y, e = fma(-t, y, 1.0);
-    y = fma(0.5 * y, e, y);
-    t = a * y; e = fma(-t, y, 1.0);
-    return fma(0.5 * y, e, y);
-  }
-  return rsqrt(a);
-#endif
-}
-// ONE thread factors the bw x bw diagonal block at k0 and inverts it entirely in registers (fully unrolled, no barriers,
-// no shared-memory round trips on the dependency chain; rows/cols >= bw are padded with the identity).
-HD void chol_diag_block(double *A, int k0, int bw, int ld, double *Di) {
-  double L[CB][CB], X[CB][CB], dd[CB];
-#pragma unroll
-  for (int r = 0; r < CB; r++)
-#pragma unroll
-    for (int c = 0; c < CB; c++) L[r][c] = (c <= r) ? ((r < bw) ? A[(k0 + r) * ld + k0 + c] : ((r == c) ? 1.0 : 0.0)) : 0.0;
-#pragma unroll
-  for (int j = 0; j < CB; j++) {
-    const double d = fast_rsqrt(L[j][j]);
-    dd[j] = d;
-    L[j][j] = L[j][j] * d;
-#pragma unroll
-    for (int r = j + 1; r < CB; r++) L[r][j] *= d;
-#pragma unroll
-    for (int r = j + 1; r < CB; r++)
-#pragma unroll
-      for (int c = j + 1; c <= r; c++) L[r][c] -= L[r][j] * L[c][j];
-  }
-  // X = L^-1 column by column in right-looking order: as soon as X[t][c] is known it is folded into the partial sums of the
-  // rows below, so the dependent chain per row is one multiply + one FMA (the 8 columns are independent chains)
-#pragma unroll
-  for (int c = 0; c < CB; c++) {
-#pragma unroll
-    for (int r = 0; r < CB; r++) X[r][c] = (r == c) ? 1.0 : 0.0;
-#pragma unroll
-    for (int t = c; t < CB; t++) {
-      X[t][c] *= dd[t];
-#pragma unroll
-      for (int r = t + 1; r < CB; r++) X[r][c] -= L[r][t] * X[t][c];
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < CB; r++)
-#pragma unroll
-    for (int c = 0; c < CB; c++) {
-      if (r < bw && c <= r) A[(k0 + r) * ld + k0 + c] = L[r][c];
-      Di[r * CB + c] = (r < bw && c < bw) ? X[r][c] : 0.0;
-    }
-}
-HD double fast_rcp(double a) { return rcp_(a); } // pivot chains: 56 cycles of dependent latency against 83 for a division (tools/ubench/lat.cu)
 #ifndef MPC_HOST_EMU
 // Device version called by ALL lanes of the group's warp 0.  Lane 0 runs the pivot chain in registers as a square-root-free
 // LDL' elimination (per column: reciprocal of the pivot -> scaled column -> update, 56 + 8.5 + 8.5 cycles of dependent
@@ -502,7 +435,7 @@ __device__ __forceinline__ void chol_diag_block_warp0(double *A, int k0, int bw,
       for (int c = 0; c < CB; c++) L[r][c] = (c <= r) ? ((r < bw) ? A[(k0 + r) * ld + k0 + c] : ((r == c) ? 1.0 : 0.0)) : 0.0;
 #pragma unroll
     for (int j = 0; j < CB; j++) {
-      const double rj = fast_rcp(L[j][j]);
+      const double rj = rcp_(L[j][j]);
       Di[j * CB + j] = L[j][j]; // pivot d_j (scratch for the finish below)
       double tcol[CB];
 #pragma unroll
@@ -549,6 +482,47 @@ __device__ __forceinline__ void chol_diag_block_warp0(double *A, int k0, int bw,
 }
 #define DIAG_BLOCK(A, k0, bw, ld, Di) do { if (threadIdx.x < 32) mpcdev::chol_diag_block_warp0(A, k0, bw, ld, Di); } while (0)
 #else
+// Host-emulation version: the bw x bw diagonal block at k0 is factored (Cholesky) and inverted in place of the device's pivot
+// chain (rows/cols >= bw are padded with the identity).
+inline void chol_diag_block(double *A, int k0, int bw, int ld, double *Di) {
+  double L[CB][CB], X[CB][CB], dd[CB];
+#pragma unroll
+  for (int r = 0; r < CB; r++)
+#pragma unroll
+    for (int c = 0; c < CB; c++) L[r][c] = (c <= r) ? ((r < bw) ? A[(k0 + r) * ld + k0 + c] : ((r == c) ? 1.0 : 0.0)) : 0.0;
+#pragma unroll
+  for (int j = 0; j < CB; j++) {
+    const double d = rsqrt_(L[j][j]);
+    dd[j] = d;
+    L[j][j] = L[j][j] * d;
+#pragma unroll
+    for (int r = j + 1; r < CB; r++) L[r][j] *= d;
+#pragma unroll
+    for (int r = j + 1; r < CB; r++)
+#pragma unroll
+      for (int c = j + 1; c <= r; c++) L[r][c] -= L[r][j] * L[c][j];
+  }
+  // X = L^-1 column by column in right-looking order: as soon as X[t][c] is known it is folded into the partial sums of the
+  // rows below, so the dependent chain per row is one multiply + one FMA (the 8 columns are independent chains)
+#pragma unroll
+  for (int c = 0; c < CB; c++) {
+#pragma unroll
+    for (int r = 0; r < CB; r++) X[r][c] = (r == c) ? 1.0 : 0.0;
+#pragma unroll
+    for (int t = c; t < CB; t++) {
+      X[t][c] *= dd[t];
+#pragma unroll
+      for (int r = t + 1; r < CB; r++) X[r][c] -= L[r][t] * X[t][c];
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < CB; r++)
+#pragma unroll
+    for (int c = 0; c < CB; c++) {
+      if (r < bw && c <= r) A[(k0 + r) * ld + k0 + c] = L[r][c];
+      Di[r * CB + c] = (r < bw && c < bw) ? X[r][c] : 0.0;
+    }
+}
 #define DIAG_BLOCK(A, k0, bw, ld, Di) chol_diag_block(A, k0, bw, ld, Di)
 #endif
 
@@ -566,7 +540,7 @@ template <int n> HD void small_spd_solve(double *A, int ld, double *B1, int n1, 
       for (int c = 0; c <= r; c++) L[r][c] = A[r * ld + c];
 #pragma unroll
     for (int j = 0; j < n; j++) {
-      const double rj = fast_rcp(L[j][j]);
+      const double rj = rcp_(L[j][j]);
       A[j * ld + j] = rj;
       double tcol[n];
 #pragma unroll

@@ -164,14 +164,14 @@ template <int N, int M, int NC> constexpr int riccati_smem_doubles() {
   constexpr int NZ = N + M, NR = 1 + N;
   constexpr int phase1 = 2 * N * N + 2 * N * NZ;
   constexpr int phase2 = NC * NZ + NC * NC + M * (NR + NC) + NC * NR + M * M;
-  return NZ * NZ + (phase1 > phase2 ? phase1 : phase2) + 8 * NZ + 36 + 2 * NC + 512 + 64 * ((NC + 7) / 8 + (N + 7) / 8) + 16;
+  return NZ * NZ + (phase1 > phase2 ? phase1 : phase2) + 8 * NZ + 2 * NC + 512 + 64 * ((NC + 7) / 8 + (N + 7) / 8) + 16;
 }
 
-// Backward + forward sweep for one instance.  ws: riccati_smem_doubles<N,M,NC>() doubles of shared memory.
-// LIE6: the first 6 state coordinates live on SE(3) (E-normalisation by T6); false for vector-space models (centroidal: T6 = I)
+// Backward + forward sweep for one instance of a model whose state is a vector space (centroidal: T6 = I, so the E normalisation
+// drops out; the SE(3)-based models use riccati_instance_fast).  ws: riccati_smem_doubles<N,M,NC>() doubles of shared memory.
 // SEEDED: solve the knots [io.k0, io.k1) only (see RiccatiIO).  dxs / dlams of knot k0 are written by leg 0 only, the terminal knot's
 // rows by the last leg only; dphi receives the leg's partial.
-template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void riccati_instance(const RiccatiIO &io, double *ws) {
+template <int N, int M, int NC, bool SEEDED = false> HD void riccati_instance(const RiccatiIO &io, double *ws) {
   constexpr int NZ = N + M, NR = 1 + N, S = M + NC;
   const int T = io.T;
   const int K0 = SEEDED ? io.k0 : 0, K1 = SEEDED ? io.k1 : T;
@@ -186,7 +186,7 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
   constexpr int phase2 = NC * NZ + NC * NC + M * (NR + NC) + NC * NR + M * M;
   double *vec = U0 + (phase1 > phase2 ? phase1 : phase2);
   double *p = vec, *pt = p + NZ, *gh = pt + NZ, *fb = gh + NZ, *tmp = fb + NZ, *dx = tmp + NZ, *z = dx + NZ, *dl = z + NZ;
-  double *T6 = dl + NZ, *dbr = T6 + 36, *dva = dbr + NC, *red = dva + NC, *dinv = red + 512;
+  double *dbr = dl + NZ, *dva = dbr + NC, *red = dva + NC, *dinv = red + 512;
   ric_start_value<N, M, NC>(io, seeded, H, NZ, p);
   for (int k = K1 - 1; k >= K0; k--) {
     const double *gAB = io.AB + (size_t)k * N * NZ, *gH = io.H + (size_t)k * NZ * NZ;
@@ -195,24 +195,11 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
       PREFETCH_LINES(io.AB + (size_t)(k - 2) * N * NZ, N * NZ * 8); PREFETCH_LINES(io.H + (size_t)(k - 2) * NZ * NZ, NZ * NZ * 8);
       PREFETCH_LINES(io.g + (size_t)(k - 2) * NZ, NZ * 8); PREFETCH_LINES(io.fbar + (size_t)(k - 2) * N, N * 8);
     }
-    // 1. load; P <- T' P T, p <- T' p
+    // 1. load
     PAR_FOR(e, N * N) { int i = e / N, j = e % N; P[e] = H[i * NZ + j]; }
-    if (LIE6) PAR_FOR(e, 36) T6[e] = io.T6[(size_t)k * 36 + e];
     PAR_FOR(i, N) fb[i] = io.fbar[(size_t)k * N + i];
     PAR_FOR(e, N * NZ) AB[e] = gAB[e];
     SYNC();
-    if (LIE6 && N >= 6) {
-      PAR_FOR(e, N * 6) { int i = e / 6, j = e % 6; double s = 0; for (int l = 0; l < 6; l++) s += P[i * N + l] * T6[6 * l + j]; W[e] = s; }
-      SYNC();
-      PAR_FOR(e, N * 6) { int i = e / 6, j = e % 6; P[i * N + j] = W[e]; }
-      SYNC();
-      PAR_FOR(e, 6 * N) { int i = e / N, j = e % N; double s = 0; for (int l = 0; l < 6; l++) s += T6[6 * l + i] * P[l * N + j]; W[e] = s; }
-      PAR_FOR(i, 6) { double s = 0; for (int l = 0; l < 6; l++) s += T6[6 * l + i] * p[l]; tmp[i] = s; }
-      SYNC();
-      PAR_FOR(e, 6 * N) P[e] = W[e];
-      PAR_FOR(i, 6) p[i] = tmp[i];
-      SYNC();
-    }
     // 2. G = chol(I + mu_d P);  pt = G^-T G^-1 (p + P f);  P <- Pt = G^-T G^-1 P
     PAR_FOR(e, N * N) G[e] = mu_d * P[e] + ((e / N == e % N) ? 1.0 : 0.0);
     PAR_FOR(i, N) { double s = p[i]; for (int j = 0; j < N; j++) s += P[i * N + j] * fb[j]; pt[i] = s; }
@@ -290,7 +277,6 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
       }
       PAR_FOR(i, N) z[i] = dx[i];
       PAR_FOR(e, N * NZ) { AB[e] = io.AB[(size_t)k * N * NZ + e]; W[e] = io.W[(size_t)k * N * NZ + e]; }
-      if (LIE6) PAR_FOR(e, 36) T6[e] = io.T6[(size_t)k * 36 + e];
     } else {
       const double *CT = io.CDact + (size_t)T * NC * NZ;
       PAR_FOR(r, nca) { double s = gdb[ai[r]]; for (int j = 0; j < N; j++) s += CT[r * NZ + j] * dx[j]; dva[r] = s / mu; }
@@ -317,11 +303,7 @@ template <int N, int M, int NC, bool LIE6 = true, bool SEEDED = false> HD void r
       acc += (2.0 * lp - lm) * (mu_d * s - fbi) - fbi * s;
     }
     SYNC();
-    PAR_FOR(i, N) {
-      double s;
-      if (LIE6 && N >= 6 && i < 6) { s = 0; for (int l = 0; l < 6; l++) s += T6[6 * i + l] * tmp[l]; } else s = tmp[i];
-      dx[i] = s; io.dxs[(size_t)(k + 1) * N + i] = s;
-    }
+    PAR_FOR(i, N) { const double s = tmp[i]; dx[i] = s; io.dxs[(size_t)(k + 1) * N + i] = s; }
     SYNC();
   }
   red[TID] = acc;

@@ -1,15 +1,13 @@
 // Proximal Riccati, tensor-core variant for state dimensions that are multiples of 8 (full / kinodynamic: n = 56).
-// Same recursion and outputs as riccati_instance (riccati.cuh, SURVEY App. A6); what changes is HOW the three dense
-// contractions per knot are executed:
-//   Lambda^-1 = Linv' Linv,   Pt = Lambda^-1 P,   W = Pt [A B],   H = H_k + [A B]' W
-// all run on the FP64 DMMA pipe out of shared memory (dmma.cuh), and the triangular solve with Lambda is replaced by an
-// explicit inverse of its Cholesky factor built by independent per-warp column chains (no block barriers).
-// Leading dimensions are padded to 8 (mod 16) doubles so the DMMA fragment loads are bank-conflict free.
-// Around them: both Cholesky factorisations (Lambda, padded control block) are tensor-core blocked with a one-panel
-// look-ahead (chol_mma) and followed by in-place blocked substitutions (trsm_mma), the value update is a DMMA product.
-// Shared memory holds only what is reused many times per knot (H, P, the factor): [A B] and W are used twice each and are
-// streamed as DMMA operands straight from L2 (bulk-prefetched one knot ahead), which is what lets TWO instances share an SM
-// (full dynamics: 107 KB per CTA) so that one instance's serial pivot chains hide behind the other's products.
+// Same recursion and outputs as riccati_instance (riccati.cuh, SURVEY App. A6), plus the E normalisation by T6; what changes is
+// HOW the dense work per knot is executed, all of it on the FP64 DMMA pipe out of shared memory (dmma.cuh):
+//   Lambda = I + mu_d P = G G' (chol_mma),  [Pt | pt] = Lambda^-1 [P | pv] (trsm_mma, in place),  W = Pt [A B] (mma_tn_g),
+//   H = H_k + [A B]' W (mma_sym_deferred),  and the value update P = H_xx + H_xu Ku (mma_tn)
+// The padded control block of the KKT is factored and solved the same way (chol_mma, trsm_mma).  Leading dimensions are padded
+// so that the DMMA fragment loads are bank-conflict free (RicFastLayout).
+// Shared memory holds H, P and the factor; [A B]_k is bulk-copied into the H buffer while it is idle and W is staged behind it, so
+// that both products read shared memory at a footprint (full dynamics: 114 KB per CTA) that lets TWO instances share an SM: one
+// instance's serial pivot chains hide behind the other's products.
 #pragma once
 #include "dmma.cuh"
 #include "riccati.cuh"
@@ -157,7 +155,7 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     // 4. W = Pt [A B] into shared memory (for the Hessian update) and straight from the accumulators to HBM (for the forward
     //    sweep); pt rides in the first padding column of W, so [A B]' pt falls out of the Hessian update
     MBAR_WAIT(mbar + 3, (K1 - 1 - k) & 1); // [A B]_k
-    mma_tn_g<N, false, false>(NBLK, ZP / 8, P, LDN, N, ABs, LDZ, ZP, Ws, LDZ, nullptr, 0, 0, 0, false, gW, LDW, ZP);
+    mma_tn_g<N>(NBLK, ZP / 8, P, LDN, ABs, LDZ, Ws, LDZ, nullptr, 0, 0, 0, false, gW, LDW, ZP);
     PHASE(17);
     PAR_FOR(i, N) { const double v = PV[8 * i]; pt[i] = v; Ws[i * LDZ + NZ] = v; gW[i * LDW + NZ] = v; io.pt[(size_t)k * N + i] = v; }
     SYNC();
@@ -165,7 +163,7 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     //    result overwrites the buffers [A B] and W sit in: accumulators stay in registers until every warp is done reading them.
     //    gh = g + [A B]' pt
     PHASE(22);
-    mma_sym_deferred<N, Lay::MAXQ, false>(ZP / 8, ABs, LDZ, Ws, LDZ, H, LDH, gH, NZ, NZ, NZ);
+    mma_sym_deferred<N, Lay::MAXQ>(ZP / 8, ABs, LDZ, Ws, LDZ, H, LDH, gH, NZ, NZ, NZ);
     PHASE(18);
     PAR_FOR(i, NZ) gh[i] = io.g[(size_t)k * NZ + i] + H[i * LDH + NZ];
     SYNC();

@@ -297,8 +297,8 @@ template <> struct KindTraits<MPC_KIND_CENT> {
   template <bool D> using EvalWs = CentWs;
   template <bool D, bool ROLL = false> static HD void knot(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_knot<D, ROLL>(md, io, f); }
   template <bool D> static HD void term(const DevModel &md, const KnotIO &io, CentWs &f) { eval_cent_term<D>(md, io, f); }
-  static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, false>(r, smem); }
-  static HD void riccati_seeded(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, false, true>(r, smem); }
+  static HD void riccati(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc>(r, smem); }
+  static HD void riccati_seeded(const RiccatiIO &r, double *smem) { riccati_instance<n, m, nc, true>(r, smem); }
   static constexpr bool lie6 = false;
   static constexpr int ric_smem = riccati_smem_doubles<n, m, nc>() * 8, ric_scratch = 2; // no global scratch: a token block
   static constexpr int ric_threads(int, int) { return 128; }

@@ -23,7 +23,7 @@ __global__ void k(long long *cyc, double *out, int reps) {
         for (int c = 0; c < 8; c++) L[i][c] = (c <= i) ? fabs(M[i * 8 + c]) + (i == c ? 10.0 : 0.0) : 0.0;
 #pragma unroll
       for (int j = 0; j < 8; j++) {
-        const double rj = fast_rcp(L[j][j]);
+        const double rj = rcp_(L[j][j]);
         double tc[8];
 #pragma unroll
         for (int i = j + 1; i < 8; i++) tc[i] = L[i][j] * rj;

@@ -20,9 +20,9 @@ __global__ void __launch_bounds__(256) k(double *gW, const double *gH, long long
   t[1] = clock64();
   for (int r = 0; r < reps; r++) trsm_mma<7>(G, LDN, dinv, P, LDN, 7, PV, 8, 8);
   t[2] = clock64();
-  for (int r = 0; r < reps; r++) mma_tn_g<N, false, false>(7, 10, P, LDN, N, ABs, LDZ, ZP, Ws, LDZ, nullptr, 0, 0, 0, false, gW, ZP, ZP);
+  for (int r = 0; r < reps; r++) mma_tn_g<N>(7, 10, P, LDN, ABs, LDZ, Ws, LDZ, nullptr, 0, 0, 0, false, gW, ZP, ZP);
   t[3] = clock64();
-  for (int r = 0; r < reps; r++) mma_sym_deferred<N, 4, false>(10, ABs, LDZ, Ws, LDZ, H, LDH, gH, NZ, NZ, NZ);
+  for (int r = 0; r < reps; r++) mma_sym_deferred<N, 4>(10, ABs, LDZ, Ws, LDZ, H, LDH, gH, NZ, NZ, NZ);
   t[4] = clock64();
   for (int r = 0; r < reps; r++) mma_tn(7, 7, 24, H + N * LDH, LDH, P, LDN, H, LDH, H, LDH, N, N, true);
   t[5] = clock64();
