@@ -130,6 +130,17 @@ int32_t mpc_cycle(mpc_solver_t *h, const mpc_knot_t *last);
 int32_t mpc_shift_multipliers(mpc_solver_t *h, int32_t n);
 /* New robot / weight constants for the same kind, horizon and batch (the shim re-derives them from the object graph at every run). */
 int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_config_t *cfg);
+/* Per-instance robot parameters and cost constants: instance i is solved with robots[i] and cfgs[i] ([batch] host arrays; NULL = the
+ * handle's shared robot / config for every instance; both NULL = back to the shared model).  The models persist across mpc_setup,
+ * mpc_run*, mpc_tick, mpc_cycle and the gait calls until cleared; mpc_reconfigure fails while they are set.  Uniform over the batch,
+ * and checked against the handle's values (the error names the instance and the field): cfg kind, T, dt, tol, mu_init, max_iters,
+ * force_initial_condition, rollout, lq_legs; robot nb, parent[], foot_body[] (one tree topology).  Everything else may differ:
+ * joint placements, axes, inertial parameters, sole placements, limits, gravity, every weight, x_ref, the cone parameters, kp / kd,
+ * contact_place, mu_contact and the centroidal mass, com_ref and weights.  The gait (mpc_gait_setup) stays uniform: f_half, the
+ * control references and the initial soles are the same for every robot.  With per-instance models set, mpc_rbd_terms* and
+ * mpc_ikid_terms* evaluate state i with model i and need count == batch.  One DevModel (about 21 KB) per instance is allocated on the
+ * first call and counted by mpc_workspace_bytes. */
+int32_t mpc_set_instance_models(mpc_solver_t *h, const mpc_robot_t *robots, const mpc_config_t *cfgs);
 /* problem.x0_init = x (full:536); host pointer [batch][nx]. */
 int32_t mpc_set_x0(mpc_solver_t *h, const double *x0);
 

@@ -14,6 +14,7 @@ dp = C.POINTER(C.c_double)
 
 EXPORTS = [
     "mpc_create", "mpc_destroy", "mpc_last_error", "mpc_setup", "mpc_update_knots", "mpc_update_terms", "mpc_cycle", "mpc_set_x0", "mpc_shift_multipliers", "mpc_reconfigure",
+    "mpc_set_instance_models",
     "mpc_run", "mpc_run_pipelined", "mpc_run_device", "mpc_tick", "mpc_get_results", "mpc_export_results_device", "mpc_result_ptrs", "mpc_get_stage_data", "mpc_last_launches", "mpc_last_device_ms",
     "mpc_get_feedback", "mpc_last_kernel_ms", "mpc_last_kernel_launches", "mpc_set_profiling",
     "mpc_qp_create", "mpc_qp_destroy", "mpc_qp_last_error", "mpc_qp_default_settings", "mpc_qp_update", "mpc_qp_solve", "mpc_qp_solve_device",
@@ -44,6 +45,7 @@ def lib():
         L.mpc_set_x0.argtypes = [C.c_void_p, dp]
         L.mpc_shift_multipliers.argtypes = [C.c_void_p, C.c_int32]
         L.mpc_reconfigure.argtypes = [C.c_void_p, C.POINTER(_abi.Robot), C.POINTER(_abi.Config)]
+        L.mpc_set_instance_models.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.mpc_run.argtypes = [C.c_void_p, dp, dp, C.c_int32]
         L.mpc_run_pipelined.argtypes = [C.c_void_p, dp, dp, C.c_int32, C.c_int32, dp, dp, dp, C.c_void_p]
         L.mpc_tick.argtypes = [C.c_void_p, C.c_void_p, dp, C.c_int32, C.c_int32]

@@ -87,6 +87,22 @@ class BatchSolver:
         self.robot, self.cfg = robot, cfg
         _native.check(_native.lib().mpc_reconfigure(self._h, C.byref(robot), C.byref(cfg)), "mpc_reconfigure")
 
+    def set_instance_models(self, robots=None, cfgs=None):
+        """Per-instance robot parameters and cost constants: instance i is solved with robots[i] / cfgs[i] (sequences of length batch of
+        _abi.Robot / _abi.Config; None = the shared robot / config for every instance; both None = back to the shared model).  Kind,
+        horizon, dt, solver constants and the tree topology stay those of the handle (`mpc_set_instance_models`, include/mpcb200.h)."""
+        B = self.batch
+        arrs = []
+        for seq, typ in ((robots, _abi.Robot), (cfgs, _abi.Config)):
+            if seq is None:
+                arrs.append(None)
+                continue
+            if len(seq) != B:
+                raise ValueError(f"set_instance_models: expected {B} {typ.__name__} blocks (one per instance), got {len(seq)}")
+            arrs.append((typ * B)(*seq))
+        _native.check(_native.lib().mpc_set_instance_models(self._h, *[None if a is None else C.cast(a, C.c_void_p) for a in arrs]),
+                      "mpc_set_instance_models")
+
     def shift_multipliers(self, n=1):
         _native.check(_native.lib().mpc_shift_multipliers(self._h, int(n)), "mpc_shift_multipliers")
 
@@ -194,7 +210,7 @@ class BatchSolver:
 
     def rbd_terms(self, x):
         """Rigid-body terms of the whole-body QPs for the states x [count][nx] (what kinodynamic_talos.py:425-431 takes from pinocchio):
-        dict(M, nle, Jc, dJv, vf).  Uses only the handle's robot model."""
+        dict(M, nle, Jc, dJv, vf).  With per-instance models set, state i uses instance i's robot and count must equal the batch."""
         x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, 57)
         B = x.shape[0]
         o = dict(M=np.zeros((B, 28, 28)), nle=np.zeros((B, 28)), Jc=np.zeros((B, 12, 28)), dJv=np.zeros((B, 12)), vf=np.zeros((B, 2, 6)))
@@ -204,7 +220,7 @@ class BatchSolver:
     def ikid_terms(self, x, frames):
         """Rigid-body terms and task terms of the IKID QP (IKIDSolver_f6, QP_utils.py:666-675) for the states x [count][nx]:
         (M, qp_utils.RBDTermsIKID).  frames = ((body, placement 12), (body, placement 12)) of the base and torso frames, whose LOCAL
-        angular Jacobians and dJ v are returned.  Uses only the handle's robot model."""
+        angular Jacobians and dJ v are returned.  With per-instance models set, state i uses instance i's robot and count must equal the batch."""
         x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, 57)
         B = x.shape[0]
         fb = np.ascontiguousarray([f[0] for f in frames], dtype=np.int32)

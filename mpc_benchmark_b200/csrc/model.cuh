@@ -4,6 +4,7 @@
 #pragma once
 #include "../../include/mpcb200.h"
 #include "dev_common.cuh"
+#include <string>
 
 namespace mpcdev {
 
@@ -82,6 +83,36 @@ inline int build_dev_model(const mpc_robot_t *rb, const mpc_config_t *cfg, DevMo
   m->total_mass = 0;
   for (int b = 0; b < NB; b++) m->total_mass += rb->mass[b];
   return 0;
+}
+
+// Per-instance models of a batch (mpc_set_instance_models): out[i] is built from robots[i] / cfgs[i], or from the shared robot / config
+// of `shared` where the array is null.  What the kernels of one launch must agree on stays uniform and is checked here: the model kind,
+// horizon and time step (workspace shape and Riccati dimensions), the solver constants (one BCL / linesearch schedule per handle, read from
+// Ws::sc and instance 0's model) and the tree topology (parent array and sole bodies: the tree tables are built once per shape).  Returns
+// an empty string, or an error naming the first offending instance and field.
+inline std::string build_instance_models(const DevModel &shared, const mpc_robot_t *robots, const mpc_config_t *cfgs, int batch, DevModel *out) {
+  const mpc_robot_t &r0 = shared.rb;
+  const mpc_config_t &c0 = shared.cfg;
+  for (int i = 0; i < batch; i++) {
+    const mpc_robot_t &r = robots ? robots[i] : r0;
+    const mpc_config_t &c = cfgs ? cfgs[i] : c0;
+    auto bad = [&](const char *field) { return "mpc_set_instance_models: instance " + std::to_string(i) + ": " + field + " differs from the handle's"; };
+    if (c.kind != c0.kind) return bad("cfg.kind");
+    if (c.T != c0.T) return bad("cfg.T");
+    if (c.dt != c0.dt) return bad("cfg.dt");
+    if (c.tol != c0.tol) return bad("cfg.tol");
+    if (c.mu_init != c0.mu_init) return bad("cfg.mu_init");
+    if (c.max_iters != c0.max_iters) return bad("cfg.max_iters");
+    if (c.force_initial_condition != c0.force_initial_condition) return bad("cfg.force_initial_condition");
+    if (c.rollout != c0.rollout) return bad("cfg.rollout");
+    if (c.lq_legs != c0.lq_legs) return bad("cfg.lq_legs");
+    if (r.nb != r0.nb) return bad("robot.nb");
+    for (int b = 0; b < NB; b++) if (r.parent[b] != r0.parent[b]) return bad("robot.parent");
+    if (r.foot_body[0] != r0.foot_body[0] || r.foot_body[1] != r0.foot_body[1]) return bad("robot.foot_body");
+    const char *err = nullptr;
+    if (build_dev_model(&r, &c, out + i, &err)) return "mpc_set_instance_models: instance " + std::to_string(i) + ": " + err;
+  }
+  return std::string();
 }
 #endif
 

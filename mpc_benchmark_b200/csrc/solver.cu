@@ -75,6 +75,12 @@ template <int KIND> __global__ void __launch_bounds__(RolloutShape<KIND>::TH) k_
   __shared__ double red[8];
   rollout_linesearch<KIND>(w, list[blockIdx.x], smem_raw, reinterpret_cast<double *>(smem_raw + EvalShape<KIND, false>::slice), red, next_eval);
 }
+// centroidal: 32-thread CTAs of 8 KB shared memory, so registers set the CTAs per SM; asking for 16 keeps the kernel at <= 128 registers
+template <> __global__ void __launch_bounds__(32, 16) k_rollout_ls<MPC_KIND_CENT>(Ws w, const int32_t *list, int32_t *next_eval) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ double red[8];
+  rollout_linesearch<MPC_KIND_CENT>(w, list[blockIdx.x], smem_raw, reinterpret_cast<double *>(smem_raw + EvalShape<MPC_KIND_CENT, false>::slice), red, next_eval);
+}
 
 template <int KIND> __global__ void __launch_bounds__(256) k_riccati(Ws w, const int32_t *list) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -117,13 +123,13 @@ __global__ void k_cycle(Ws w, const mpc_knot_t *last) {
   for (int i = threadIdx.x; i < nd; i += blockDim.x) kn[(w.T - 1) * nd + i] = reinterpret_cast<const double *>(last + b)[i];
 }
 
-// rigid-body terms of the whole-body QPs for `count` states (rbd_terms.cuh): one 128-thread CTA per state
-__global__ void __launch_bounds__(128) k_rbd_terms(const DevModel *model, const double *x, int count, double *M, double *nle, double *Jc, double *dJv, double *vf) {
+// rigid-body terms of the whole-body QPs for `count` states (rbd_terms.cuh): one 128-thread CTA per state, state i with model[i * model_stride]
+__global__ void __launch_bounds__(128) k_rbd_terms(const DevModel *model, int model_stride, const double *x, int count, double *M, double *nle, double *Jc, double *dJv, double *vf) {
   extern __shared__ double rbd_smem[];
   const int i = blockIdx.x;
   if (i >= count) return;
   FullWsT<false> &w = *reinterpret_cast<FullWsT<false> *>(rbd_smem);
-  rbd_terms_group(*model, x + (size_t)i * (NQ + NV), w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV, dJv + (size_t)i * 12, vf + (size_t)i * 12);
+  rbd_terms_group(model[(size_t)i * model_stride], x + (size_t)i * (NQ + NV), w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV, dJv + (size_t)i * 12, vf + (size_t)i * 12);
 }
 
 // the same terms plus the IKID QP's task terms (ikid_terms_group) of two frames for `count` states, one 128-thread CTA per state
@@ -131,13 +137,13 @@ struct IkidFrames {
   int32_t body[2];
   double place[24];
 };
-__global__ void __launch_bounds__(128) k_ikid_terms(const DevModel *model, const double *x, int count, const IkidFrames fr, double *M, double *nle, double *Jc,
+__global__ void __launch_bounds__(128) k_ikid_terms(const DevModel *model, int model_stride, const double *x, int count, const IkidFrames fr, double *M, double *nle, double *Jc,
                                                     double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
   extern __shared__ double rbd_smem[];
   const int i = blockIdx.x;
   if (i >= count) return;
   FullWsT<false> &w = *reinterpret_cast<FullWsT<false> *>(rbd_smem);
-  ikid_terms_group(*model, x + (size_t)i * (NQ + NV), fr.body, fr.place, w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV,
+  ikid_terms_group(model[(size_t)i * model_stride], x + (size_t)i * (NQ + NV), fr.body, fr.place, w, M + (size_t)i * NV * NV, nle + (size_t)i * NV, Jc + (size_t)i * 12 * NV,
                    dJv + (size_t)i * 12, Ag + (size_t)i * 6 * NV, dAgv + (size_t)i * 6, Jang + (size_t)i * 6 * NV, dJang + (size_t)i * 6);
 }
 
@@ -147,15 +153,16 @@ __global__ void __launch_bounds__(128) k_gait_tick(Ws w, const GaitCfg *g, GaitR
   const size_t b = blockIdx.x;
   gait_tick_group(*g, robots[b], t, lf ? lf + b * 12 : nullptr, rf ? rf + b * 12 : nullptr, w.knots + b * w.T, w.terms + b, sm);
 }
-// sole placements at the state the next tick starts from (the model prediction xs[1]): forward kinematics of the evaluation kernel
-__global__ void __launch_bounds__(128) k_feet_of_prediction(Ws w, const DevModel *model, double *lf, double *rf) {
+// sole placements at the state the next tick starts from (the model prediction xs[1]): forward kinematics of the evaluation kernel with
+// each robot's own model
+__global__ void __launch_bounds__(128) k_feet_of_prediction(Ws w, double *lf, double *rf) {
   extern __shared__ double rbd_smem[];
   const size_t b = blockIdx.x;
   FullWsT<false> &ws = *reinterpret_cast<FullWsT<false> *>(rbd_smem);
   const double *x = w.xs + b * ((size_t)w.T + 1) * w.nx + w.nx;
   PAR_FOR(i, NQ + NV) ws.x[i] = x[i];
   SYNC();
-  mb_kinematics(*model, ws);
+  mb_kinematics(model_of(w, (int)b), ws);
   PAR_FOR(i, 12) { lf[b * 12 + i] = ws.ofoot[i]; rf[b * 12 + i] = ws.ofoot[12 + i]; }
 }
 
@@ -192,6 +199,9 @@ struct mpc_solver {
   Ws w{};
   DevModel *d_model = nullptr;
   DevModel h_model;
+  // per-instance models (mpc_set_instance_models): [batch] DevModels, allocated on first use; w.model points here while instance_models
+  DevModel *d_models = nullptr;
+  bool instance_models = false;
   std::vector<void *> allocs;
   double *d_xs_in = nullptr, *d_us_in = nullptr, *d_meas = nullptr;
   mpc_knot_t *d_last = nullptr;
@@ -388,6 +398,7 @@ void mpc_destroy(mpc_solver_t *h) {
   if (h->d_meas) cudaFree(h->d_meas);
   if (h->d_last) cudaFree(h->d_last);
   if (h->d_model) cudaFree(h->d_model);
+  if (h->d_models) cudaFree(h->d_models);
   if (h->h_counters) cudaFreeHost(h->h_counters);
   if (h->h_st) cudaFreeHost(h->h_st);
   if (h->d_k0) cudaFree(h->d_k0);
@@ -488,6 +499,7 @@ int32_t mpc_shift_multipliers(mpc_solver_t *h, int32_t n) {
 // swap in new model / weight constants without touching the workspace (same kind, horizon and batch)
 int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_config_t *cfg) {
   CK(cudaSetDevice(h->device));
+  if (h->instance_models) return fail("mpc_reconfigure: per-instance models are set; clear them first with mpc_set_instance_models(h, NULL, NULL)");
   if (cfg->kind != h->w.kind || cfg->T != h->w.T) return fail("mpc_reconfigure: kind / horizon must not change");
   if (const char *le = check_lq_legs(cfg)) return fail(std::string("mpc_reconfigure: ") + le);
   const char *err = nullptr;
@@ -496,6 +508,31 @@ int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_con
   h->w.sc = default_consts(cfg->tol, cfg->mu_init, cfg->rollout);
   CK(cudaMemcpyAsync(h->d_model, &h->h_model, sizeof(DevModel), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+// one DevModel per instance (robots / cfgs [batch], NULL = the handle's shared robot / config), or back to the shared model (both NULL)
+int32_t mpc_set_instance_models(mpc_solver_t *h, const mpc_robot_t *robots, const mpc_config_t *cfgs) {
+  if (!h) return fail("null handle");
+  CK(cudaSetDevice(h->device));
+  Ws &w = h->w;
+  if (!robots && !cfgs) {
+    CK(cudaStreamSynchronize(h->stream)); // no kernel of the handle still reads the per-instance models
+    w.model = h->d_model; w.model_stride = 0;
+    h->instance_models = false;
+    return 0;
+  }
+  std::vector<DevModel> models(w.B);
+  const std::string err = build_instance_models(h->h_model, robots, cfgs, w.B, models.data());
+  if (!err.empty()) return fail(err);
+  if (!h->d_models && cudaMalloc(&h->d_models, sizeof(DevModel) * (size_t)w.B) != cudaSuccess) {
+    h->d_models = nullptr;
+    return fail("cudaMalloc(per-instance models) failed");
+  }
+  CK(cudaMemcpyAsync(h->d_models, models.data(), sizeof(DevModel) * (size_t)w.B, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  w.model = h->d_models; w.model_stride = 1;
+  h->instance_models = true;
   return 0;
 }
 
@@ -743,7 +780,7 @@ int32_t mpc_get_feedback(mpc_solver_t *h, int32_t k, double *K) {
   return 0;
 }
 double mpc_last_device_ms(mpc_solver_t *h) { return h->last_ms; }
-uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return h->bytes + h->leg_bytes; }
+uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return h->bytes + h->leg_bytes + (h->d_models ? sizeof(DevModel) * (size_t)h->w.B : 0); }
 // per-phase cycle counters of the Riccati kernel for instance 0 (all zero unless built with -DMPC_PHASE_TIMING)
 int32_t mpc_debug_phases(mpc_solver_t *h, double *out64) {
   CK(cudaSetDevice(h->device));
@@ -831,15 +868,20 @@ double mpc_measure_fp64_peak(int32_t device) { return time_peak(device, k_dfma_p
 double mpc_measure_fp64_peak_dmma(int32_t device) { return time_peak(device, k_dmma_peak, 256, 1 << 14, 512.0 * 8 / 32); }
 
 // ---- rigid-body terms in front of the whole-body QPs (include/mpcb200.h)
+// with per-instance models, state i is evaluated with instance i's model: only a full batch of states has a model for each
+static const char *check_model_count(const mpc_solver *h, int count) {
+  return (h->instance_models && count != h->w.B) ? "per-instance models are set: count must equal the solver batch" : nullptr;
+}
 int32_t mpc_rbd_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, uint64_t M_dev, uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t vf_dev,
                              uint64_t stream) {
   if (!h) return fail("null handle");
   if (h->w.kind == MPC_KIND_CENT) return fail("mpc_rbd_terms: the centroidal model has no rigid-body tree");
   if (count <= 0) return fail("mpc_rbd_terms: count out of range");
+  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_rbd_terms: ") + e);
   CK(cudaSetDevice(h->device));
   const size_t smem = sizeof(FullWsT<false>);
   CK(cudaFuncSetAttribute(k_rbd_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); // per device: set on every call (microseconds)
-  k_rbd_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->d_model, (const double *)x_dev, count, (double *)M_dev, (double *)nle_dev,
+  k_rbd_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, (double *)M_dev, (double *)nle_dev,
                                                                                   (double *)Jc_dev, (double *)dJv_dev, (double *)vf_dev);
   CK(cudaGetLastError());
   return 0;
@@ -847,6 +889,7 @@ int32_t mpc_rbd_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, uin
 int32_t mpc_rbd_terms(mpc_solver_t *h, int32_t count, const double *x, double *M, double *nle, double *Jc, double *dJv, double *vf) {
   if (!h) return fail("null handle");
   if (count <= 0) return fail("mpc_rbd_terms: count out of range");
+  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_rbd_terms: ") + e);
   CK(cudaSetDevice(h->device));
   const size_t B = count, per = (NQ + NV) + NV * NV + NV + 12 * NV + 12 + 12;
   double *d = nullptr;
@@ -868,6 +911,7 @@ int32_t mpc_ikid_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, co
   if (!h || !frame_body || !frame_place) return fail("null handle / frames");
   if (h->w.kind == MPC_KIND_CENT) return fail("mpc_ikid_terms: the centroidal model has no rigid-body tree");
   if (count <= 0) return fail("mpc_ikid_terms: count out of range");
+  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_ikid_terms: ") + e);
   if (frame_body[0] < 0 || frame_body[0] >= NB || frame_body[1] < 0 || frame_body[1] >= NB) return fail("mpc_ikid_terms: frame body out of range [0, nb)");
   CK(cudaSetDevice(h->device));
   IkidFrames fr;
@@ -877,7 +921,7 @@ int32_t mpc_ikid_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, co
   }
   const size_t smem = sizeof(FullWsT<false>);
   CK(cudaFuncSetAttribute(k_ikid_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_ikid_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->d_model, (const double *)x_dev, count, fr, (double *)M_dev, (double *)nle_dev,
+  k_ikid_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, fr, (double *)M_dev, (double *)nle_dev,
                                                                                    (double *)Jc_dev, (double *)dJv_dev, (double *)Ag_dev, (double *)dAgv_dev,
                                                                                    (double *)Jang_dev, (double *)dJang_dev);
   CK(cudaGetLastError());
@@ -887,6 +931,7 @@ int32_t mpc_ikid_terms(mpc_solver_t *h, int32_t count, const double *x, const in
                        double *Jc, double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
   if (!h) return fail("null handle");
   if (count <= 0) return fail("mpc_ikid_terms: count out of range");
+  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_ikid_terms: ") + e);
   CK(cudaSetDevice(h->device));
   const size_t B = count, per = (NQ + NV) + NV * NV + NV + 12 * NV + 12 + 6 * NV + 6 + 6 * NV + 6;
   double *d = nullptr;
@@ -954,7 +999,7 @@ int32_t mpc_gait_tick(mpc_solver_t *h, const double *lf, const double *rf) {
   } else {
     const size_t smem = sizeof(FullWsT<false>);
     CK(cudaFuncSetAttribute(k_feet_of_prediction, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); // per device: set on every call
-    k_feet_of_prediction<<<w.B, 128, smem, h->stream>>>(w, h->d_model, dl, dr);
+    k_feet_of_prediction<<<w.B, 128, smem, h->stream>>>(w, dl, dr);
   }
   k_gait_tick<<<w.B, 128, 0, h->stream>>>(w, h->d_gait, h->d_gait_robots, h->gait_t, dl, dr);
   CK(cudaGetLastError());

@@ -47,6 +47,7 @@ struct InstState {
 struct Ws {
   int B, T, kind, nx, n, m, nc, nz;
   const DevModel *model;
+  int model_stride; // DevModels between consecutive instances: 0 = one model shared by the batch, 1 = one per instance
   SolverConst sc;
   mpc_knot_t *knots; mpc_term_t *terms; double *x0;
   double *xs, *us, *vs, *lams, *vs_prev, *lams_prev;
@@ -62,6 +63,8 @@ struct Ws {
   double *phase;     // 16 doubles: per-phase cycle counters of instance 0 (MPC_PHASE_TIMING builds)
   int32_t *lists;    // [4][B] compacted instance lists: 0,1 = evaluation lists (double-buffered), 2,3 = linesearch lists
 };
+// the robot / problem constants of instance b
+HDH const DevModel &model_of(const Ws &w, int b) { return w.model[(size_t)b * w.model_stride]; }
 HDH int32_t *eval_list(const Ws &w, int which) { return w.lists + (size_t)(which & 1) * w.B; }
 HDH int32_t *ls_list(const Ws &w, int which) { return w.lists + (size_t)(2 + (which & 1)) * w.B; }
 
@@ -97,6 +100,7 @@ HD void init_instance(const Ws &w, int b, const double *xs_in, const double *us_
   PAR_FOR(i, (int)(T1 * w.nx)) w.xs[b * T1 * w.nx + i] = xs_in[b * T1 * w.nx + i];
   PAR_FOR(i, w.T * w.m) w.us[(size_t)b * w.T * w.m + i] = us_in[(size_t)b * w.T * w.m + i];
   SYNC();
+  // force_initial_condition is uniform over the batch (build_instance_models): instance 0's model answers for every instance
   if (w.model->cfg.force_initial_condition) PAR_FOR(i, w.nx) w.xs[b * T1 * w.nx + i] = w.x0[(size_t)b * w.nx + i];
   PAR_FOR(i, (int)(T1 * w.nc)) w.vs_prev[b * T1 * w.nc + i] = w.vs[b * T1 * w.nc + i];
   PAR_FOR(i, (int)(T1 * w.n)) w.lams_prev[b * T1 * w.n + i] = w.lams[b * T1 * w.n + i];
@@ -313,7 +317,8 @@ template <int KIND, bool DERIV> HD void eval_dispatch(const Ws &w, int b, int k,
   if (mode != (DERIV ? MODE_EVAL : MODE_LS)) return;
   KnotIO io = make_io(w, b, k, !DERIV);
   auto &f = *reinterpret_cast<typename K::template EvalWs<DERIV> *>(smem);
-  if (k < w.T) K::template knot<DERIV>(*w.model, io, f); else K::template term<DERIV>(*w.model, io, f);
+  const DevModel &md = model_of(w, b);
+  if (k < w.T) K::template knot<DERIV>(md, io, f); else K::template term<DERIV>(md, io, f);
 }
 
 // ---- ROLLOUT_NONLINEAR: one trial point of the fused rollout + linesearch kernel (one CTA = one evaluation group per instance).
@@ -330,6 +335,7 @@ template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void
   const int ldw = (KIND == MPC_KIND_CENT) ? nz : ((nz + 7) & ~7);
   double *dx = xv, *z = xv + 64, *slack = xv + 160;
   const double mu = w.st[b].mu, mu_d = mu;
+  const DevModel &md = model_of(w, b);
   const double *xs = w.xs + b * T1 * nx, *us = w.us + (size_t)b * T * m, *vs = w.vs + b * T1 * nc, *lams = w.lams + b * T1 * n;
   double *txs = w.txs + b * T1 * nx, *tus = w.tus + (size_t)b * T * m, *tvs = w.tvs + b * T1 * nc, *tlams = w.tlams + b * T1 * n;
   const double *lams_prev = w.lams_prev + b * T1 * n, *dbar = w.dbar + b * T1 * nc;
@@ -366,7 +372,7 @@ template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void
       }
       SYNC();
       KnotIO io = make_io(w, b, k, true);
-      K::template term<false>(*w.model, io, f);
+      K::template term<false>(md, io, f);
       SYNC();
       break;
     }
@@ -392,7 +398,7 @@ template <int KIND> HD void rollout_trial(const Ws &w, int b, double alpha, void
     SYNC();
     KnotIO io = make_io(w, b, k, true);
     io.xn = io.x; io.slack = slack; io.xn_out = txs + (size_t)(k + 1) * nx;
-    K::template knot<false, true>(*w.model, io, f);
+    K::template knot<false, true>(md, io, f);
     SYNC();
   }
 }

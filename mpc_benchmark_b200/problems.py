@@ -287,6 +287,41 @@ def sub_problem(prob, lo, hi):
     return out
 
 
+def perturbed_robots(robot, batch, seed, mass=0.1, com=0.01, payload=0.0, payload_com=(0.0, 0.0, 0.25), payload_body=None, jplace=0.0):
+    """`batch` copies of `robot` with randomised inertial parameters, for BatchSolver.set_instance_models (domain randomisation,
+    robustness studies).  Per body, with `default_rng(seed)`:
+      - mass and rotational inertia scaled together by one factor uniform in [1 - mass, 1 + mass] (the inertia stays physically valid);
+      - CoM shifted by a normal offset of standard deviation `com` metres per axis;
+      - a point payload uniform in [0, payload] kg at `payload_com` in `payload_body` (default: the Talos-shaped torso) merged into that
+        body's mass, CoM and inertia about the new CoM (parallel-axis theorem).
+    The kinematics (joint placements, sole frames) are left alone, so nominal x0 and sole references stay valid, unless `jplace` > 0:
+    then every joint translation gets a normal offset of standard deviation `jplace` metres per axis.  Instance 0 is randomised too."""
+    from .talos_like import JOINT_NAMES
+
+    rng = np.random.default_rng(seed)
+    pb = JOINT_NAMES.index("torso_2_joint") if payload_body is None else int(payload_body)
+    out = []
+    for _ in range(batch):
+        rb = _abi.Robot.from_buffer_copy(robot)
+        for b in range(robot.nb):
+            s = rng.uniform(1.0 - mass, 1.0 + mass)
+            rb.mass[b] = robot.mass[b] * s
+            rb.inertia[b][:] = list(np.asarray(robot.inertia[b][:]) * s)
+            rb.com[b][:] = list(np.asarray(robot.com[b][:]) + rng.normal(size=3) * com)
+            if jplace > 0 and b > 0:
+                rb.jplace[b][9:12] = list(np.asarray(robot.jplace[b][9:12]) + rng.normal(size=3) * jplace)
+        p = rng.uniform(0.0, payload) if payload > 0 else 0.0
+        if p > 0:
+            m0, c0, r = rb.mass[pb], np.asarray(rb.com[pb][:]), np.asarray(payload_com, float)
+            m1 = m0 + p
+            c1 = (m0 * c0 + p * r) / m1
+            shift = lambda mm, d: mm * (d @ d * np.eye(3) - np.outer(d, d))  # noqa: E731
+            I1 = np.asarray(rb.inertia[pb][:]).reshape(3, 3) + shift(m0, c0 - c1) + shift(p, r - c1)
+            rb.mass[pb], rb.com[pb][:], rb.inertia[pb][:] = m1, list(c1), list(I1.reshape(9))
+        out.append(rb)
+    return out
+
+
 def lq_flops(n, m, c):
     """ALGORITHMIC dense-LQ FLOPs per knot (SURVEY 8d): backward + forward."""
     s = m + c

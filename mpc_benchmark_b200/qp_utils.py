@@ -75,7 +75,7 @@ class IDSolver_ulim:
     def solve_from_state(self, solver, x_measured, cs, a, forces):
         """kinodynamic_talos.py:425-445 in one call for the whole batch: the pinocchio step (crba, nonLinearEffects, frame Jacobians and
         their time variation at the MEASURED states x_measured [batch][57]) runs on the device through `solver` (a batch.BatchSolver of
-        the same robot), then the assembly and the QP."""
+        the same robot, or with per-instance models and the QP's batch: robot i for state i), then the assembly and the QP."""
         self.qp.assemble_id_from_state(solver, x_measured, a, forces, cs, self.mu, self.L, self.W, float(self.baum_Kd[0, 0]))
         self.qp.solve()
         nv, nf = self.model.nv, self.force_size * self.nk
@@ -181,8 +181,8 @@ class IKIDSolver_f6:
                          dtorso_diff, forces, dH):
         """centroidal_talos.py:435-445 in one call for the whole batch: the pinocchio step (crba, nonLinearEffects, the contact, base and
         torso frame Jacobians with their time variation, the centroidal momentum matrix and dAg v at the MEASURED states x_measured
-        [batch][57]) runs on the device through `solver` (a kinodynamic or full-dynamics batch.BatchSolver of the same robot), then the
-        whole cost and constraint assembly and the QP.  Only x, the task errors, forces and cs are uploaded per robot.  Returns what
+        [batch][57]) runs on the device through `solver` (a kinodynamic or full-dynamics batch.BatchSolver of the same robot, or with
+        per-instance models and the QP's batch: robot i for state i), then the whole cost and constraint assembly and the QP.  Only x, the task errors, forces and cs are uploaded per robot.  Returns what
         `solve` returns.  The base / torso rows use the LOCAL frame."""
         B = self.batch
         f = lambda a, per: np.broadcast_to(np.asarray(a, float).reshape(-1, per), (B, per))  # noqa: E731
