@@ -112,44 +112,13 @@ template <bool DERIV, bool ROLL = false> HD void eval_full_knot(const DevModel &
   double *X = io.scratch, *DL = io.scratch + NV * FNZ; // derivative pass only (null otherwise)
   double *Yr = DERIV ? DL : w.Y;
   const double a0[6] = {-rb.gravity[0], -rb.gravity[1], -rb.gravity[2], 0, 0, 0};
-  // bias accelerations (qdd = 0, gravity folded in) and bias forces
-  PAR_FOR(b, NB) {
-    double acc[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
-    uint32_t mask = m.anc_mask[b];
-    for (int k = 1; k <= b; k++)
-      if (mask >> k & 1) {
-        double sj[6], c[6];
-        for (int i = 0; i < 6; i++) sj[i] = w.S[6 * (5 + k) + i] * w.x[NQ + 5 + k];
-        cross_mm(w.v + 6 * k, sj, c);
-        for (int i = 0; i < 6; i++) acc[i] += c[i];
-      }
-    for (int i = 0; i < 6; i++) w.a[6 * b + i] = acc[i];
-    double t1[6], t2[6];
-    inertia_mul(w.I + 10 * b, acc, t1);
-    cross_mf(w.v + 6 * b, w.hb + 6 * b, t2);
-    for (int i = 0; i < 6; i++) w.f[6 * b + i] = t1[i] + t2[i];
-  }
+  mb_bias_forces(m, w, a0); // qdd = 0
   SYNC();
-  PAR_FOR(e, NB * 6) {
-    int b = e / 6, c = e % 6;
-    uint32_t mask = m.sub_mask[b];
-    double s = 0;
-    for (int d = b; d < NB; d++) if (mask >> d & 1) s += w.f[6 * d + c];
-    w.Fsub[e] = s;
-  }
-  PAR_FOR(e, NV * NV) { // CRBA
-    int i = e / NV, j = e % NV, bi = body_of_dof(i), bj = body_of_dof(j);
-    double v = 0;
-    if (m.anc_mask[bj] >> bi & 1) v = dot6(w.S + 6 * i, w.U + 6 * j);
-    else if (m.anc_mask[bi] >> bj & 1) v = dot6(w.S + 6 * j, w.U + 6 * i);
-    w.M[e] = v;
-  }
+  mb_subtree_sum<6>(m, w.f, w.Fsub);
+  mb_crba(m, w, w.M);
   PAR_FOR(c, nact) { // contact kinematics + Baumgarte terms
-    int f = w.act[c], fb = rb.foot_body[f];
-    se3_actinv_motion(w.ofoot + 12 * f, w.v + 6 * fb, w.vc + 6 * c);
-    double an[6];
-    for (int i = 0; i < 6; i++) an[i] = w.a[6 * fb + i] - a0[i];
-    se3_actinv_motion(w.ofoot + 12 * f, an, w.gam + 6 * c);
+    const int f = w.act[c];
+    mb_sole_motion(m, w, f, a0, w.vc + 6 * c, w.gam + 6 * c);
     se3_inv_mul(w.ofoot + 12 * f, cfg.contact_place[f], w.c1Mc2 + 12 * c);
     double lg[6];
     log6(w.c1Mc2 + 12 * c, lg);
@@ -230,58 +199,34 @@ template <bool DERIV, bool ROLL = false> HD void eval_full_knot(const DevModel &
     }
     SYNC();
     PAR_FOR(b, NB) {
-      double t1[6], t2[6];
-      inertia_mul(w.I + 10 * b, w.a + 6 * b, t1);
-      cross_mf(w.v + 6 * b, w.hb + 6 * b, t2);
-      for (int i = 0; i < 6; i++) t1[i] += t2[i];
+      double fb[6];
+      mb_body_force(w, b, w.a + 6 * b, fb);
       for (int c = 0; c < nact; c++)
         if (rb.foot_body[w.act[c]] == b) {
           double fw[6];
           se3_act_force(w.ofoot + 12 * w.act[c], w.rhs + 6 * c, fw);
-          for (int i = 0; i < 6; i++) t1[i] -= fw[i];
+          for (int i = 0; i < 6; i++) fb[i] -= fw[i];
         }
-      for (int i = 0; i < 6; i++) w.f[6 * b + i] = t1[i];
+      for (int i = 0; i < 6; i++) w.f[6 * b + i] = fb[i];
     }
     PAR_FOR(e, NV * FNZ) X[e] = 0.0;
     PAR_FOR(e, 12 * FNZ) DL[e] = 0.0;
     SYNC();
-    PAR_FOR(e, NB * 6) {
-      int b = e / 6, c = e % 6;
-      uint32_t mask = m.sub_mask[b];
-      double s = 0;
-      for (int d = b; d < NB; d++) if (mask >> d & 1) s += w.f[6 * d + c];
-      w.Fsub[e] = s;
-    }
+    mb_subtree_sum<6>(m, w.f, w.Fsub);
     EPH(5);
     mb_composite_B(m, w);
     EPH(6);
     PAR_FOR(e, 2 * m.npairs) {
-      int kind = e / m.npairs, p = e % m.npairs;
-      int j = m.pair_j[p], mb = m.pair_m[p], J = body_of_dof(j), pJ = rb.parent[J];
-      const double *s = w.S + 6 * j;
-      double vp[6] = {0, 0, 0, 0, 0, 0}, ap[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
-      if (pJ >= 0) for (int i = 0; i < 6; i++) { vp[i] = w.v[6 * pJ + i]; ap[i] = w.a[6 * pJ + i]; }
-      double cj[6], wj[6], t1[6], g[6], g2[6];
-      if (kind == 0) {
-        cross_mm(s, vp, wj);
-        cross_mm(s, ap, cj);
-        cross_mm(wj, vp, t1);
-        for (int i = 0; i < 6; i++) cj[i] -= t1[i];
-      } else {
-        for (int i = 0; i < 6; i++) { wj[i] = s[i]; t1[i] = w.v[6 * J + i] + vp[i]; }
-        cross_mm(s, t1, cj);
-        for (int i = 0; i < 6; i++) cj[i] = -cj[i];
-      }
-      inertia_mul(w.Ic + 10 * mb, cj, g);
-      mat6_vec(w.Bc + 36 * mb, wj, g2);
-      for (int i = 0; i < 6; i++) g[i] += g2[i];
+      const int kind = e / m.npairs, p = e % m.npairs, j = m.pair_j[p], mb = m.pair_m[p], J = body_of_dof(j);
+      double g[6], t1[6];
+      mb_force_column(m, w, kind, j, mb, a0, g);
       int i0 = first_dof(mb), nd = ndof_of(mb);
       for (int d = 0; d < nd; d++) {
         double val = dot6(w.S + 6 * (i0 + d), g);
         X[(i0 + d) * FNZ + kind * NV + j] = kind == 0 ? -val : val;
       }
       if (mb == J) {
-        if (kind == 0) { cross_mf(s, w.Fsub + 6 * J, t1); for (int i = 0; i < 6; i++) w.top[6 * j + i] = t1[i] - g[i]; }
+        if (kind == 0) { cross_mf(w.S + 6 * j, w.Fsub + 6 * J, t1); for (int i = 0; i < 6; i++) w.top[6 * j + i] = t1[i] - g[i]; }
         else for (int i = 0; i < 6; i++) w.top[6 * (NV + j) + i] = g[i];
       }
     }

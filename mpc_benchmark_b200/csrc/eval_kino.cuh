@@ -66,29 +66,8 @@ template <bool DERIV, bool ROLL = false> HD void eval_kino_knot(const DevModel &
   ONE_THREAD { w.active[0] = kn.cs[0] != 0.0; w.active[1] = kn.cs[1] != 0.0; }
   mb_kinematics(m, w);
   const double a0[6] = {-rb.gravity[0], -rb.gravity[1], -rb.gravity[2], 0, 0, 0};
-  // body accelerations for qdd = [0; a_j] (gravity folded in), forces, centroidal map
-  PAR_FOR(b, NB) {
-    double acc[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
-    uint32_t mask = m.anc_mask[b];
-    for (int k = 1; k <= b; k++)
-      if (mask >> k & 1) {
-        double sj[6], c[6];
-        for (int i = 0; i < 6; i++) sj[i] = w.S[6 * (5 + k) + i] * w.x[NQ + 5 + k];
-        cross_mm(w.v + 6 * k, sj, c);
-        for (int i = 0; i < 6; i++) acc[i] += c[i] + w.S[6 * (5 + k) + i] * w.u[12 + k - 1];
-      }
-    for (int i = 0; i < 6; i++) w.a[6 * b + i] = acc[i];
-    double t1[6], t2[6];
-    inertia_mul(w.I + 10 * b, acc, t1);
-    cross_mf(w.v + 6 * b, w.hb + 6 * b, t2);
-    for (int i = 0; i < 6; i++) w.f[6 * b + i] = t1[i] + t2[i];
-  }
-  PAR_FOR(j, NV) { // A_g column j = shift_to_com(U_j)
-    const double *Uj = w.U + 6 * j;
-    double c[3];
-    cross3(w.com, Uj, c);
-    for (int r = 0; r < 3; r++) { w.Ag[r * NV + j] = Uj[r]; w.Ag[(3 + r) * NV + j] = Uj[3 + r] - c[r]; }
-  }
+  mb_bias_forces<true>(m, w, a0, w.u + 12); // qdd = [0; a_j]
+  mb_centroidal_map(w, w.Ag);
   SYNC();
   PAR_FOR(task, 64) {
     if (task == 0) { // total bias force at the CoM
@@ -116,10 +95,10 @@ template <bool DERIV, bool ROLL = false> HD void eval_kino_knot(const DevModel &
     if (i < 6) { double s = 0; for (int k = 0; k < 6; k++) s += w.Abi[6 * i + k] * (w.hd[k] - w.Fg0[k]); w.acc[i] = s; }
     else w.acc[i] = w.u[12 + i - 6];
   }
-  PAR_FOR(c, 2) { // LOCAL sole velocities (zero-velocity constraint values)
-    double vl[6] = {0, 0, 0, 0, 0, 0};
-    se3_actinv_motion(w.ofoot + 12 * c, w.v + 6 * rb.foot_body[c], vl);
-    for (int r = 0; r < 6; r++) w.vl[6 * c + r] = vl[r];
+  PAR_FOR(f, 2) { // LOCAL sole velocities (zero-velocity constraint values)
+    double vl[6];
+    mb_sole_motion<false>(m, w, f, a0, vl);
+    for (int r = 0; r < 6; r++) w.vl[6 * f + r] = vl[r];
   }
   SYNC();
   PAR_FOR(i, NV) { io.xdot[i] = w.x[NQ + i]; io.xdot[NV + i] = w.acc[i]; }
@@ -135,39 +114,15 @@ template <bool DERIV, bool ROLL = false> HD void eval_kino_knot(const DevModel &
     }
     PAR_FOR(e, NV * KNZ) w.X[e] = 0.0;
     SYNC();
-    PAR_FOR(b, NB) {
-      double t1[6], t2[6];
-      inertia_mul(w.I + 10 * b, w.a + 6 * b, t1);
-      cross_mf(w.v + 6 * b, w.hb + 6 * b, t2);
-      for (int i = 0; i < 6; i++) w.f[6 * b + i] = t1[i] + t2[i];
-    }
+    PAR_FOR(b, NB) mb_body_force(w, b, w.a + 6 * b, w.f + 6 * b);
     SYNC();
-    PAR_FOR(e, NB * 6) {
-      int b = e / 6, c = e % 6;
-      uint32_t mask = m.sub_mask[b];
-      double s = 0;
-      for (int d = b; d < NB; d++) if (mask >> d & 1) s += w.f[6 * d + c];
-      w.Fsub[e] = s;
-    }
+    mb_subtree_sum<6>(m, w.f, w.Fsub);
     mb_composite_B(m, w);
     PAR_FOR(e, 2 * NV) { // top vectors: d F_o/d q_j (kind 0), d F_o/d v_j (kind 1)
-      int kind = e / NV, j = e % NV, J = body_of_dof(j), pJ = rb.parent[J];
-      const double *s = w.S + 6 * j;
-      double vp[6] = {0, 0, 0, 0, 0, 0}, ap[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
-      if (pJ >= 0) for (int i = 0; i < 6; i++) { vp[i] = w.v[6 * pJ + i]; ap[i] = w.a[6 * pJ + i]; }
-      double cj[6], wj[6], t1[6], g[6], g2[6];
-      if (kind == 0) {
-        cross_mm(s, vp, wj); cross_mm(s, ap, cj); cross_mm(wj, vp, t1);
-        for (int i = 0; i < 6; i++) cj[i] -= t1[i];
-      } else {
-        for (int i = 0; i < 6; i++) { wj[i] = s[i]; t1[i] = w.v[6 * J + i] + vp[i]; }
-        cross_mm(s, t1, cj);
-        for (int i = 0; i < 6; i++) cj[i] = -cj[i];
-      }
-      inertia_mul(w.Ic + 10 * J, cj, g);
-      mat6_vec(w.Bc + 36 * J, wj, g2);
-      for (int i = 0; i < 6; i++) g[i] += g2[i];
-      if (kind == 0) { cross_mf(s, w.Fsub + 6 * J, t1); for (int i = 0; i < 6; i++) w.top[6 * j + i] = t1[i] - g[i]; }
+      const int kind = e / NV, j = e % NV, J = body_of_dof(j);
+      double g[6], t1[6];
+      mb_force_column(m, w, kind, j, J, a0, g);
+      if (kind == 0) { cross_mf(w.S + 6 * j, w.Fsub + 6 * J, t1); for (int i = 0; i < 6; i++) w.top[6 * j + i] = t1[i] - g[i]; }
       else for (int i = 0; i < 6; i++) w.top[6 * (NV + j) + i] = g[i];
     }
     PAR_FOR(j, NV) { // d hdot'/dq_j (angular rows): sum_i (dp_i/dq_j - dc/dq_j) x f_i

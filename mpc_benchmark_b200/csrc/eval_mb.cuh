@@ -1,7 +1,8 @@
-// What the full-dynamics and kinodynamic evaluations of a Talos knot share: the knot's I/O, the world-frame kinematics and
-// composite-inertia phases, the multibody cost stack (state, centroidal momentum, foot placements), the normal-cone projection,
-// the back end of a running knot (constraint rows and shooting gap -> merit partials and LQ blocks) and the terminal knot.
-// Each model file keeps its own dynamics, tangent, constraint-row definitions and extra cost terms.
+// What the full-dynamics and kinodynamic evaluations of a Talos knot share: the knot's I/O, the world-frame rigid-body phases
+// (kinematics, subtree sums, body forces, bias pass, CRBA, sole motion, centroidal map, composite inertias and force-derivative
+// columns; rbd_terms.cuh runs them too), the multibody cost stack (state, centroidal momentum, foot placements), the normal-cone
+// projection, the back end of a running knot (constraint rows and shooting gap -> merit partials and LQ blocks) and the terminal knot.
+// Each model file keeps its own dynamics solve, tangent assembly, constraint-row definitions and extra cost terms.
 #pragma once
 #include "model.cuh"
 
@@ -33,6 +34,29 @@ struct KnotIO {
                      // holds the tangent X = da/dz (NV x nz) and dlam/dz (12 x nz), which stay L2-resident between the phases
   double *phase_out; // profiling builds only
 };
+
+// ------------------------------------------------------------------ rigid-body phases
+// One copy of each recursion of the evaluations and of rbd_terms.cuh, after the oracle's (oracle/rbd.hpp).  A helper is either one
+// PAR_FOR phase or the body of one work item; none has a barrier inside, so every caller keeps its own SYNC() placement.
+
+// subtree sums dst_b = sum_{d in sub(b)} src_d of a per-body quantity W doubles wide, one thread per element
+template <int W> HD void mb_subtree_sum(const DevModel &m, const double *src, double *dst) {
+  PAR_FOR(e, NB * W) {
+    const int b = e / W, c = e % W;
+    const uint32_t mask = m.sub_mask[b];
+    double s = 0;
+    for (int d = b; d < NB; d++) if (mask >> d & 1) s += src[W * d + c];
+    dst[e] = s;
+  }
+}
+
+// body force I_b a_b + v_b x* (I_b v_b) for the body acceleration ab (hb = I_b v_b from mb_kinematics)
+template <class WS> HD void mb_body_force(const WS &w, int b, const double *ab, double *fb) {
+  double t1[6], t2[6];
+  inertia_mul(w.I + 10 * b, ab, t1);
+  cross_mf(w.v + 6 * b, w.hb + 6 * b, t2);
+  for (int i = 0; i < 6; i++) fb[i] = t1[i] + t2[i];
+}
 
 // ------------------------------------------------------------------ kinematics shared by running / terminal knots
 // fills oM, S, I, v, hb, Ic, hsub, com, ofoot, Jf
@@ -100,24 +124,12 @@ template <class WS> HD void mb_kinematics(const DevModel &m, WS &w) {
     if (m.ancdof_mask[rb.foot_body[f]] >> j & 1) se3_actinv_motion(w.ofoot + 12 * f, w.S + 6 * j, col);
     for (int r = 0; r < 6; r++) w.Jf[(6 * f + r) * NV + j] = col[r];
   }
-  PAR_FOR(e, NB * 10) {
-    int b = e / 10, c = e % 10;
-    uint32_t mask = m.sub_mask[b];
-    double s = 0;
-    for (int d = b; d < NB; d++) if (mask >> d & 1) s += w.I[10 * d + c];
-    w.Ic[e] = s;
-  }
+  mb_subtree_sum<10>(m, w.I, w.Ic);
   SYNC();
   PAR_FOR(b, NB) inertia_mul(w.I + 10 * b, w.v + 6 * b, w.hb + 6 * b);
   PAR_FOR(j, NV) inertia_mul(w.Ic + 10 * body_of_dof(j), w.S + 6 * j, w.U + 6 * j);
   SYNC();
-  PAR_FOR(e, NB * 6) {
-    int b = e / 6, c = e % 6;
-    uint32_t mask = m.sub_mask[b];
-    double s = 0;
-    for (int d = b; d < NB; d++) if (mask >> d & 1) s += w.hb[6 * d + c];
-    w.hsub[e] = s;
-  }
+  mb_subtree_sum<6>(m, w.hb, w.hsub);
   ONE_THREAD { for (int i = 0; i < 3; i++) w.com[i] = w.Ic[1 + i] / w.Ic[0]; }
   SYNC();
 }
@@ -143,6 +155,81 @@ template <class WS> HD void mb_composite_B(const DevModel &m, WS &w) {
     for (int b = NB - 1; b > 0; b--) w.Bc[36 * m.rb.parent[b] + e] += w.Bc[36 * b + e];
   }
   SYNC();
+}
+
+// bias pass: body accelerations with gravity folded in (a0 = [-g; 0] at the root) into w.a and body forces into w.f, for zero
+// joint accelerations or, with JACC, for qdd = [0; qdd_j] (the kinodynamic joint accelerations; the base term comes later)
+template <bool JACC = false, class WS> HD void mb_bias_forces(const DevModel &m, WS &w, const double *a0, const double *qdd_j = nullptr) {
+  PAR_FOR(b, NB) {
+    double acc[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
+    const uint32_t mask = m.anc_mask[b];
+    for (int k = 1; k <= b; k++)
+      if (mask >> k & 1) {
+        double sj[6], c[6];
+        for (int i = 0; i < 6; i++) sj[i] = w.S[6 * (5 + k) + i] * w.x[NQ + 5 + k];
+        cross_mm(w.v + 6 * k, sj, c);
+        if (JACC) for (int i = 0; i < 6; i++) acc[i] += c[i] + w.S[6 * (5 + k) + i] * qdd_j[k - 1];
+        else for (int i = 0; i < 6; i++) acc[i] += c[i];
+      }
+    for (int i = 0; i < 6; i++) w.a[6 * b + i] = acc[i];
+    mb_body_force(w, b, acc, w.f + 6 * b);
+  }
+}
+
+// composite-rigid-body mass matrix M (NV x NV) from S and U = Ic S
+template <class WS> HD void mb_crba(const DevModel &m, const WS &w, double *M) {
+  PAR_FOR(e, NV * NV) {
+    const int i = e / NV, j = e % NV, bi = body_of_dof(i), bj = body_of_dof(j);
+    double v = 0;
+    if (m.anc_mask[bj] >> bi & 1) v = dot6(w.S + 6 * i, w.U + 6 * j);
+    else if (m.anc_mask[bi] >> bj & 1) v = dot6(w.S + 6 * j, w.U + 6 * i);
+    M[e] = v;
+  }
+}
+
+// LOCAL velocity of sole f and, with ACC, its acceleration at zero joint acceleration (dJ v: the bias acceleration w.a minus a0)
+template <bool ACC = true, class WS> HD void mb_sole_motion(const DevModel &m, const WS &w, int f, const double *a0, double *vel, double *dJv = nullptr) {
+  const int fb = m.rb.foot_body[f];
+  se3_actinv_motion(w.ofoot + 12 * f, w.v + 6 * fb, vel);
+  if (ACC) {
+    double an[6];
+    for (int i = 0; i < 6; i++) an[i] = w.a[6 * fb + i] - a0[i];
+    se3_actinv_motion(w.ofoot + 12 * f, an, dJv);
+  }
+}
+
+// centroidal momentum matrix A_g (6 x NV, linear rows first): column j = shift_to_com(U_j)
+template <class WS> HD void mb_centroidal_map(const WS &w, double *Ag) {
+  PAR_FOR(j, NV) {
+    const double *Uj = w.U + 6 * j;
+    double c[3];
+    cross3(w.com, Uj, c);
+    for (int r = 0; r < 3; r++) { Ag[r * NV + j] = Uj[r]; Ag[(3 + r) * NV + j] = Uj[3 + r] - c[r]; }
+  }
+}
+
+// force-derivative column of dof j at body mb of subtree(J), J = body_of_dof(j): g = Ic_mb c_j + Bc_mb w_j (the oracle's
+// total_force_derivatives), kind 0 (d/dq_j): w_j = s_j x v_pJ, c_j = s_j x a_pJ - w_j x v_pJ; kind 1 (d/dv_j): w_j = s_j,
+// c_j = -s_j x (v_J + v_pJ); v_pJ, a_pJ of the parent of J, zero velocity and a0 at the root
+template <class WS> HD void mb_force_column(const DevModel &m, const WS &w, int kind, int j, int mb, const double *a0, double *g) {
+  const int J = body_of_dof(j), pJ = m.rb.parent[J];
+  const double *s = w.S + 6 * j;
+  double vp[6] = {0, 0, 0, 0, 0, 0}, ap[6] = {a0[0], a0[1], a0[2], 0, 0, 0};
+  if (pJ >= 0) for (int i = 0; i < 6; i++) { vp[i] = w.v[6 * pJ + i]; ap[i] = w.a[6 * pJ + i]; }
+  double cj[6], wj[6], t1[6], g2[6];
+  if (kind == 0) {
+    cross_mm(s, vp, wj);
+    cross_mm(s, ap, cj);
+    cross_mm(wj, vp, t1);
+    for (int i = 0; i < 6; i++) cj[i] -= t1[i];
+  } else {
+    for (int i = 0; i < 6; i++) { wj[i] = s[i]; t1[i] = w.v[6 * J + i] + vp[i]; }
+    cross_mm(s, t1, cj);
+    for (int i = 0; i < 6; i++) cj[i] = -cj[i];
+  }
+  inertia_mul(w.Ic + 10 * mb, cj, g);
+  mat6_vec(w.Bc + 36 * mb, wj, g2);
+  for (int i = 0; i < 6; i++) g[i] += g2[i];
 }
 
 // centroidal momentum residual + Jacobian [dh/dq | A_g] (6 x 56), pose residuals + Jacobians, state error and — for running
