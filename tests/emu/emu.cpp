@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 #include <vector>
 
 using namespace mpcdev;
@@ -54,16 +55,29 @@ struct EmuBackend {
   void read_counters(int *c) { for (int i = 0; i < 4; i++) c[i] = w.counters[i]; }
 };
 
-extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, int batch, const mpc_knot_t *knots, const mpc_term_t *terms,
-                         const double *x0, double *xs, double *us, double *K, double *vs, double *lams, mpc_info_t *info, double *stage0,
-                         int max_iters, double *lq_dump /* optional: AB,H,g of instance 0 after the first derivative pass */) {
+static std::string g_err;
+extern "C" const char *emu_last_error() { return g_err.c_str(); }
+
+// robots / cfgs [batch] are nullable, as in mpc_set_instance_models.  If either is given, every instance gets its own DevModel
+// (Ws::model_stride 1), built and checked by build_instance_models like the C-ABI's, a null array standing for rb / cfg.  With both null
+// the batch shares one DevModel (model_stride 0).  A rejected model returns 1 with the message in emu_last_error().
+extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, const mpc_robot_t *robots, const mpc_config_t *cfgs, int batch,
+                         const mpc_knot_t *knots, const mpc_term_t *terms, const double *x0, double *xs, double *us, double *K, double *vs,
+                         double *lams, mpc_info_t *info, double *stage0, int max_iters,
+                         double *lq_dump /* optional: AB,H,g of instance 0 after the first derivative pass */) {
   static_assert(sizeof(FullWsT<true>) <= 40000 * 8 && sizeof(KinoWsT<true>) <= 40000 * 8, "smem");
-  DevModel *model = new DevModel;
+  std::vector<DevModel> shared(1), models;
   const char *err = nullptr;
-  if (build_dev_model(rb, cfg, model, &err)) return 1;
+  if (build_dev_model(rb, cfg, shared.data(), &err)) { g_err = err; return 1; }
+  if (robots || cfgs) {
+    models.resize(batch);
+    g_err = build_instance_models(shared[0], robots, cfgs, batch, models.data());
+    if (!g_err.empty()) return 1;
+  }
   EmuBackend be;
   Ws &w = be.w;
-  init_ws(w, *cfg, batch, model);
+  init_ws(w, *cfg, batch, models.empty() ? shared.data() : models.data());
+  w.model_stride = models.empty() ? 0 : 1;
   std::vector<void *> allocs;
   auto calloc_ = [&](size_t bytes) { void *p = calloc(bytes ? bytes : 8, 1); allocs.push_back(p); return p; };
   alloc_ws(w, calloc_);
@@ -95,7 +109,6 @@ extern "C" int emu_solve(const mpc_robot_t *rb, const mpc_config_t *cfg, int bat
     if (stage0) { std::memcpy(stage0 + b * 68, w.xdot + b * T1 * 56, 8 * 56); std::memcpy(stage0 + b * 68 + 56, w.lamc + b * T1 * 12, 8 * 12); }
   }
   for (void *p : allocs) free(p);
-  delete model;
   return 0;
 }
 

@@ -14,11 +14,16 @@ dp = C.POINTER(C.c_double)
 _lib = None
 
 
+class EmuError(RuntimeError):
+    pass
+
+
 def lib():
     global _lib
     if _lib is None:
         subprocess.check_call(["make", "-C", os.path.join(ROOT, "tests", "emu")], stdout=subprocess.DEVNULL)
         _lib = C.CDLL(_LIB)
+        _lib.emu_last_error.restype = C.c_char_p
     return _lib
 
 
@@ -26,10 +31,15 @@ def _p(a):
     return a.ctypes.data_as(dp) if a is not None else None
 
 
-def solve(prob, max_iters, dump=False, xs=None, us=None, vs=None, lams=None):
+def solve(prob, max_iters, dump=False, xs=None, us=None, vs=None, lams=None, robots=None, cfgs=None):
+    """robots / cfgs: sequences of length batch of _abi.Robot / _abi.Config giving every instance its own model (mpc_set_instance_models),
+    or None for prob's shared robot / config.  A rejected model raises EmuError with the message of the C validation."""
     cfg = prob["cfg"]
     nx, n, m, nc = _abi.DIMS[cfg.kind]
     T, B, nz = cfg.T, prob["x0"].shape[0], n + m
+    for seq in (robots, cfgs):
+        if seq is not None and len(seq) != B:
+            raise EmuError(f"expected {B} per-instance models, got {len(seq)}")
     xs = np.ascontiguousarray(prob["xs"] if xs is None else xs, float).copy()
     us = np.ascontiguousarray(prob["us"] if us is None else us, float).copy()
     K = np.zeros((B, T, m, n))
@@ -38,9 +48,12 @@ def solve(prob, max_iters, dump=False, xs=None, us=None, vs=None, lams=None):
     info = (_abi.Info * B)()
     st = np.zeros((B, 68))
     d = np.zeros(T * n * nz + (T + 1) * nz * nz + (T + 1) * nz + T * n + (T + 1) * nc + (T + 1) * 8) if dump else None
-    rc = lib().emu_solve(C.byref(prob["robot"]), C.byref(cfg), B, prob["knots"], prob["terms"], _p(np.ascontiguousarray(prob["x0"], float)),
+    rbs = None if robots is None else (_abi.Robot * B)(*robots)
+    cfs = None if cfgs is None else (_abi.Config * B)(*cfgs)
+    rc = lib().emu_solve(C.byref(prob["robot"]), C.byref(cfg), rbs, cfs, B, prob["knots"], prob["terms"], _p(np.ascontiguousarray(prob["x0"], float)),
                          _p(xs), _p(us), _p(K), _p(vs), _p(lams), info, _p(st), int(max_iters), _p(d))
-    assert rc == 0
+    if rc != 0:
+        raise EmuError(lib().emu_last_error().decode())
     out = dict(xs=xs, us=us, K=K, vs=vs, lams=lams, info=info, stage0=st)
     if dump:
         o = 0

@@ -1,7 +1,7 @@
 """Per-instance robot parameters and cost constants (mpc_set_instance_models / BatchSolver.set_instance_models).
 
-CPU: the kernel sources under the host emulation (emu_solve_models) with a heterogeneous batch against the oracle run per instance on
-its own (robot_i, cfg_i), and the validation of what must stay uniform.  GPU (`-m gpu`): the device path against the oracle per instance,
+CPU: the kernel sources under the host emulation (emu_solve with per-instance robots / configs) with a heterogeneous batch against the
+oracle run per instance on its own (robot_i, cfg_i), and the validation of the models.  GPU (`-m gpu`): the device path against the oracle per instance,
 bitwise equality with the shared path when every instance carries the shared model, bitwise equality of instance i of a heterogeneous
 batch with instance i of a homogeneous batch of (robot_i, cfg_i), the device gait's sole placements from each robot's own kinematics,
 the rigid-body terms per robot and the error paths."""
@@ -9,7 +9,6 @@ import numpy as np
 import pytest
 
 import emu_lib
-import emu_models_lib
 from mpc_benchmark_b200 import _abi, problems
 
 RTOL = 1e-6
@@ -84,7 +83,7 @@ COLD = [(problems.cent_standing_problem, 30, 0), (problems.full_standing_problem
 def test_emulated_cold_solve_matches_oracle_per_instance(oracle, maker, T, rollout):
     prob = _with_solver_consts(maker(batch=3, T=T), rollout)
     robots, cfgs = hetero_models(prob, 1)
-    e = emu_models_lib.solve_models(prob, robots, cfgs, 100)
+    e = emu_lib.solve(prob, 100, robots=robots, cfgs=cfgs)
     ref = oracle_per_instance(oracle, prob, robots, cfgs, 100)
     _check(e["xs"], e["us"], e["K"], [i.num_iters for i in e["info"]], ref)
     assert [i.conv for i in e["info"]] == [i.conv for i in ref["info"]]
@@ -99,7 +98,7 @@ def test_emulated_walking_batch_matches_oracle_per_instance(oracle, kind, rollou
     prob = _with_solver_consts(problems.walk_batch(kind, 2, seed=2, T=40, ticks=[15, 90], mirror=[False, True]), rollout)
     assert 0.1 < prob["ds_fraction"] < 0.9
     robots, cfgs = hetero_models(prob, 2)
-    e = emu_models_lib.solve_models(prob, robots, cfgs, 4)
+    e = emu_lib.solve(prob, 4, robots=robots, cfgs=cfgs)
     ref = oracle_per_instance(oracle, prob, robots, cfgs, 4)
     _check(e["xs"], e["us"], e["K"], [i.num_iters for i in e["info"]], ref, e["vs"])
     assert [i.ls_evals for i in e["info"]] == [i.ls_evals for i in ref["info"]]
@@ -111,15 +110,15 @@ def test_emulated_identical_copies_equal_the_shared_model():
     prob = problems.walk_batch(_abi.KIND_FULL, 2, seed=3, T=20, ticks=[60, 99], mirror=[False, True])
     B = 2
     a = emu_lib.solve(prob, 3)
-    b = emu_models_lib.solve_models(prob, [prob["robot"]] * B, [prob["cfg"]] * B, 3)
-    c = emu_models_lib.solve_models(prob, None, [prob["cfg"]] * B, 3)
+    b = emu_lib.solve(prob, 3, robots=[prob["robot"]] * B, cfgs=[prob["cfg"]] * B)
+    c = emu_lib.solve(prob, 3, cfgs=[prob["cfg"]] * B)
     for k in ("xs", "us", "K", "vs", "lams"):
         assert np.array_equal(a[k], b[k]) and np.array_equal(a[k], c[k]), k
 
 
 def _rejected(prob, robots, cfgs):
-    with pytest.raises(emu_models_lib.EmuError) as ei:
-        emu_models_lib.solve_models(prob, robots, cfgs, 1)
+    with pytest.raises(emu_lib.EmuError) as ei:
+        emu_lib.solve(prob, 1, robots=robots, cfgs=cfgs)
     return str(ei.value)
 
 
@@ -143,6 +142,14 @@ def test_validation_rejects_a_differing_topology(field):
         robots[2].foot_body[1] = 11
     msg = _rejected(prob, robots, None)
     assert "instance 2" in msg and f"robot.{field}" in msg, msg
+
+
+def test_validation_rejects_an_invalid_shared_model():
+    prob = problems.full_standing_problem(batch=3, T=4)
+    prob["robot"] = _copy(prob["robot"])
+    prob["robot"].parent[5] = 7
+    msg = _rejected(prob, None, None)
+    assert msg == "bodies must be ordered parents-first", msg
 
 
 def test_perturbed_robots_keep_kinematics_and_valid_inertia():
