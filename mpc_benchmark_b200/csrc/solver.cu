@@ -10,6 +10,7 @@
 // There is deliberately NO CPU fallback: every entry point fails if CUDA is unavailable.
 #include "driver.hpp"
 #include "ws_alloc.hpp"
+#include "cuda_owned.hpp"
 #include "rbd_terms.cuh"
 #include "gait_host.hpp"
 #include <cuda_runtime.h>
@@ -194,38 +195,37 @@ __global__ void k_dmma_peak(double *out, int iters) {
 }
 
 // ------------------------------------------------------------------ host side
+// device buffers of the gait generator (mpc_gait_setup / mpc_gait_tick); feet: [2][B][12]
+struct GaitBufs { CudaArray<GaitCfg> cfg; CudaArray<GaitRobot> robots; CudaArray<int8_t> phases; CudaArray<double> urefs, feet; };
+
 struct mpc_solver {
   int device = 0;
+  CudaStream stream, stream_copy; // stream_copy: uploads / downloads of mpc_run_pipelined
+  CudaEvent ev0, ev1, ev_part[2 * 8];
   Ws w{};
-  DevModel *d_model = nullptr;
+  CudaArray<DevModel> d_model;
   DevModel h_model;
   // per-instance models (mpc_set_instance_models): [batch] DevModels, allocated on first use; w.model points here while instance_models
-  DevModel *d_models = nullptr;
+  CudaArray<DevModel> d_models;
   bool instance_models = false;
-  std::vector<void *> allocs;
-  double *d_xs_in = nullptr, *d_us_in = nullptr, *d_meas = nullptr;
-  mpc_knot_t *d_last = nullptr;
-  int32_t *h_counters = nullptr; // pinned
-  cudaStream_t stream = nullptr, stream_copy = nullptr; // stream_copy: uploads / downloads of mpc_run_pipelined
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_part[2 * 8] = {};
-  double *d_k0 = nullptr; // first feedback gains, packed (mpc_run_pipelined)
-  InstState *h_st = nullptr; // pinned copy of the per-instance summaries (mpc_run_pipelined)
+  std::vector<CudaArray<unsigned char>> allocs; // the workspace blocks behind w
+  CudaArray<double> d_xs_in, d_us_in, d_meas;
+  CudaArray<mpc_knot_t> d_last;
+  CudaArray<int32_t, true> h_counters; // pinned
+  CudaArray<double> d_k0; // first feedback gains, packed (mpc_run_pipelined)
+  CudaArray<InstState, true> h_st; // pinned copy of the per-instance summaries (mpc_run_pipelined)
   int num_sms = 148;
   int last_launches = 0;
   float last_ms = 0;
   size_t bytes = 0;
   bool setup_done = false;
   // per-kernel-category device timing of the last run: 0 eval+derivatives, 1 riccati, 2 trial evaluation, 3 bookkeeping
-  std::vector<cudaEvent_t> evpool;
+  std::vector<CudaEvent> evpool;
   std::vector<int> evcat;
   double cat_ms[4] = {0, 0, 0, 0};
   int cat_launches[4] = {0, 0, 0, 0};
   bool profile = true;
-  // device-side gait generator (mpc_gait_setup / mpc_gait_tick)
-  GaitCfg *d_gait = nullptr;
-  GaitRobot *d_gait_robots = nullptr;
-  int8_t *d_gait_phases = nullptr;
-  double *d_gait_urefs = nullptr, *d_feet = nullptr; // d_feet: [2][B][12]
+  GaitBufs gait;
   int gait_t = 0;
   bool gait_ready = false;
   int tail_mode = 0; // warm start of the knot appended by mpc_tick (mpc_set_tail_warmstart)
@@ -233,6 +233,7 @@ struct mpc_solver {
   // first need for lw.L legs
   int lq_legs = 0;
   LegWs lw{};
+  std::vector<CudaArray<unsigned char>> leg_allocs; // the blocks behind lw
   size_t leg_bytes = 0;
 };
 
@@ -243,7 +244,7 @@ struct CudaBackend {
   void mark(int cat) { // event before a launch of category `cat`; the matching end event is the next mark (or run end)
     if (!h->profile) return;
     size_t i = h->evcat.size();
-    if (i >= h->evpool.size()) { cudaEvent_t e; cudaEventCreate(&e); h->evpool.push_back(e); }
+    if (i >= h->evpool.size()) { h->evpool.emplace_back(); h->evpool.back().ensure(cudaEventDefault); }
     cudaEventRecord(h->evpool[i], s);
     h->evcat.push_back(cat);
   }
@@ -288,9 +289,11 @@ struct CudaBackend {
   }
 };
 
-// the SM count (Riccati launch shape) and the dynamic shared memory of the handle's kernels
+// the SM count (Riccati launch shape) and the dynamic shared memory of the handle's kernels, on the handle's device
 static int set_kernel_attrs(mpc_solver *h) {
   { int dev = 0, sms = 0; if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && sms > 0) h->num_sms = sms; }
+  for (const void *k : {(const void *)k_rbd_terms, (const void *)k_ikid_terms, (const void *)k_feet_of_prediction})
+    CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FullWsT<false>)));
   return dispatch_kind(h->w.kind, [&](auto kind) {
     constexpr int KIND = decltype(kind)::value;
     CK(cudaFuncSetAttribute(k_eval<KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EvalShape<KIND, true>::G * EvalShape<KIND, true>::slice)));
@@ -313,7 +316,7 @@ static int zero_multipliers(mpc_solver *h, cudaStream_t s) {
 
 // upload `last` (host, [batch]) and append it to the horizon (k_cycle), on the handle's stream
 static int cycle_knots(mpc_solver *h, const mpc_knot_t *last) {
-  if (!h->d_last) CK(cudaMalloc(&h->d_last, sizeof(mpc_knot_t) * h->w.B)); // owned by the handle, released in mpc_destroy
+  CK(h->d_last.ensure(h->w.B));
   CK(cudaMemcpyAsync(h->d_last, last, sizeof(mpc_knot_t) * h->w.B, cudaMemcpyHostToDevice, h->stream));
   k_cycle<<<h->w.B, 96, 0, h->stream>>>(h->w, h->d_last);
   return 0;
@@ -333,6 +336,24 @@ static int read_run_times(mpc_solver *h) {
   return 0;
 }
 
+// the host-array form of a term entry point: stage the B states x, run launch(dev) (the _device variant on the handle's stream) with
+// dev = the device addresses of x and of each output, copy back every output whose host pointer is not null
+struct TermOut { double *host; size_t per; }; // per: doubles per state
+template <size_t N, class Launch> static int stage_terms(mpc_solver *h, size_t B, const double *x, const TermOut (&outs)[N], Launch &&launch) {
+  size_t per = NQ + NV;
+  for (const TermOut &o : outs) per += o.per;
+  CudaArray<double> d;
+  CK(d.ensure(B * per));
+  uint64_t dev[N + 1] = {(uint64_t)d.get()};
+  for (size_t i = 0; i < N; i++) dev[i + 1] = dev[i] + 8 * B * (i ? outs[i - 1].per : NQ + NV);
+  CK(cudaMemcpyAsync(d, x, 8 * B * (NQ + NV), cudaMemcpyHostToDevice, h->stream));
+  if (launch(dev)) return 1;
+  for (size_t i = 0; i < N; i++)
+    if (outs[i].host) CK(cudaMemcpyAsync(outs[i].host, (const double *)dev[i + 1], 8 * B * outs[i].per, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
 extern "C" {
 
 const char *mpc_last_error(void) { return g_err.c_str(); }
@@ -344,20 +365,41 @@ static const char *check_lq_legs(const mpc_config_t *cfg) {
   if (cfg->lq_legs > cfg->T) return "lq_legs must not exceed the horizon T";
   return nullptr;
 }
+// allocator of alloc_ws / alloc_leg_ws: a block of `bytes` owned by `blocks`; `ok` turns false at the first failure
+static void *alloc_block(std::vector<CudaArray<unsigned char>> &blocks, size_t bytes, bool &ok) {
+  blocks.emplace_back();
+  ok = ok && blocks.back().ensure(bytes ? bytes : 8) == cudaSuccess;
+  return blocks.back();
+}
 // the per-(instance, leg) blocks of the time-parallel LQ solve for the handle's lq_legs (allocated before the first run that needs them)
 static int ensure_leg_ws(mpc_solver *h) {
   if (h->lq_legs < 2 || h->lw.L == h->lq_legs) return 0;
-  free_leg_ws(h->lw, [](void *p) { cudaFree(p); });
-  h->leg_bytes = 0;
+  h->leg_allocs.clear();
   bool ok = true;
-  const size_t bytes = alloc_leg_ws(h->w, h->lw, h->lq_legs, [&](size_t b) -> void * {
-    void *p = nullptr;
-    if (!ok || cudaMalloc(&p, b ? b : 8) != cudaSuccess) { ok = false; return nullptr; }
-    return p;
-  });
-  if (!ok) { free_leg_ws(h->lw, [](void *p) { cudaFree(p); }); return fail("cudaMalloc(lq_legs workspace) failed: batch x lq_legs too large for this GPU"); }
+  const size_t bytes = alloc_leg_ws(h->w, h->lw, h->lq_legs, [&](size_t b) { return alloc_block(h->leg_allocs, b, ok); });
+  if (!ok) { h->leg_allocs.clear(); h->lw = LegWs{}; h->leg_bytes = 0; return fail("cudaMalloc(lq_legs workspace) failed: batch x lq_legs too large for this GPU"); }
   h->leg_bytes = bytes;
   return 0;
+}
+
+// preamble of every entry point with a handle: a null handle fails before any CUDA call, then the device, then (needs_setup) call order
+static int enter(const mpc_solver *h, const char *fn, bool needs_setup) {
+  if (!h) return fail(std::string(fn) + ": null handle");
+  CK(cudaSetDevice(h->device));
+  if (needs_setup && !h->setup_done) return fail(std::string(fn) + " before mpc_setup");
+  return 0;
+}
+
+// the handle's stream, events, model and kernel attributes on its (current) device
+static int init_handle(mpc_solver *h, const mpc_config_t &cfg, int batch) {
+  CK(h->stream.ensure(cudaStreamNonBlocking));
+  CK(h->ev0.ensure(cudaEventDefault)); CK(h->ev1.ensure(cudaEventDefault));
+  CK(h->h_counters.ensure(4));
+  CK(h->d_model.ensure(1));
+  CK(cudaMemcpyAsync(h->d_model, &h->h_model, sizeof(DevModel), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  init_ws(h->w, cfg, batch, h->d_model);
+  return set_kernel_attrs(h);
 }
 
 mpc_solver_t *mpc_create(const mpc_robot_t *robot, const mpc_config_t *cfg, int32_t batch, int32_t device) {
@@ -368,66 +410,37 @@ mpc_solver_t *mpc_create(const mpc_robot_t *robot, const mpc_config_t *cfg, int3
   if (batch <= 0 || cfg->T <= 0) { g_err = "mpc_create: batch and horizon must be positive"; return nullptr; }
   if (const char *le = check_lq_legs(cfg)) { g_err = std::string("mpc_create: ") + le; return nullptr; }
   if (cudaSetDevice(device) != cudaSuccess) { g_err = "cudaSetDevice failed"; return nullptr; }
-  mpc_solver *h = new mpc_solver;
+  std::unique_ptr<mpc_solver> h(new mpc_solver); // a failure below releases what was created so far
   h->device = device;
   h->lq_legs = cfg->lq_legs;
   const char *err = nullptr;
-  if (build_dev_model(robot, cfg, &h->h_model, &err)) { g_err = err; delete h; return nullptr; }
-  // every failure below releases what was created so far through mpc_destroy (all members start null)
-  auto bail = [&](const char *what, cudaError_t e) -> mpc_solver_t * { g_err = std::string(what) + ": " + cudaGetErrorString(e); mpc_destroy(h); return nullptr; };
-  cudaError_t e;
-  if ((e = cudaMalloc(&h->d_model, sizeof(DevModel))) != cudaSuccess) return bail("cudaMalloc(model)", e);
-  if ((e = cudaMemcpy(h->d_model, &h->h_model, sizeof(DevModel), cudaMemcpyHostToDevice)) != cudaSuccess) return bail("cudaMemcpy(model)", e);
-  init_ws(h->w, *cfg, batch, h->d_model);
-  if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
-  if ((e = cudaEventCreate(&h->ev0)) != cudaSuccess || (e = cudaEventCreate(&h->ev1)) != cudaSuccess) return bail("cudaEventCreate", e);
-  if ((e = cudaMallocHost(&h->h_counters, 4 * sizeof(int32_t))) != cudaSuccess) return bail("cudaMallocHost", e);
-  if (set_kernel_attrs(h)) { std::string keep = g_err; mpc_destroy(h); g_err = keep; return nullptr; }
-  return h;
+  if (build_dev_model(robot, cfg, &h->h_model, &err)) { g_err = err; return nullptr; }
+  if (init_handle(h.get(), *cfg, batch)) return nullptr;
+  return h.release();
 }
 
 void mpc_destroy(mpc_solver_t *h) {
   if (!h) return;
   cudaSetDevice(h->device);
-  if (h->stream) cudaStreamSynchronize(h->stream);
-  for (void *p : h->allocs) cudaFree(p);
-  free_leg_ws(h->lw, [](void *p) { cudaFree(p); });
-  for (cudaEvent_t e : h->evpool) cudaEventDestroy(e);
-  if (h->d_xs_in) cudaFree(h->d_xs_in);
-  if (h->d_us_in) cudaFree(h->d_us_in);
-  if (h->d_meas) cudaFree(h->d_meas);
-  if (h->d_last) cudaFree(h->d_last);
-  if (h->d_model) cudaFree(h->d_model);
-  if (h->d_models) cudaFree(h->d_models);
-  if (h->h_counters) cudaFreeHost(h->h_counters);
-  if (h->h_st) cudaFreeHost(h->h_st);
-  if (h->d_k0) cudaFree(h->d_k0);
-  cudaFree(h->d_gait); cudaFree(h->d_gait_robots); cudaFree(h->d_gait_phases); cudaFree(h->d_gait_urefs); cudaFree(h->d_feet);
-  for (cudaEvent_t e : h->ev_part) if (e) cudaEventDestroy(e);
-  if (h->stream_copy) cudaStreamDestroy(h->stream_copy);
-  if (h->ev0) cudaEventDestroy(h->ev0);
-  if (h->ev1) cudaEventDestroy(h->ev1);
-  if (h->stream) cudaStreamDestroy(h->stream);
+  cudaStreamSynchronize(h->stream);
   delete h;
 }
 
 int32_t mpc_setup(mpc_solver_t *h, const mpc_knot_t *knots, const mpc_term_t *terms, const double *x0) {
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_setup", false)) return 1;
   Ws &w = h->w;
-  const size_t T1 = w.T + 1;
   if (!h->setup_done) {
     bool ok = true;
-    h->bytes = alloc_ws(w, [&](size_t bytes) -> void * {
-      void *p = nullptr;
-      if (!ok) return nullptr;
-      if (cudaMalloc(&p, bytes ? bytes : 8) != cudaSuccess) { ok = false; return nullptr; }
-      cudaMemsetAsync(p, 0, bytes ? bytes : 8, h->stream);
-      h->allocs.push_back(p);
+    h->allocs.clear(); // the blocks of an earlier attempt that failed
+    h->bytes = alloc_ws(w, [&](size_t bytes) {
+      void *p = alloc_block(h->allocs, bytes, ok);
+      if (p) cudaMemsetAsync(p, 0, bytes ? bytes : 8, h->stream);
       return p;
     });
     if (!ok) return fail("cudaMalloc(workspace) failed: batch too large for this GPU");
-    CK(cudaMalloc(&h->d_xs_in, w.B * T1 * w.nx * 8));
-    CK(cudaMalloc(&h->d_us_in, (size_t)w.B * w.T * w.m * 8));
+    const TrajSizes t = traj_sizes(w);
+    CK(h->d_xs_in.ensure(w.B * t.xs));
+    CK(h->d_us_in.ensure(w.B * t.us));
     h->setup_done = true;
   } else {
     // solver.setup() re-creates the workspace: multipliers restart from zero (fulldynamic_talos.py:539)
@@ -441,9 +454,8 @@ int32_t mpc_setup(mpc_solver_t *h, const mpc_knot_t *knots, const mpc_term_t *te
 }
 
 int32_t mpc_update_knots(mpc_solver_t *h, const mpc_knot_t *knots, int32_t first, int32_t count) {
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_update_knots", true)) return 1;
   Ws &w = h->w;
-  if (!h->setup_done) return fail("mpc_update_knots before mpc_setup");
   if (first < 0 || count < 0 || first + count > w.T) return fail("knot range out of bounds");
   // host layout [batch][count]
   CK(cudaMemcpy2DAsync(w.knots + first, sizeof(mpc_knot_t) * w.T, knots, sizeof(mpc_knot_t) * count, sizeof(mpc_knot_t) * count, w.B,
@@ -453,16 +465,14 @@ int32_t mpc_update_knots(mpc_solver_t *h, const mpc_knot_t *knots, int32_t first
 }
 
 int32_t mpc_update_terms(mpc_solver_t *h, const mpc_term_t *terms) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_update_terms before mpc_setup");
+  if (enter(h, "mpc_update_terms", true)) return 1;
   CK(cudaMemcpyAsync(h->w.terms, terms, sizeof(mpc_term_t) * h->w.B, cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
 int32_t mpc_cycle(mpc_solver_t *h, const mpc_knot_t *last) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_cycle before mpc_setup");
+  if (enter(h, "mpc_cycle", true)) return 1;
   if (cycle_knots(h, last)) return 1;
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
@@ -487,8 +497,7 @@ __global__ void k_shift_multipliers(Ws w, int n) {
 }
 
 int32_t mpc_shift_multipliers(mpc_solver_t *h, int32_t n) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_shift_multipliers before mpc_setup");
+  if (enter(h, "mpc_shift_multipliers", true)) return 1;
   if (n <= 0) return 0;
   k_shift_multipliers<<<h->w.B, 128, 0, h->stream>>>(h->w, n);
   CK(cudaGetLastError());
@@ -498,7 +507,7 @@ int32_t mpc_shift_multipliers(mpc_solver_t *h, int32_t n) {
 
 // swap in new model / weight constants without touching the workspace (same kind, horizon and batch)
 int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_config_t *cfg) {
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_reconfigure", false)) return 1;
   if (h->instance_models) return fail("mpc_reconfigure: per-instance models are set; clear them first with mpc_set_instance_models(h, NULL, NULL)");
   if (cfg->kind != h->w.kind || cfg->T != h->w.T) return fail("mpc_reconfigure: kind / horizon must not change");
   if (const char *le = check_lq_legs(cfg)) return fail(std::string("mpc_reconfigure: ") + le);
@@ -513,8 +522,7 @@ int32_t mpc_reconfigure(mpc_solver_t *h, const mpc_robot_t *robot, const mpc_con
 
 // one DevModel per instance (robots / cfgs [batch], NULL = the handle's shared robot / config), or back to the shared model (both NULL)
 int32_t mpc_set_instance_models(mpc_solver_t *h, const mpc_robot_t *robots, const mpc_config_t *cfgs) {
-  if (!h) return fail("null handle");
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_set_instance_models", false)) return 1;
   Ws &w = h->w;
   if (!robots && !cfgs) {
     CK(cudaStreamSynchronize(h->stream)); // no kernel of the handle still reads the per-instance models
@@ -525,10 +533,7 @@ int32_t mpc_set_instance_models(mpc_solver_t *h, const mpc_robot_t *robots, cons
   std::vector<DevModel> models(w.B);
   const std::string err = build_instance_models(h->h_model, robots, cfgs, w.B, models.data());
   if (!err.empty()) return fail(err);
-  if (!h->d_models && cudaMalloc(&h->d_models, sizeof(DevModel) * (size_t)w.B) != cudaSuccess) {
-    h->d_models = nullptr;
-    return fail("cudaMalloc(per-instance models) failed");
-  }
+  if (h->d_models.ensure(w.B) != cudaSuccess) return fail("cudaMalloc(per-instance models) failed");
   CK(cudaMemcpyAsync(h->d_models, models.data(), sizeof(DevModel) * (size_t)w.B, cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   w.model = h->d_models; w.model_stride = 1;
@@ -537,30 +542,42 @@ int32_t mpc_set_instance_models(mpc_solver_t *h, const mpc_robot_t *robots, cons
 }
 
 int32_t mpc_set_x0(mpc_solver_t *h, const double *x0) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_set_x0 before mpc_setup");
+  if (enter(h, "mpc_set_x0", true)) return 1;
   CK(cudaMemcpyAsync(h->w.x0, x0, 8 * (size_t)h->w.B * h->w.nx, cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
-static int run_impl(mpc_solver *h, const double *d_xs, const double *d_us, int max_iters, cudaStream_t s, bool sync_events) {
-  if (!h->setup_done) return fail("mpc_run before mpc_setup");
+// solve the instances [first, first + count) on be's stream from the warm start d_xs / d_us ([batch] layouts): the k_init prologue
+// and the iterations between two category marks; adds the kernel launches to `launches`
+static int solve_instances(mpc_solver *h, CudaBackend &be, const double *d_xs, const double *d_us, int max_iters, int first, int count, int &launches) {
+  be.mark(3);
+  k_init<<<count, 128, 0, be.s>>>(h->w, d_xs, d_us, max_iters, first);
+  launches += 1 + run_loop(be, h->w, max_iters, h->w.sc, first, count);
+  be.mark(-1);
+  if (be.err != cudaSuccess) return fail(std::string("kernel failure: ") + cudaGetErrorString(be.err));
+  return 0;
+}
+
+// the whole batch on s, then the device times of the run
+static int run_impl(mpc_solver *h, const double *d_xs, const double *d_us, int max_iters, cudaStream_t s) {
   if (ensure_leg_ws(h)) return 1;
   CK(cudaEventRecord(h->ev0, s));
   h->evcat.clear();
   CudaBackend be{h, s};
-  be.mark(3);
-  k_init<<<h->w.B, 128, 0, s>>>(h->w, d_xs, d_us, max_iters, 0);
-  h->last_launches = 1 + run_loop(be, h->w, max_iters, h->w.sc);
-  be.mark(-1);
+  h->last_launches = 0;
+  if (solve_instances(h, be, d_xs, d_us, max_iters, 0, h->w.B, h->last_launches)) return 1;
   CK(cudaEventRecord(h->ev1, s));
-  if (be.err != cudaSuccess) return fail(std::string("kernel failure: ") + cudaGetErrorString(be.err));
   CK(cudaGetLastError());
-  if (sync_events) {
-    CK(cudaEventSynchronize(h->ev1));
-    return read_run_times(h);
-  }
+  CK(cudaEventSynchronize(h->ev1));
+  return read_run_times(h);
+}
+
+// the warm start of the instances [first, first + count) from host xs / us ([batch] layouts) into d_xs_in / d_us_in, on s
+static int upload_warm_start(mpc_solver *h, const double *xs, const double *us, size_t first, size_t count, cudaStream_t s) {
+  const TrajSizes t = traj_sizes(h->w);
+  CK(cudaMemcpyAsync(h->d_xs_in + first * t.xs, xs + first * t.xs, 8 * count * t.xs, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(h->d_us_in + first * t.us, us + first * t.us, 8 * count * t.us, cudaMemcpyHostToDevice, s));
   return 0;
 }
 
@@ -595,44 +612,35 @@ __global__ void k_shift_warmstart(Ws w, double *xs_in, double *us_in, const doub
 // rotate the horizon (append `last`), shift the warm start, take x0 from x_meas (host [batch][nx]) or from the model
 // prediction, reset (setup-per-tick, full/cent) or shift (cycleProblem, kino) the multipliers, run max_iters iterations.
 int32_t mpc_tick(mpc_solver_t *h, const mpc_knot_t *last, const double *x_meas, int32_t keep_multipliers, int32_t max_iters) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_tick before mpc_setup");
+  if (enter(h, "mpc_tick", true)) return 1;
   Ws &w = h->w;
   if (last && cycle_knots(h, last)) return 1;
-  double *d_meas = nullptr;
   if (x_meas) {
-    if (!h->d_meas) CK(cudaMalloc(&h->d_meas, (size_t)w.B * w.nx * 8));
+    CK(h->d_meas.ensure((size_t)w.B * w.nx));
     CK(cudaMemcpyAsync(h->d_meas, x_meas, (size_t)w.B * w.nx * 8, cudaMemcpyHostToDevice, h->stream));
-    d_meas = h->d_meas;
   }
-  k_shift_warmstart<<<w.B, 128, 0, h->stream>>>(w, h->d_xs_in, h->d_us_in, d_meas, h->tail_mode);
+  k_shift_warmstart<<<w.B, 128, 0, h->stream>>>(w, h->d_xs_in, h->d_us_in, x_meas ? h->d_meas.get() : nullptr, h->tail_mode);
   if (keep_multipliers) k_shift_multipliers<<<w.B, 128, 0, h->stream>>>(w, 1);
   else if (zero_multipliers(h, h->stream)) return 1;
   CK(cudaGetLastError());
-  return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream, true);
+  return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream);
 }
 
 int32_t mpc_set_tail_warmstart(mpc_solver_t *h, int32_t mode) {
-  if (!h) return fail("null handle");
+  if (enter(h, "mpc_set_tail_warmstart", false)) return 1;
   if (mode != 0 && mode != 1) return fail("mpc_set_tail_warmstart: mode must be 0 (previous knot) or 1 (nearest knot of the same contact phase)");
   h->tail_mode = mode;
   return 0;
 }
 
 int32_t mpc_reset_multipliers(mpc_solver_t *h, uint64_t stream) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_reset_multipliers before mpc_setup");
+  if (enter(h, "mpc_reset_multipliers", true)) return 1;
   return zero_multipliers(h, stream ? reinterpret_cast<cudaStream_t>(stream) : h->stream);
 }
 
 int32_t mpc_run(mpc_solver_t *h, const double *xs_init, const double *us_init, int32_t max_iters) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_run before mpc_setup");
-  Ws &w = h->w;
-  const size_t T1 = w.T + 1;
-  CK(cudaMemcpyAsync(h->d_xs_in, xs_init, w.B * T1 * w.nx * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaMemcpyAsync(h->d_us_in, us_init, (size_t)w.B * w.T * w.m * 8, cudaMemcpyHostToDevice, h->stream));
-  return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream, true);
+  if (enter(h, "mpc_run", true) || upload_warm_start(h, xs_init, us_init, 0, h->w.B, h->stream)) return 1;
+  return run_impl(h, h->d_xs_in, h->d_us_in, max_iters, h->stream);
 }
 
 // pack what the MPC loop consumes (fulldynamic_talos.py:548-550) of the instances [first, first + gridDim.x): the first feedback
@@ -649,25 +657,22 @@ __global__ void k_pack_k0_info(Ws w, double *K0, double *info, int first) {
 
 int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *us_init, int32_t max_iters, int32_t parts, double *xs_out,
                           double *us_out, double *K0_out, mpc_info_t *info_out) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_run_pipelined before mpc_setup");
-  if (ensure_leg_ws(h)) return 1;
+  if (enter(h, "mpc_run_pipelined", true) || ensure_leg_ws(h)) return 1;
   Ws &w = h->w;
-  const size_t T1 = w.T + 1, sx = T1 * w.nx, su = (size_t)w.T * w.m, sk = (size_t)w.m * w.n;
+  const TrajSizes t = traj_sizes(w);
+  const size_t sk = (size_t)w.m * w.n;
   if (parts < 1) parts = 1;
   if (parts > 8) parts = 8;
   if (parts > w.B) parts = w.B;
-  if (!h->stream_copy) CK(cudaStreamCreateWithFlags(&h->stream_copy, cudaStreamNonBlocking));
-  for (int i = 0; i < 2 * parts; i++) if (!h->ev_part[i]) CK(cudaEventCreateWithFlags(&h->ev_part[i], cudaEventDisableTiming));
-  if (K0_out && !h->d_k0) CK(cudaMalloc(&h->d_k0, (size_t)w.B * sk * 8));
-  if (info_out && !h->h_st) CK(cudaMallocHost(&h->h_st, sizeof(InstState) * w.B));
+  CK(h->stream_copy.ensure(cudaStreamNonBlocking));
+  for (int i = 0; i < 2 * parts; i++) CK(h->ev_part[i].ensure(cudaEventDisableTiming));
+  if (K0_out) CK(h->d_k0.ensure((size_t)w.B * sk));
+  if (info_out) CK(h->h_st.ensure(w.B));
   cudaStream_t s = h->stream, sc = h->stream_copy;
   auto lo = [&](int p) { return (int)((long long)w.B * p / parts); };
   // every upload is queued at once on the copy stream; the solve of part p waits for its own
   for (int p = 0; p < parts; p++) {
-    const size_t o = lo(p), n = lo(p + 1) - lo(p);
-    CK(cudaMemcpyAsync(h->d_xs_in + o * sx, xs_init + o * sx, n * sx * 8, cudaMemcpyHostToDevice, sc));
-    CK(cudaMemcpyAsync(h->d_us_in + o * su, us_init + o * su, n * su * 8, cudaMemcpyHostToDevice, sc));
+    if (upload_warm_start(h, xs_init, us_init, lo(p), lo(p + 1) - lo(p), sc)) return 1;
     CK(cudaEventRecord(h->ev_part[p], sc));
   }
   CK(cudaEventRecord(h->ev0, s));
@@ -677,16 +682,13 @@ int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *
   for (int p = 0; p < parts; p++) {
     const int o = lo(p), n = lo(p + 1) - o;
     CK(cudaStreamWaitEvent(s, h->ev_part[p], 0));
-    be.mark(3);
-    k_init<<<n, 128, 0, s>>>(w, h->d_xs_in, h->d_us_in, max_iters, o);
-    launches += 1 + run_loop(be, w, max_iters, w.sc, o, n); // returns with the part finished (its last counter read synchronises)
-    be.mark(-1);
-    if (be.err != cudaSuccess) return fail(std::string("kernel failure: ") + cudaGetErrorString(be.err));
+    // returns with the part finished (its last counter read synchronises)
+    if (solve_instances(h, be, h->d_xs_in, h->d_us_in, max_iters, o, n, launches)) return 1;
     // the download of this part overlaps the solve of the next one
     CK(cudaEventRecord(h->ev_part[parts + p], s));
     CK(cudaStreamWaitEvent(sc, h->ev_part[parts + p], 0));
-    if (xs_out) CK(cudaMemcpyAsync(xs_out + (size_t)o * sx, w.xs + (size_t)o * sx, (size_t)n * sx * 8, cudaMemcpyDeviceToHost, sc));
-    if (us_out) CK(cudaMemcpyAsync(us_out + (size_t)o * su, w.us + (size_t)o * su, (size_t)n * su * 8, cudaMemcpyDeviceToHost, sc));
+    if (xs_out) CK(cudaMemcpyAsync(xs_out + o * t.xs, w.xs + o * t.xs, n * t.xs * 8, cudaMemcpyDeviceToHost, sc));
+    if (us_out) CK(cudaMemcpyAsync(us_out + o * t.us, w.us + o * t.us, n * t.us * 8, cudaMemcpyDeviceToHost, sc));
     if (K0_out) {
       k_pack_k0_info<<<n, 128, 0, sc>>>(w, h->d_k0, nullptr, o);
       CK(cudaMemcpyAsync(K0_out + (size_t)o * sk, h->d_k0 + (size_t)o * sk, (size_t)n * sk * 8, cudaMemcpyDeviceToHost, sc));
@@ -705,22 +707,21 @@ int32_t mpc_run_pipelined(mpc_solver_t *h, const double *xs_init, const double *
 }
 
 int32_t mpc_run_device(mpc_solver_t *h, uint64_t xs_dev, uint64_t us_dev, int32_t max_iters, uint64_t stream) {
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_run_device", true)) return 1;
   cudaStream_t s = stream ? reinterpret_cast<cudaStream_t>(stream) : h->stream;
-  return run_impl(h, reinterpret_cast<const double *>(xs_dev), reinterpret_cast<const double *>(us_dev), max_iters, s, true);
+  return run_impl(h, reinterpret_cast<const double *>(xs_dev), reinterpret_cast<const double *>(us_dev), max_iters, s);
 }
 
 int32_t mpc_get_results(mpc_solver_t *h, double *xs, double *us, double *K, double *vs, double *lams, mpc_info_t *info) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_get_results before mpc_setup");
+  if (enter(h, "mpc_get_results", true)) return 1;
   Ws &w = h->w;
-  const size_t T1 = w.T + 1;
+  const TrajSizes t = traj_sizes(w);
   cudaStream_t s = h->stream;
-  if (xs) CK(cudaMemcpyAsync(xs, w.xs, w.B * T1 * w.nx * 8, cudaMemcpyDeviceToHost, s));
-  if (us) CK(cudaMemcpyAsync(us, w.us, (size_t)w.B * w.T * w.m * 8, cudaMemcpyDeviceToHost, s));
-  if (K) CK(cudaMemcpyAsync(K, w.Kfb, (size_t)w.B * w.T * w.m * w.n * 8, cudaMemcpyDeviceToHost, s));
-  if (vs) CK(cudaMemcpyAsync(vs, w.vs, w.B * T1 * w.nc * 8, cudaMemcpyDeviceToHost, s));
-  if (lams) CK(cudaMemcpyAsync(lams, w.lams, w.B * T1 * w.n * 8, cudaMemcpyDeviceToHost, s));
+  if (xs) CK(cudaMemcpyAsync(xs, w.xs, w.B * t.xs * 8, cudaMemcpyDeviceToHost, s));
+  if (us) CK(cudaMemcpyAsync(us, w.us, w.B * t.us * 8, cudaMemcpyDeviceToHost, s));
+  if (K) CK(cudaMemcpyAsync(K, w.Kfb, w.B * t.K * 8, cudaMemcpyDeviceToHost, s));
+  if (vs) CK(cudaMemcpyAsync(vs, w.vs, w.B * t.vs * 8, cudaMemcpyDeviceToHost, s));
+  if (lams) CK(cudaMemcpyAsync(lams, w.lams, w.B * t.lams * 8, cudaMemcpyDeviceToHost, s));
   std::vector<InstState> st;
   if (info) { st.resize(w.B); CK(cudaMemcpyAsync(st.data(), w.st, sizeof(InstState) * w.B, cudaMemcpyDeviceToHost, s)); }
   CK(cudaStreamSynchronize(s));
@@ -730,7 +731,7 @@ int32_t mpc_get_results(mpc_solver_t *h, double *xs, double *us, double *K, doub
 }
 
 int32_t mpc_result_ptrs(mpc_solver_t *h, uint64_t *xs, uint64_t *us, uint64_t *K, uint64_t *info) {
-  if (!h->setup_done) return fail("mpc_result_ptrs before mpc_setup");
+  if (enter(h, "mpc_result_ptrs", true)) return 1;
   if (xs) *xs = (uint64_t)h->w.xs;
   if (us) *us = (uint64_t)h->w.us;
   if (K) *K = (uint64_t)h->w.Kfb;
@@ -740,12 +741,12 @@ int32_t mpc_result_ptrs(mpc_solver_t *h, uint64_t *xs, uint64_t *us, uint64_t *K
 
 // xs, us, K0 and the per-instance summary into device buffers, e.g. for a gather over NVLink
 int32_t mpc_export_results_device(mpc_solver_t *h, uint64_t xs_dev, uint64_t us_dev, uint64_t K0_dev, uint64_t info_dev, uint64_t stream) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_export_results_device before mpc_setup");
+  if (enter(h, "mpc_export_results_device", true)) return 1;
   Ws &w = h->w;
+  const TrajSizes t = traj_sizes(w);
   cudaStream_t s = stream ? reinterpret_cast<cudaStream_t>(stream) : h->stream;
-  if (xs_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(xs_dev), w.xs, (size_t)w.B * (w.T + 1) * w.nx * 8, cudaMemcpyDeviceToDevice, s));
-  if (us_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(us_dev), w.us, (size_t)w.B * w.T * w.m * 8, cudaMemcpyDeviceToDevice, s));
+  if (xs_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(xs_dev), w.xs, w.B * t.xs * 8, cudaMemcpyDeviceToDevice, s));
+  if (us_dev) CK(cudaMemcpyAsync(reinterpret_cast<void *>(us_dev), w.us, w.B * t.us * 8, cudaMemcpyDeviceToDevice, s));
   if (K0_dev || info_dev) {
     k_pack_k0_info<<<w.B, 128, 0, s>>>(w, reinterpret_cast<double *>(K0_dev), reinterpret_cast<double *>(info_dev), 0);
     CK(cudaGetLastError());
@@ -754,24 +755,24 @@ int32_t mpc_export_results_device(mpc_solver_t *h, uint64_t xs_dev, uint64_t us_
 }
 
 int32_t mpc_get_stage_data(mpc_solver_t *h, int32_t k, double *xdot, double *contact_force) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_get_stage_data before mpc_setup");
+  if (enter(h, "mpc_get_stage_data", true)) return 1;
   Ws &w = h->w;
   if (k < 0 || k >= w.T) return fail("stage index out of range");
   const size_t T1 = w.T + 1;
-  if (xdot) CK(cudaMemcpy2D(xdot, w.n * 8, w.xdot + (size_t)k * 56, T1 * 56 * 8, w.n * 8, w.B, cudaMemcpyDeviceToHost));
-  if (contact_force) CK(cudaMemcpy2D(contact_force, 12 * 8, w.lamc + (size_t)k * 12, T1 * 12 * 8, 12 * 8, w.B, cudaMemcpyDeviceToHost));
+  if (xdot) CK(cudaMemcpy2DAsync(xdot, w.n * 8, w.xdot + (size_t)k * 56, T1 * 56 * 8, w.n * 8, w.B, cudaMemcpyDeviceToHost, h->stream));
+  if (contact_force) CK(cudaMemcpy2DAsync(contact_force, 12 * 8, w.lamc + (size_t)k * 12, T1 * 12 * 8, 12 * 8, w.B, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
-int32_t mpc_last_launches(mpc_solver_t *h) { return h->last_launches; }
-double mpc_last_kernel_ms(mpc_solver_t *h, int32_t category) { return (category >= 0 && category < 4) ? h->cat_ms[category] : -1.0; }
-int32_t mpc_last_kernel_launches(mpc_solver_t *h, int32_t category) { return (category >= 0 && category < 4) ? h->cat_launches[category] : -1; }
-void mpc_set_profiling(mpc_solver_t *h, int32_t on) { h->profile = on != 0; }
+// getters without a status: a null handle gives the out-of-range value
+int32_t mpc_last_launches(mpc_solver_t *h) { return enter(h, "mpc_last_launches", false) ? -1 : h->last_launches; }
+double mpc_last_kernel_ms(mpc_solver_t *h, int32_t category) { return (enter(h, "mpc_last_kernel_ms", false) || category < 0 || category >= 4) ? -1.0 : h->cat_ms[category]; }
+int32_t mpc_last_kernel_launches(mpc_solver_t *h, int32_t category) { return (enter(h, "mpc_last_kernel_launches", false) || category < 0 || category >= 4) ? -1 : h->cat_launches[category]; }
+void mpc_set_profiling(mpc_solver_t *h, int32_t on) { if (!enter(h, "mpc_set_profiling", false)) h->profile = on != 0; }
 
 int32_t mpc_get_feedback(mpc_solver_t *h, int32_t k, double *K) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_get_feedback before mpc_setup");
+  if (enter(h, "mpc_get_feedback", true)) return 1;
   Ws &w = h->w;
   if (k < 0 || k >= w.T) return fail("stage index out of range");
   const size_t sz = (size_t)w.m * w.n * 8;
@@ -779,25 +780,23 @@ int32_t mpc_get_feedback(mpc_solver_t *h, int32_t k, double *K) {
   CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
-double mpc_last_device_ms(mpc_solver_t *h) { return h->last_ms; }
-uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return h->bytes + h->leg_bytes + (h->d_models ? sizeof(DevModel) * (size_t)h->w.B : 0); }
+double mpc_last_device_ms(mpc_solver_t *h) { return enter(h, "mpc_last_device_ms", false) ? -1.0 : h->last_ms; }
+uint64_t mpc_workspace_bytes(mpc_solver_t *h) { return enter(h, "mpc_workspace_bytes", false) ? 0 : h->bytes + h->leg_bytes + (h->d_models ? sizeof(DevModel) * (size_t)h->w.B : 0); }
 // per-phase cycle counters of the Riccati kernel for instance 0 (all zero unless built with -DMPC_PHASE_TIMING)
 int32_t mpc_debug_phases(mpc_solver_t *h, double *out64) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_debug_phases before mpc_setup");
-  CK(cudaMemcpy(out64, h->w.phase, 64 * 8, cudaMemcpyDeviceToHost)); // [0:16)+[48:64) Riccati, [16:32) derivative eval, [32:48) values eval
+  if (enter(h, "mpc_debug_phases", true)) return 1;
+  CK(cudaMemcpyAsync(out64, h->w.phase, 64 * 8, cudaMemcpyDeviceToHost, h->stream)); // [0:16)+[48:64) Riccati, [16:32) derivative eval, [32:48) values eval
+  CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
 int32_t mpc_debug_lq(mpc_solver_t *h, const double *xs, const double *us, int32_t inst, double *AB, double *H, double *g, double *gap,
                      double *hval, double *scal) {
-  CK(cudaSetDevice(h->device));
-  if (!h->setup_done) return fail("mpc_debug_lq before mpc_setup");
+  if (enter(h, "mpc_debug_lq", true)) return 1;
   Ws &w = h->w;
   const size_t T1 = w.T + 1, T = w.T;
   if (inst < 0 || inst >= w.B) return fail("instance out of range");
-  CK(cudaMemcpyAsync(h->d_xs_in, xs, w.B * T1 * w.nx * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaMemcpyAsync(h->d_us_in, us, (size_t)w.B * w.T * w.m * 8, cudaMemcpyHostToDevice, h->stream));
+  if (upload_warm_start(h, xs, us, 0, w.B, h->stream)) return 1;
   k_init<<<w.B, 128, 0, h->stream>>>(w, h->d_xs_in, h->d_us_in, 1, 0);
   CudaBackend be{h, h->stream};
   be.reset_counters();
@@ -805,12 +804,13 @@ int32_t mpc_debug_lq(mpc_solver_t *h, const double *xs, const double *us, int32_
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   const size_t b = inst;
-  if (AB) CK(cudaMemcpy(AB, w.AB + b * T * w.n * w.nz, T * w.n * w.nz * 8, cudaMemcpyDeviceToHost));
-  if (H) CK(cudaMemcpy(H, w.H + b * T1 * w.nz * w.nz, T1 * w.nz * w.nz * 8, cudaMemcpyDeviceToHost));
-  if (g) CK(cudaMemcpy(g, w.g + b * T1 * w.nz, T1 * w.nz * 8, cudaMemcpyDeviceToHost));
-  if (gap) CK(cudaMemcpy(gap, w.gap + b * T * w.n, T * w.n * 8, cudaMemcpyDeviceToHost));
-  if (hval) CK(cudaMemcpy(hval, w.h + b * T1 * w.nc, T1 * w.nc * 8, cudaMemcpyDeviceToHost));
-  if (scal) CK(cudaMemcpy(scal, w.scal + b * T1 * SC_COUNT, T1 * SC_COUNT * 8, cudaMemcpyDeviceToHost));
+  if (AB) CK(cudaMemcpyAsync(AB, w.AB + b * T * w.n * w.nz, T * w.n * w.nz * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (H) CK(cudaMemcpyAsync(H, w.H + b * T1 * w.nz * w.nz, T1 * w.nz * w.nz * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (g) CK(cudaMemcpyAsync(g, w.g + b * T1 * w.nz, T1 * w.nz * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (gap) CK(cudaMemcpyAsync(gap, w.gap + b * T * w.n, T * w.n * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (hval) CK(cudaMemcpyAsync(hval, w.h + b * T1 * w.nc, T1 * w.nc * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (scal) CK(cudaMemcpyAsync(scal, w.scal + b * T1 * SC_COUNT, T1 * SC_COUNT * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
@@ -826,15 +826,14 @@ __global__ void k_gemm_tn_test(int mt, int nt, int K, const double *A, int lda, 
 
 // unit-test hook for the DMMA tile GEMM: C (8mt x 8nt) = A^T B, A [K][lda], B [K][ldb], host pointers
 int32_t mpc_debug_gemm_tn(int32_t mt, int32_t nt, int32_t K, const double *A, int32_t lda, const double *B, int32_t ldb, double *C, int32_t ldc) {
-  double *dA, *dB, *dC;
+  CudaArray<double> dA, dB, dC;
   size_t sa = (size_t)K * lda * 8, sb = (size_t)K * ldb * 8, sc = (size_t)8 * mt * ldc * 8;
-  CK(cudaMalloc(&dA, sa)); CK(cudaMalloc(&dB, sb)); CK(cudaMalloc(&dC, sc));
+  CK(dA.ensure(sa / 8)); CK(dB.ensure(sb / 8)); CK(dC.ensure(sc / 8));
   CK(cudaMemcpy(dA, A, sa, cudaMemcpyHostToDevice)); CK(cudaMemcpy(dB, B, sb, cudaMemcpyHostToDevice));
   CK(cudaFuncSetAttribute(k_gemm_tn_test, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sa + sb + sc)));
   k_gemm_tn_test<<<1, 256, sa + sb + sc>>>(mt, nt, K, dA, lda, dB, ldb, dC, ldc);
   CK(cudaGetLastError());
   CK(cudaMemcpy(C, dC, sc, cudaMemcpyDeviceToHost));
-  cudaFree(dA); cudaFree(dB); cudaFree(dC);
   return 0;
 }
 
@@ -845,10 +844,10 @@ static double time_peak(int device, void (*kernel)(double *, int), int warm_iter
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, device);
   const int blocks = prop.multiProcessorCount * 8, threads = 256;
-  double *out = nullptr;
-  if (cudaMalloc(&out, (size_t)blocks * threads * 8) != cudaSuccess) return -1.0;
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
+  CudaArray<double> out;
+  if (out.ensure((size_t)blocks * threads) != cudaSuccess) return -1.0;
+  CudaEvent e0, e1;
+  e0.ensure(cudaEventDefault); e1.ensure(cudaEventDefault);
   kernel<<<blocks, threads>>>(out, warm_iters);
   float best = 1e30f;
   for (int rep = 0; rep < 5; rep++) {
@@ -859,7 +858,6 @@ static double time_peak(int device, void (*kernel)(double *, int), int warm_iter
     float ms; cudaEventElapsedTime(&ms, e0, e1);
     if (ms < best) best = ms;
   }
-  cudaFree(out); cudaEventDestroy(e0); cudaEventDestroy(e1);
   double flops = flop_per_thread * (double)iters * blocks * threads;
   return flops / (best * 1e-3) / 1e12;
 }
@@ -868,149 +866,110 @@ double mpc_measure_fp64_peak(int32_t device) { return time_peak(device, k_dfma_p
 double mpc_measure_fp64_peak_dmma(int32_t device) { return time_peak(device, k_dmma_peak, 256, 1 << 14, 512.0 * 8 / 32); }
 
 // ---- rigid-body terms in front of the whole-body QPs (include/mpcb200.h)
-// with per-instance models, state i is evaluated with instance i's model: only a full batch of states has a model for each
-static const char *check_model_count(const mpc_solver *h, int count) {
-  return (h->instance_models && count != h->w.B) ? "per-instance models are set: count must equal the solver batch" : nullptr;
+// the checks of mpc_rbd_terms* and mpc_ikid_terms*; with per-instance models, state i is evaluated with instance i's model: only a
+// full batch of states has a model for each
+static int check_terms(const mpc_solver *h, const char *fn, int count) {
+  if (enter(h, fn, false)) return 1;
+  if (h->w.kind == MPC_KIND_CENT) return fail(std::string(fn) + ": the centroidal model has no rigid-body tree");
+  if (count <= 0) return fail(std::string(fn) + ": count out of range");
+  if (h->instance_models && count != h->w.B) return fail(std::string(fn) + ": per-instance models are set: count must equal the solver batch");
+  return 0;
 }
+
 int32_t mpc_rbd_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, uint64_t M_dev, uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t vf_dev,
                              uint64_t stream) {
-  if (!h) return fail("null handle");
-  if (h->w.kind == MPC_KIND_CENT) return fail("mpc_rbd_terms: the centroidal model has no rigid-body tree");
-  if (count <= 0) return fail("mpc_rbd_terms: count out of range");
-  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_rbd_terms: ") + e);
-  CK(cudaSetDevice(h->device));
-  const size_t smem = sizeof(FullWsT<false>);
-  CK(cudaFuncSetAttribute(k_rbd_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); // per device: set on every call (microseconds)
-  k_rbd_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, (double *)M_dev, (double *)nle_dev,
-                                                                                  (double *)Jc_dev, (double *)dJv_dev, (double *)vf_dev);
+  if (check_terms(h, "mpc_rbd_terms_device", count)) return 1;
+  k_rbd_terms<<<count, 128, sizeof(FullWsT<false>), stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, (double *)M_dev,
+                                                                                                 (double *)nle_dev, (double *)Jc_dev, (double *)dJv_dev, (double *)vf_dev);
   CK(cudaGetLastError());
   return 0;
 }
 int32_t mpc_rbd_terms(mpc_solver_t *h, int32_t count, const double *x, double *M, double *nle, double *Jc, double *dJv, double *vf) {
-  if (!h) return fail("null handle");
-  if (count <= 0) return fail("mpc_rbd_terms: count out of range");
-  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_rbd_terms: ") + e);
-  CK(cudaSetDevice(h->device));
-  const size_t B = count, per = (NQ + NV) + NV * NV + NV + 12 * NV + 12 + 12;
-  double *d = nullptr;
-  CK(cudaMalloc(&d, 8 * B * per));
-  double *dx = d, *dM = dx + B * (NQ + NV), *dn = dM + B * NV * NV, *dJ = dn + B * NV, *dd = dJ + B * 12 * NV, *dv = dd + B * 12;
-  int rc = 0;
-  if (cudaMemcpyAsync(dx, x, 8 * B * (NQ + NV), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) rc = fail("H2D of the states failed");
-  if (!rc) rc = mpc_rbd_terms_device(h, count, (uint64_t)dx, (uint64_t)dM, (uint64_t)dn, (uint64_t)dJ, (uint64_t)dd, (uint64_t)dv, 0);
-  auto back = [&](double *dst, const double *src, size_t n) { if (!rc && dst && cudaMemcpyAsync(dst, src, 8 * B * n, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) rc = fail("D2H failed"); };
-  back(M, dM, NV * NV); back(nle, dn, NV); back(Jc, dJ, 12 * NV); back(dJv, dd, 12); back(vf, dv, 12);
-  if (cudaStreamSynchronize(h->stream) != cudaSuccess && !rc) rc = fail("mpc_rbd_terms: kernel failed");
-  cudaFree(d);
-  return rc;
+  if (check_terms(h, "mpc_rbd_terms", count)) return 1;
+  return stage_terms(h, count, x, {{M, NV * NV}, {nle, NV}, {Jc, 12 * NV}, {dJv, 12}, {vf, 12}}, [&](const uint64_t *o) {
+    return mpc_rbd_terms_device(h, count, o[0], o[1], o[2], o[3], o[4], o[5], 0);
+  });
 }
 
 int32_t mpc_ikid_terms_device(mpc_solver_t *h, int32_t count, uint64_t x_dev, const int32_t frame_body[2], const double frame_place[2][12], uint64_t M_dev,
                               uint64_t nle_dev, uint64_t Jc_dev, uint64_t dJv_dev, uint64_t Ag_dev, uint64_t dAgv_dev, uint64_t Jang_dev, uint64_t dJang_dev,
                               uint64_t stream) {
-  if (!h || !frame_body || !frame_place) return fail("null handle / frames");
-  if (h->w.kind == MPC_KIND_CENT) return fail("mpc_ikid_terms: the centroidal model has no rigid-body tree");
-  if (count <= 0) return fail("mpc_ikid_terms: count out of range");
-  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_ikid_terms: ") + e);
-  if (frame_body[0] < 0 || frame_body[0] >= NB || frame_body[1] < 0 || frame_body[1] >= NB) return fail("mpc_ikid_terms: frame body out of range [0, nb)");
-  CK(cudaSetDevice(h->device));
+  if (check_terms(h, "mpc_ikid_terms_device", count)) return 1;
+  if (!frame_body || !frame_place) return fail("mpc_ikid_terms_device: null frames");
+  if (frame_body[0] < 0 || frame_body[0] >= NB || frame_body[1] < 0 || frame_body[1] >= NB) return fail("mpc_ikid_terms_device: frame body out of range [0, nb)");
   IkidFrames fr;
   for (int f = 0; f < 2; f++) {
     fr.body[f] = frame_body[f];
     for (int i = 0; i < 12; i++) fr.place[12 * f + i] = frame_place[f][i];
   }
-  const size_t smem = sizeof(FullWsT<false>);
-  CK(cudaFuncSetAttribute(k_ikid_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_ikid_terms<<<count, 128, smem, stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, fr, (double *)M_dev, (double *)nle_dev,
-                                                                                   (double *)Jc_dev, (double *)dJv_dev, (double *)Ag_dev, (double *)dAgv_dev,
-                                                                                   (double *)Jang_dev, (double *)dJang_dev);
+  k_ikid_terms<<<count, 128, sizeof(FullWsT<false>), stream ? (cudaStream_t)stream : h->stream>>>(h->w.model, h->w.model_stride, (const double *)x_dev, count, fr,
+                                                                                                  (double *)M_dev, (double *)nle_dev, (double *)Jc_dev, (double *)dJv_dev,
+                                                                                                  (double *)Ag_dev, (double *)dAgv_dev, (double *)Jang_dev, (double *)dJang_dev);
   CK(cudaGetLastError());
   return 0;
 }
 int32_t mpc_ikid_terms(mpc_solver_t *h, int32_t count, const double *x, const int32_t frame_body[2], const double frame_place[2][12], double *M, double *nle,
                        double *Jc, double *dJv, double *Ag, double *dAgv, double *Jang, double *dJang) {
-  if (!h) return fail("null handle");
-  if (count <= 0) return fail("mpc_ikid_terms: count out of range");
-  if (const char *e = check_model_count(h, count)) return fail(std::string("mpc_ikid_terms: ") + e);
-  CK(cudaSetDevice(h->device));
-  const size_t B = count, per = (NQ + NV) + NV * NV + NV + 12 * NV + 12 + 6 * NV + 6 + 6 * NV + 6;
-  double *d = nullptr;
-  CK(cudaMalloc(&d, 8 * B * per));
-  double *dx = d, *dM = dx + B * (NQ + NV), *dn = dM + B * NV * NV, *dJ = dn + B * NV, *dd = dJ + B * 12 * NV, *dA = dd + B * 12, *dAv = dA + B * 6 * NV,
-         *dJa = dAv + B * 6, *dJav = dJa + B * 6 * NV;
-  int rc = 0;
-  if (cudaMemcpyAsync(dx, x, 8 * B * (NQ + NV), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) rc = fail("H2D of the states failed");
-  if (!rc) rc = mpc_ikid_terms_device(h, count, (uint64_t)dx, frame_body, frame_place, (uint64_t)dM, (uint64_t)dn, (uint64_t)dJ, (uint64_t)dd, (uint64_t)dA,
-                                      (uint64_t)dAv, (uint64_t)dJa, (uint64_t)dJav, 0);
-  auto back = [&](double *dst, const double *src, size_t n) { if (!rc && dst && cudaMemcpyAsync(dst, src, 8 * B * n, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) rc = fail("D2H failed"); };
-  back(M, dM, NV * NV); back(nle, dn, NV); back(Jc, dJ, 12 * NV); back(dJv, dd, 12);
-  back(Ag, dA, 6 * NV); back(dAgv, dAv, 6); back(Jang, dJa, 6 * NV); back(dJang, dJav, 6);
-  if (cudaStreamSynchronize(h->stream) != cudaSuccess && !rc) rc = fail("mpc_ikid_terms: kernel failed");
-  cudaFree(d);
-  return rc;
+  if (check_terms(h, "mpc_ikid_terms", count)) return 1;
+  return stage_terms(h, count, x, {{M, NV * NV}, {nle, NV}, {Jc, 12 * NV}, {dJv, 12}, {Ag, 6 * NV}, {dAgv, 6}, {Jang, 6 * NV}, {dJang, 6}}, [&](const uint64_t *o) {
+    return mpc_ikid_terms_device(h, count, o[0], frame_body, frame_place, o[1], o[2], o[3], o[4], o[5], o[6], o[7], o[8], 0);
+  });
 }
 
 // ---- device-side gait / swing-foot references (include/mpcb200.h, SURVEY 8f row f-4)
 int32_t mpc_gait_setup(mpc_solver_t *h, const mpc_gait_t *gait, const int32_t *mirror, const double *urefs) {
-  if (!h || !gait) return fail("null handle / gait");
-  if (!h->setup_done) return fail("mpc_gait_setup before mpc_setup");
+  if (enter(h, "mpc_gait_setup", true)) return 1;
+  if (!gait) return fail("mpc_gait_setup: null gait");
   if (gait->T_ds <= 0 || gait->T_ss <= 0 || gait->cycles < 0 || gait->cycles > 3) return fail("mpc_gait_setup: schedule out of range (T_ds, T_ss > 0, cycles <= 3)");
   if (h->w.kind != MPC_KIND_FULL && (gait->n_uref <= 0 || !urefs)) return fail("mpc_gait_setup: the kinodynamic / centroidal gaits need the control-reference table");
-  CK(cudaSetDevice(h->device));
   Ws &w = h->w;
+  h->gait_ready = false; // until every buffer of the new gait is uploaded
   GaitCfg g;
   std::memset(&g, 0, sizeof g);
   gait_fill_cfg(*gait, w.kind, w.T, g);
   std::vector<int8_t> phases;
   gait_build_schedule(*gait, w.T, phases, g);
-  cudaFree(h->d_gait); cudaFree(h->d_gait_robots); cudaFree(h->d_gait_phases); cudaFree(h->d_gait_urefs); cudaFree(h->d_feet);
-  h->d_gait = nullptr; h->d_gait_robots = nullptr; h->d_gait_phases = nullptr; h->d_gait_urefs = nullptr; h->d_feet = nullptr;
-  CK(cudaMalloc(&h->d_gait, sizeof(GaitCfg)));
-  CK(cudaMalloc(&h->d_gait_robots, sizeof(GaitRobot) * w.B));
-  CK(cudaMalloc(&h->d_gait_phases, phases.size()));
-  CK(cudaMalloc(&h->d_feet, 8 * (size_t)w.B * 24));
-  CK(cudaMemcpy(h->d_gait_phases, phases.data(), phases.size(), cudaMemcpyHostToDevice));
-  g.phases = h->d_gait_phases;
-  if (gait->n_uref > 0 && urefs) {
-    CK(cudaMalloc(&h->d_gait_urefs, 8 * (size_t)gait->n_uref * MPC_MAXU));
-    CK(cudaMemcpy(h->d_gait_urefs, urefs, 8 * (size_t)gait->n_uref * MPC_MAXU, cudaMemcpyHostToDevice));
-    g.urefs = h->d_gait_urefs;
-  }
-  CK(cudaMemcpy(h->d_gait, &g, sizeof g, cudaMemcpyHostToDevice));
   const std::vector<GaitRobot> rs = gait_init_robots(*gait, w.B, mirror);
-  CK(cudaMemcpy(h->d_gait_robots, rs.data(), sizeof(GaitRobot) * w.B, cudaMemcpyHostToDevice));
+  GaitBufs nb; // the previous gait's buffers stay allocated until these exist
+  CK(nb.cfg.ensure(1)); CK(nb.robots.ensure(w.B)); CK(nb.phases.ensure(phases.size())); CK(nb.feet.ensure((size_t)w.B * 24));
+  CK(cudaMemcpyAsync(nb.phases, phases.data(), phases.size(), cudaMemcpyHostToDevice, h->stream));
+  g.phases = nb.phases;
+  if (gait->n_uref > 0 && urefs) {
+    CK(nb.urefs.ensure((size_t)gait->n_uref * MPC_MAXU));
+    CK(cudaMemcpyAsync(nb.urefs, urefs, 8 * (size_t)gait->n_uref * MPC_MAXU, cudaMemcpyHostToDevice, h->stream));
+    g.urefs = nb.urefs;
+  }
+  CK(cudaMemcpyAsync(nb.cfg, &g, sizeof g, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(nb.robots, rs.data(), sizeof(GaitRobot) * w.B, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->gait = std::move(nb);
   h->gait_t = 0;
   h->gait_ready = true;
   return 0;
 }
 
 int32_t mpc_gait_tick(mpc_solver_t *h, const double *lf, const double *rf) {
-  if (!h) return fail("null handle");
+  if (enter(h, "mpc_gait_tick", false)) return 1;
   if (!h->gait_ready) return fail("mpc_gait_tick before mpc_gait_setup");
   if ((lf == nullptr) != (rf == nullptr)) return fail("mpc_gait_tick: pass both measured placements or neither");
-  CK(cudaSetDevice(h->device));
   Ws &w = h->w;
-  double *dl = h->d_feet, *dr = h->d_feet + (size_t)w.B * 12;
+  double *dl = h->gait.feet, *dr = dl + (size_t)w.B * 12;
   if (lf) {
     CK(cudaMemcpyAsync(dl, lf, 8 * (size_t)w.B * 12, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(dr, rf, 8 * (size_t)w.B * 12, cudaMemcpyHostToDevice, h->stream));
   } else if (w.kind == MPC_KIND_CENT) {
     dl = dr = nullptr; // the centroidal state carries no feet: the soles are taken where last tick's plan wanted them (exact tracking)
   } else {
-    const size_t smem = sizeof(FullWsT<false>);
-    CK(cudaFuncSetAttribute(k_feet_of_prediction, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); // per device: set on every call
-    k_feet_of_prediction<<<w.B, 128, smem, h->stream>>>(w, dl, dr);
+    k_feet_of_prediction<<<w.B, 128, sizeof(FullWsT<false>), h->stream>>>(w, dl, dr);
   }
-  k_gait_tick<<<w.B, 128, 0, h->stream>>>(w, h->d_gait, h->d_gait_robots, h->gait_t, dl, dr);
+  k_gait_tick<<<w.B, 128, 0, h->stream>>>(w, h->gait.cfg, h->gait.robots, h->gait_t, dl, dr);
   CK(cudaGetLastError());
   h->gait_t++;
   return 0;
 }
 
 int32_t mpc_get_knots(mpc_solver_t *h, mpc_knot_t *knots, mpc_term_t *terms) {
-  if (!h) return fail("null handle");
-  if (!h->setup_done) return fail("mpc_get_knots before mpc_setup");
-  CK(cudaSetDevice(h->device));
+  if (enter(h, "mpc_get_knots", true)) return 1;
   Ws &w = h->w;
   if (knots) CK(cudaMemcpyAsync(knots, w.knots, sizeof(mpc_knot_t) * (size_t)w.B * w.T, cudaMemcpyDeviceToHost, h->stream));
   if (terms) CK(cudaMemcpyAsync(terms, w.terms, sizeof(mpc_term_t) * (size_t)w.B, cudaMemcpyDeviceToHost, h->stream));

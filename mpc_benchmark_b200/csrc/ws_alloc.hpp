@@ -53,11 +53,13 @@ template <class Alloc> size_t alloc_ws(Ws &w, Alloc &&alloc) {
   return total;
 }
 
-template <class Free> void free_ws(Ws &w, Free &&fr) {
-  void *ptrs[] = {w.knots, w.terms, w.x0, w.xs, w.us, w.vs, w.lams, w.vs_prev, w.lams_prev, w.txs, w.tus, w.tvs, w.tlams, w.dxs, w.dus, w.dvs,
-                  w.dlams, w.AB, w.H, w.lxu, w.g, w.T6, w.E6, w.gE, w.fbar, w.dbar, w.vplus, w.lplus, w.CDact, w.nca, w.act_idx, w.gap, w.h,
-                  w.scal, w.tscal, w.xdot, w.lamc, w.W, w.pt, w.K, w.Kfb, w.dphi, w.ric_scratch, w.phase, w.st, w.counters, w.lists};
-  for (void *p : ptrs) if (p) fr(p);
+// doubles per instance of the trajectory arrays the C-ABI moves in and out: xs, us, vs, lams and the feedback gains Kfb
+struct TrajSizes {
+  size_t xs, us, vs, lams, K;
+};
+inline TrajSizes traj_sizes(const Ws &w) {
+  const size_t T = w.T, T1 = T + 1;
+  return {T1 * w.nx, T * w.m, T1 * w.nc, T1 * w.n, T * w.m * w.n};
 }
 
 // the time-parallel LQ solve's per-(instance, leg) blocks for `legs` legs (lq_legs >= 2), allocated on first need; returns bytes
@@ -73,10 +75,6 @@ template <class Alloc> size_t alloc_leg_ws(const Ws &w, LegWs &lw, int legs, All
   for (int i = 0; i < 4; i++) { *p[i] = (double *)alloc(n * sz[i] * 8); total += n * sz[i] * 8; }
   lw.L = legs;
   return total;
-}
-template <class Free> void free_leg_ws(LegWs &lw, Free &&fr) {
-  for (double *p : {lw.sum, lw.ws, lw.buf, lw.scratch}) if (p) fr(p);
-  lw = LegWs{};
 }
 
 } // namespace mpcdev
