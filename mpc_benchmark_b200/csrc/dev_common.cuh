@@ -346,10 +346,15 @@ HD void inv6(const double *A, double *Ai) {
   for (int i = 0; i < 6; i++) for (int j = 0; j < 6; j++) Ai[6 * i + j] = M[i][6 + j];
 }
 
-// y[i] = (y0 ? y0[i] : 0) + sum_j A[i * lda + j] x[j] for a matrix in shared memory: rows over warps (RB at a time, independent
+// y[i * incy] = (y0 ? y0[i] : 0) + sum_j A[i * lda + j] x[j] for a matrix in shared memory: rows over warps (RB at a time, independent
 // reduction chains), columns over lanes — consecutive lanes read consecutive doubles, so there are no bank conflicts whatever
-// the leading dimension (a row per thread is a 16-way conflict for ld = 8 mod 16).  No barrier inside.
-template <int RB = 7> HD void matvec_rows(const double *A, int lda, int rows, int cols, const double *x, const double *y0, double *y) {
+// the leading dimension (a row per thread is a 16-way conflict for ld = 8 mod 16).  No barrier inside.  each(i, j, a) is called
+// once for every entry a = A[i * lda + j] read, so that a caller can derive another matrix from A in the same pass.
+struct NoEach {
+  HD void operator()(int, int, double) const {}
+};
+template <int RB = 7, class Each = NoEach>
+HD void matvec_rows(const double *A, int lda, int rows, int cols, const double *x, const double *y0, double *y, int incy = 1, Each each = Each()) {
   for (int base = WARP_ID * RB; base < rows; base += NWARPS * RB) {
     double acc[RB];
 #pragma unroll
@@ -358,14 +363,14 @@ template <int RB = 7> HD void matvec_rows(const double *A, int lda, int rows, in
       const double xj = x[j];
 #pragma unroll
       for (int r = 0; r < RB; r++)
-        if (base + r < rows) acc[r] += A[(base + r) * lda + j] * xj;
+        if (base + r < rows) { const double a = A[(base + r) * lda + j]; acc[r] += a * xj; each(base + r, j, a); }
     }
 #pragma unroll
     for (int r = 0; r < RB; r++) acc[r] = WARP_SUM(acc[r]);
     if (LANE0) {
 #pragma unroll
       for (int r = 0; r < RB; r++)
-        if (base + r < rows) y[base + r] = acc[r] + (y0 ? y0[base + r] : 0.0);
+        if (base + r < rows) y[(base + r) * incy] = acc[r] + (y0 ? y0[base + r] : 0.0);
     }
   }
 }

@@ -19,19 +19,23 @@ namespace mpcdev {
 #ifdef MPC_HOST_EMU
 // host reference of mma_tn and mma_tn_g
 inline void mma_tn_ref(int mt, int nt, int K, const double *A, int lda, const double *B, int ldb, double *C, int ldc, const double *Cinit, int ldci,
-                       int vr, int vc, bool upper_only, double *Cg, int ldcg, int vcg) {
+                       int vr, int vc, bool upper_only, double *Cg, int ldcg, int vcg, double *C2 = nullptr, int ldc2 = 0) {
   for (int i = 0; i < 8 * mt; i++)
     for (int j = 0; j < 8 * nt; j++) {
       if (upper_only && (j / 16) < (i / 16)) continue;
       double s = (Cinit && i < vr && j < vc) ? Cinit[i * ldci + j] : 0.0;
       for (int k = 0; k < K; k++) s += A[k * lda + i] * B[k * ldb + j];
       C[i * ldc + j] = s;
+      if (C2) C2[i * ldc2 + j] = s;
       if (Cg && j < vcg) Cg[i * ldcg + j] = s;
     }
   if (upper_only)
     for (int i = 0; i < 8 * mt; i++)
       for (int j = 0; j < 8 * nt; j++)
-        if ((j / 16) < (i / 16) && i < (Cinit ? vc : 8 * nt)) C[i * ldc + j] = C[j * ldc + i];
+        if ((j / 16) < (i / 16) && i < (Cinit ? vc : 8 * nt)) {
+          C[i * ldc + j] = C[j * ldc + i];
+          if (C2) C2[i * ldc2 + j] = C[j * ldc + i];
+        }
 }
 #else
 __device__ __forceinline__ void dmma_8x8x4(double &c0, double &c1, double a, double b) {
@@ -79,11 +83,11 @@ __device__ __forceinline__ void acc_init(double (&c)[2][2][2], const TilePair &w
       }
     }
 }
-// store the existing tiles to C, and their columns < vcg to the global mirror Cg (if any; vcg, ldcg even).  mirror: the block lies
-// above the diagonal of a symmetric result and is also stored transposed (never a tile anyone reads as Cinit); columns >= vcm are
-// scratch and stay out of the rows below
+// store the existing tiles to C (and the same entries to the shared-memory copy C2, if any; ldc2 even), and their columns < vcg to
+// the global mirror Cg (if any; vcg, ldcg even).  mirror: the block lies above the diagonal of a symmetric result and is also stored
+// transposed (never a tile anyone reads as Cinit); columns >= vcm are scratch and stay out of the rows below
 __device__ __forceinline__ void acc_store(const double (&c)[2][2][2], const TilePair &w, int g, int t, double *C, int ldc, double *Cg, int ldcg, int vcg,
-                                          bool mirror, int vcm) {
+                                          bool mirror, int vcm, double *C2 = nullptr, int ldc2 = 0) {
 #pragma unroll
   for (int a = 0; a < 2; a++)
 #pragma unroll
@@ -91,10 +95,11 @@ __device__ __forceinline__ void acc_store(const double (&c)[2][2][2], const Tile
       if ((a == 1 && !w.r2) || (b == 1 && !w.c2)) continue;
       const int row = (w.ti + a) * 8 + g, col = (w.tj + b) * 8 + 2 * t;
       *reinterpret_cast<double2 *>(C + row * ldc + col) = make_double2(c[a][b][0], c[a][b][1]);
+      if (C2) *reinterpret_cast<double2 *>(C2 + row * ldc2 + col) = make_double2(c[a][b][0], c[a][b][1]);
       if (Cg && col < vcg) *reinterpret_cast<double2 *>(Cg + row * ldcg + col) = make_double2(c[a][b][0], c[a][b][1]);
       if (mirror) {
-        if (col < vcm) C[col * ldc + row] = c[a][b][0];
-        if (col + 1 < vcm) C[(col + 1) * ldc + row] = c[a][b][1];
+        if (col < vcm) { C[col * ldc + row] = c[a][b][0]; if (C2) C2[col * ldc2 + row] = c[a][b][0]; }
+        if (col + 1 < vcm) { C[(col + 1) * ldc + row] = c[a][b][1]; if (C2) C2[(col + 1) * ldc2 + row] = c[a][b][1]; }
       }
     }
 }
@@ -104,10 +109,11 @@ __device__ __forceinline__ void acc_store(const double (&c)[2][2][2], const Tile
 //   init: 0 (Cinit == nullptr) or Cinit (ldci) restricted to rows < vr and cols < vc (zero outside) — lets the
 //   Hessian update read H_k straight from global memory while keeping the shared copy zero-padded.
 // upper_only: square symmetric result; only the 16 x 16 blocks on / above the block diagonal are computed, the rest is mirrored.
+// C2 (optional, ldc2 even): a second copy of the result, stored from the accumulators with it.
 HD void mma_tn(int mt, int nt, int K, const double *A, int lda, const double *B, int ldb, double *C, int ldc, const double *Cinit, int ldci,
-               int vr, int vc, bool upper_only) {
+               int vr, int vc, bool upper_only, double *C2 = nullptr, int ldc2 = 0) {
 #ifdef MPC_HOST_EMU
-  mma_tn_ref(mt, nt, K, A, lda, B, ldb, C, ldc, Cinit, ldci, vr, vc, upper_only, nullptr, 0, 0);
+  mma_tn_ref(mt, nt, K, A, lda, B, ldb, C, ldc, Cinit, ldci, vr, vc, upper_only, nullptr, 0, 0, C2, ldc2);
 #else
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   const int g = lane >> 2, t = lane & 3;
@@ -124,7 +130,7 @@ HD void mma_tn(int mt, int nt, int K, const double *A, int lda, const double *B,
       const double a0 = ap[k0 * lda], a1 = ap[k0 * lda + ao], b0 = bp[k0 * ldb], b1 = bp[k0 * ldb + bo];
       dmma_2x2(c, a0, a1, b0, b1);
     }
-    acc_store(c, w, g, t, C, ldc, nullptr, 0, 0, upper_only && w.bi < w.bj, vcm);
+    acc_store(c, w, g, t, C, ldc, nullptr, 0, 0, upper_only && w.bi < w.bj, vcm, C2, ldc2);
   }
 #endif
   SYNC();

@@ -133,23 +133,18 @@ HD void ric_kkt_schur(int nca, int na, int nk, double mu, const double *CD, cons
   }
   SYNC();
 }
-// ... then, once Kv <- Sg^-1 Kv:  [ku | Ku] = -Z0 - Z_D Kv  (into Z0's place)
-template <int M> HD void ric_kkt_ku(int nca, int nk, double *Z, int ldz, const double *Kv) {
+// ... then, once Kv <- Sg^-1 Kv:  [ku | Ku] = -Z0 - Z_D Kv  (into Z0's place).  gK (optional; then nk = 1 + n): the gain block of the
+// knot, which receives the same rows straight away, [ku | Ku] (Ku also into Kfb, M x n) and then [kv | Kv] (active rows, compact)
+template <int M> HD void ric_kkt_ku(int nca, int nk, double *Z, int ldz, const double *Kv, double *gK = nullptr, double *Kfb = nullptr) {
   PAR_FOR(e, M * nk) {
     int i = e / nk, c = e % nk;
     double s = -Z[i * ldz + c];
     for (int r = 0; r < nca; r++) s -= Z[i * ldz + nk + r] * Kv[r * nk + c];
     Z[i * ldz + c] = s;
+    if (gK) { gK[e] = s; if (c > 0) Kfb[i * (nk - 1) + c - 1] = s; }
   }
+  if (gK) PAR_FOR(e, nca * nk) gK[M * nk + e] = Kv[e];
   SYNC();
-}
-
-// store the gains of knot k: rows 0..M-1 = [ku | Ku] (and Ku into Kfb), rows M.. = [kv | Kv] (active rows, compact)
-template <int N, int M, int NC> HD void ric_store_gains(const RiccatiIO &io, int k, const double *Z, int ldz, const double *Kv, int nca) {
-  constexpr int NR = 1 + N, S = M + NC;
-  double *gK = io.K + (size_t)k * S * NR;
-  PAR_FOR(e, M * NR) { int i = e / NR, c = e % NR; double v = Z[i * ldz + c]; gK[e] = v; if (c > 0) io.Kfb[((size_t)k * M + i) * N + c - 1] = v; }
-  PAR_FOR(e, nca * NR) gK[M * NR + e] = Kv[e];
 }
 
 // forward sweep start: dx = dx0 of a SEEDED leg, else 0 (force_initial_condition, fulldynamic_talos.py:384); knot k0 = 0 also writes
@@ -238,8 +233,7 @@ template <int N, int M, int NC, bool SEEDED = false> HD void riccati_instance(co
     }
     ric_kkt_schur<N, M>(nca, 1, NR, mu, CD, dbr, Z, ncol, Sg, Kv);
     if (nca > 0) { chol_blocked(Sg, nca, nca, dinv); trsm_blocked(Sg, nca, nca, dinv, Kv, NR, NR); }
-    ric_kkt_ku<M>(nca, NR, Z, ncol, Kv);
-    ric_store_gains<N, M, NC>(io, k, Z, ncol, Kv, nca);
+    ric_kkt_ku<M>(nca, NR, Z, ncol, Kv, io.K + (size_t)k * S * NR, io.Kfb + (size_t)k * M * N);
     // 5. P = Qh + Sh Ku + C' Kv, p = qh + Sh ku + C' kv : in place in H[0:N,0:N] / p, then symmetrise
     PAR_FOR(e, N * NR) {
       int i = e / NR, c = e % NR;

@@ -50,8 +50,9 @@ template <int N, int M, int NC, int NCAP = NC> struct RicFastLayout {
   static constexpr int scratch = need2_all + 64 * ((NC + 7) / 8);   // doubles per instance
   static constexpr int NDINV = (NBLK > MR / 8 ? NBLK : MR / 8) > (NCAP + 7) / 8 ? (NBLK > MR / 8 ? NBLK : MR / 8) : (NCAP + 7) / 8;
   static_assert(need2(NCAP) <= un && NCAP <= NC, "fast carving");
+  static_assert(MR * ldz_of(0) <= N * LDN, "without active rows the value update reads nothing from U0 but Z, which stays clear of P");
   static_assert(un % 2 == 0 && (ZP * LDH) % 2 == 0 && ZP > NZ, "16-byte alignment of the bulk-copy destinations; spare padding column for pt");
-  static constexpr int vecs = 6 * N + 2 * ZP + 36 + 2 * NC + 64 * NDINV + 8 * N + 32 + 16; // vectors, T6, dbr / dva, dinv, [pv | 0] tile, one reduction slot per warp, 8 mbarriers
+  static constexpr int vecs = 5 * N + 2 * ZP + 36 + 2 * NC + 64 * NDINV + 8 * N + 32 + 16; // vectors, T6, dbr / dva, dinv, [pv | 0] tile, one reduction slot per warp, 8 mbarriers
   static constexpr int total = ZP * LDH + un + vecs;
 };
 
@@ -72,14 +73,17 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
   double *G = U0, *P = G + N * LDN;            // phase 1 (the factor first: W spills into its slot, see Ws)
   double *Ws = H + N * LDZ;                    // W (N x LDZ) between its product and the Hessian update: behind [A B], over the tail of the H buffer and the dead factor
   double *vec = U0 + Lay::un;
-  double *p = vec, *pt = p + N, *gh = pt + N, *fb = gh + ZP, *tmp = fb + N, *dx = tmp + N, *z = dx + N, *pv = z + ZP; // gh, z: n + m entries, the others n
-  double *T6 = pv + N, *dbr = T6 + 36, *dva = dbr + NC, *dinv_s = dva + NC, *PV = dinv_s + 64 * Lay::NDINV, *red = PV + 8 * N; // (red: one slot per warp)
+  double *p = vec, *pt = p + N, *gh = pt + N, *fb = gh + ZP, *tmp = fb + N, *dx = tmp + N, *z = dx + N; // gh, z: n + m entries, the others n
+  double *T6 = z + ZP, *dbr = T6 + 36, *dva = dbr + NC, *dinv_s = dva + NC, *PV = dinv_s + 64 * Lay::NDINV, *red = PV + 8 * N; // (red: one slot per warp)
   unsigned long long *mbar = reinterpret_cast<unsigned long long *>(vec + Lay::vecs - 8); // mbarriers in the spare tail of vecs
   ONE_THREAD { for (int i_ = 0; i_ < 7; i_++) MBAR_INIT(mbar + i_, 1); } // 2: T6 / fbar, 3: [A B]; forward sweep: 4, 5: gain rows + vectors, 6: W + [A B]
   // ---- zero the padding of H once; terminal value function: P = H_T[xx] + C'C/mu, p = g_T[x] + C' d/mu
   PAR_FOR(e, ZP * LDH) H[e] = 0.0;
+  PAR_FOR(e, N * 8) PV[e] = 0.0; // columns 1..7 of the [pv | 0] tile stay zero: the substitution solves each column on its own
   SYNC();
   ric_start_value<N, M, NC>(io, seeded, H, LDH, p);
+  PAR_FOR(e, N * N) P[(e / N) * LDN + e % N] = H[(e / N) * LDH + e % N]; // the value update of every later knot writes P itself
+  SYNC();
   // T6 and fbar of a knot arrive by bulk copies one knot ahead (mbar[2]); [A B]_k streams into the H buffer once the value Hessian
   // has been taken out of it (mbar[3]); [A B]_k and H_k are bulk-prefetched into L2 one knot ahead (H_k is read from there as
   // the initial value of the Hessian update's accumulators).
@@ -101,17 +105,10 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     double *gW = io.W + (size_t)k * N * LDW;
     const int nca = io.nca[k];
     if (k > K0) prefetch_knot(k - 1);
-    // 1. ONE pass over the value Hessian left in H by the previous knot: P <- T' H T (E normalisation: T = blockdiag(T6, I)
-    //    touches the 6 base rows / columns only), G <- I + mu_d P, and the normalised gradient tmp <- T' p
+    // 1. P <- T' H T (E normalisation: T = blockdiag(T6, I) touches the 6 base rows / columns only) and the normalised gradient
+    //    tmp <- T' p.  Rows and columns >= 6 of P are already in place: the previous knot's value update stored them with H.
     MBAR_WAIT(mbar + 2, (K1 - 1 - k) & 1); // T6 and fbar of this knot (issued one knot ahead)
     PHASE(21);
-    PAR_FOR(e, N * N) { // rows / columns >= 6: a plain copy — the value update mirrors its upper blocks, H is symmetric up to rounding inside the diagonal blocks
-      const int i = e / N, j = e % N;
-      if (i < 6 || j < 6) continue;
-      const double v = H[i * LDH + j];
-      P[i * LDN + j] = v;
-      G[i * LDN + j] = mu_d * v + ((i == j) ? 1.0 : 0.0);
-    }
     // the 6 base rows / columns, enumerated compactly so that no warp diverges over them: corner (36 terms), top edge, left edge
     PAR_FOR(s_, 36 + 12 * (N - 6)) {
       int i, j;
@@ -131,19 +128,17 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
         for (int q = 0; q < 6; q++) v += H[q * LDH + i] * T6[6 * q + j]; // (row q, column i: the same entries as the top edge, so P stays symmetric bit for bit there)
       }
       P[i * LDN + j] = v;
-      G[i * LDN + j] = mu_d * v + ((i == j) ? 1.0 : 0.0);
     }
     PAR_FOR(i, N) { double v = p[i]; if (i < 6) { v = 0; for (int q = 0; q < 6; q++) v += T6[6 * q + i] * p[q]; } tmp[i] = v; }
-    PAR_FOR(e, N * 8) PV[e] = 0.0;
-    SYNC();
+    SYNC(); // the base rows / columns of P and tmp are complete
     PHASE(16);
-    // the H buffer is idle until the Hessian update: [A B]_k streams into it (one padded row per bulk copy);  pv = p + P f
+    // the H buffer is idle until the Hessian update: [A B]_k streams into it (one padded row per bulk copy; the products read columns
+    // < ZP);  pv = tmp + P f into column 0 of the [pv | 0] tile and G <- I + mu_d P in the same pass over P
     ONE_THREAD MBAR_EXPECT_TX(mbar + 3, N * NZ * 8);
     PAR_FOR(i, N) { FENCE_PROXY_ASYNC(); BULK_G2S(ABs + i * LDZ, gAB + i * NZ, NZ * 8, mbar + 3); }
-    PAR_FOR(e, N * (LDZ - NZ)) { const int i = e / (LDZ - NZ), j = NZ + e % (LDZ - NZ); ABs[i * LDZ + j] = 0.0; }
-    matvec_rows(P, LDN, N, N, fb, tmp, pv);
-    SYNC();
-    PAR_FOR(i, N) PV[8 * i] = pv[i];
+    PAR_FOR(e, N * (ZP - NZ)) { const int i = e / (ZP - NZ), j = NZ + e % (ZP - NZ); ABs[i * LDZ + j] = 0.0; }
+    matvec_rows(P, LDN, N, N, fb, tmp, PV, 8, [&](int i, int j, double v) { G[i * LDN + j] = mu_d * v + ((i == j) ? 1.0 : 0.0); });
+    SYNC(); // G and pv are complete
     if (k > K0) stage_small(k - 1); // T6 and fbar of this knot are consumed
     PHASE(1);
     // 2. G = chol(I + mu_d P)
@@ -165,9 +160,6 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     PHASE(22);
     mma_sym_deferred<N, Lay::MAXQ>(ZP / 8, ABs, LDZ, Ws, LDZ, H, LDH, gH, NZ, NZ, NZ);
     PHASE(18);
-    PAR_FOR(i, NZ) gh[i] = io.g[(size_t)k * NZ + i] + H[i * LDH + NZ];
-    SYNC();
-    PHASE(5);
     // 8. KKT by block elimination.  Buffers [Z | Kv | Rh | CD | Sg] carved for this knot's active rows: over P | G (dead now), or
     //    in the instance's global scratch block when they do not fit
     const int ncol = NR + nca, ldz = (NR + nca + 7) & ~7; // Z columns: [rh | Sh' | D'], padded with zero columns to whole tiles
@@ -178,6 +170,7 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     const double *gCD = io.CDact + (size_t)k * NC * NZ;
     const int32_t *ai = io.act_idx + (size_t)k * NC;
     const double *CD = fits ? CDs : gCD;
+    PAR_FOR(i, N) gh[i] = io.g[(size_t)k * NZ + i] + H[i * LDH + NZ]; // (the control part goes straight into Z's column 0)
     if (fits) PAR_FOR(e, nca * NZ) CDs[e] = gCD[e];
     PAR_FOR(r, nca) dbr[r] = io.dbar[(size_t)k * NC + ai[r]];
     PAR_FOR(e, MR * MR) { // R^ = sym(H_uu), padded with the identity to MR x MR
@@ -186,9 +179,10 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     }
     PAR_FOR(e, MR * ldz) { // (reads the active rows from global memory: no barrier between the copy above and this loop)
       int i = e / ldz, c = e % ldz;
-      Z[e] = (i >= M || c >= ncol) ? 0.0 : ((c == 0) ? gh[N + i] : (c < NR ? H[(N + i) * LDH + c - 1] : gCD[(c - NR) * NZ + N + i])); // H_ux row i (H is symmetric to rounding): conflict-free
+      Z[e] = (i >= M || c >= ncol) ? 0.0
+           : ((c == 0) ? io.g[(size_t)k * NZ + N + i] + H[(N + i) * LDH + NZ] : (c < NR ? H[(N + i) * LDH + c - 1] : gCD[(c - NR) * NZ + N + i])); // H_ux row i (H is symmetric to rounding): conflict-free
     }
-    SYNC();
+    SYNC(); // R^, Z, CD, dbar and gh are staged
     PHASE(6);
     // Z <- R^-1 Z on the tensor pipe: blocked Cholesky, then forward / backward substitution with one warp per 8-column tile of Z
     chol_mma<MR / 8>(Rh, LDR, dinv);
@@ -199,10 +193,10 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     PHASE(9);
     if (nca > 0) { chol_blocked(Sg, nca, nca, dinv); trsm_blocked(Sg, nca, nca, dinv, Kv, NR, NR); }
     PHASE(10);
-    ric_kkt_ku<M>(nca, NR, Z, ldz, Kv);
-    ric_store_gains<N, M, NC>(io, k, Z, ldz, Kv, nca);
+    ric_kkt_ku<M>(nca, NR, Z, ldz, Kv, io.K + (size_t)k * S * NR, io.Kfb + (size_t)k * M * N);
     PHASE(11);
-    // 9. P = Qh + Sh Ku + C' Kv, p = qh + Sh ku + C' kv : in place in H[0:N,0:N] / p.
+    // 9. P = Qh + Sh Ku + C' Kv, p = qh + Sh ku + C' kv : in place in H[0:N,0:N] / p, and the result also into the P buffer (its
+    //    rows / columns >= 6 are the next knot's P as they stand).
     //    Sh Ku = H[N:, 0:N]' Z[:, 1:] runs on the DMMA pipe (K = MP, zero rows beyond M); the active-row part is usually empty.
     PAR_FOR(i, N) {
       double s = gh[i];
@@ -213,7 +207,8 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
     //    Without active rows the product is symmetric up to the rounding of well-scaled terms: upper blocks computed, lower mirrored.
     //    With active rows Ku and Kv carry 1/mu-sized entries that cancel in the sum, and the rounding of that cancellation must be
     //    averaged out as the oracle does: full product, then P <- (P + P') / 2.
-    mma_tn(NBLK, NBLK, MR, H + N * LDH, LDH, Z + 1, ldz, H, LDH, H, LDH, N, N, nca == 0);
+    //    Without active rows the product stores P from its accumulators: the value update reads only Z of U0 then (Lay's static_assert).
+    mma_tn(NBLK, NBLK, MR, H + N * LDH, LDH, Z + 1, ldz, H, LDH, H, LDH, N, N, nca == 0, nca == 0 ? P : nullptr, LDN);
     if (nca > 0) { // 2 x 4 register tiles over (row i, column c)
       constexpr int TC = N / 4;
       PAR_FOR(t, (N / 2) * TC) {
@@ -234,12 +229,15 @@ template <int N, int M, int NC, int NCAP = NC, bool SEEDED = false> HD void ricc
 #pragma unroll
           for (int q = 0; q < 4; q++) H[(i0 + r) * LDH + c0 + q] = a[r][q];
       }
-      SYNC();
+      SYNC(); // the rank-nca update is complete (and CD / Kv over P are consumed)
       PAR_FOR(e, N * N) { // lanes: 8 consecutive j x 4 consecutive i, which keeps the transposed access at 8-way bank conflicts
         const int blk = e >> 5, l = e & 31, i = (blk / (N / 8)) * 4 + (l >> 3), j = (blk % (N / 8)) * 8 + (l & 7);
-        if (i < j) { const double v = 0.5 * (H[i * LDH + j] + H[j * LDH + i]); H[i * LDH + j] = v; H[j * LDH + i] = v; }
+        if (i < j) {
+          const double v = 0.5 * (H[i * LDH + j] + H[j * LDH + i]);
+          H[i * LDH + j] = v; H[j * LDH + i] = v; P[i * LDN + j] = v; P[j * LDN + i] = v;
+        } else if (i == j) P[i * LDN + i] = H[i * LDH + i];
       }
-      SYNC();
+      SYNC(); // H[0:N,0:N] and P are symmetric
     }
     PHASE(19);
     PHASE(12);
